@@ -505,6 +505,17 @@ def guarded(fn, *a, **k):
         return {"error": "%s: %s" % (type(e).__name__, str(e)[:300])}
 
 
+def dump_outputs(out_dir, terms, value):
+    """What the last timed step computed, one float64 DIR/<name>.npy per array: the terms DenseLikelihood.terms
+    returned to its caller and the -2 loglik formed from them.  The data and the theta of every step are fixed by
+    --sites, --warmup and --steps, so two builds run with the same arguments can be compared array by array."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"neg2loglik": value, "logdet": terms["logdet"], "quad": terms["quad"], "logdet_w": terms["logdet_w"],
+              "rank": terms["rank"]}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.atleast_1d(np.asarray(a, dtype=np.float64)))
+
+
 def cusolver_potrf_comparator(torch, dev, n):
     """SURVEY.md §8(d): the library bar - torch.linalg.cholesky (cuSOLVER potrf, FP64) on an SPD matrix of the same
     n.  Comparison only; nothing of it is on the product path."""
@@ -615,6 +626,8 @@ def run_ours(args, rank, world, local_rank):
     launches = L.cocons_launch_count() - launches0
     elapsed = max_over_ranks(e0.elapsed_time(e1) * 1e-3)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, t, values[-1])
     # run-to-run reproducibility of the device-resident arm: the first timed point once more, bit for bit
     tl = point(args.warmup)[1]
     again = n2ll(ctx.terms(_lib.ML, tl, LIMITS, tl["mean"]))
@@ -757,7 +770,13 @@ def main():
     ap.add_argument("--no-large", action="store_true", help="N = 1: skip the n = 100 000 north-star evaluation")
     ap.add_argument("--profile", action="store_true",
                     help="profiling run: device-resident arm only (no DGEMM probe, no e2e leg, no CPU sample)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm times a CPU sample and computes no objective to dump")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

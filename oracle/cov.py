@@ -11,6 +11,7 @@ this module.  Matrices are numpy float64, column-major (Fortran order), as R
 holds them.
 """
 import ctypes
+import json
 import os
 import subprocess
 
@@ -19,18 +20,34 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 ASPECTS = ("std.dev", "scale", "aniso", "tilt", "smooth", "nugget")
 
+
+def _reference_path():
+    """Source tree of the reference R package (cocons 0.1.5), which this repository does not ship: $COCONS_REFERENCE,
+    else BASELINE.json's reference_path.  oracle/Makefile asks this module for it."""
+    if os.environ.get("COCONS_REFERENCE"):
+        return os.environ["COCONS_REFERENCE"]
+    with open(os.path.join(os.path.dirname(_HERE), "BASELINE.json")) as f:
+        return json.load(f)["reference_path"]
+
+
+REFERENCE = _reference_path()
+
 _dp = ctypes.POINTER(ctypes.c_double)
 _libs = {}
 
 
+def _reference_source_present():
+    return os.path.exists(os.path.join(REFERENCE, "src", "cocons_full.cpp"))
+
+
 def build(force=False):
-    """Compile liboracle.so (and _ref when /root/reference is present)."""
+    """Compile liboracle.so (and _ref when REFERENCE holds the reference's source)."""
     so = os.path.join(_HERE, "liboracle.so")
     if force or not os.path.exists(so) or os.path.getmtime(so) < os.path.getmtime(os.path.join(_HERE, "cov_oracle.cpp")):
         subprocess.check_call(["make", "-s", "-C", _HERE, "liboracle.so"])
     ref = os.path.join(_HERE, "_ref", "libcocons_ref.so")
-    if os.path.exists("/root/reference/src/cocons_full.cpp") and (force or not os.path.exists(ref)):
-        subprocess.check_call(["make", "-s", "-C", _HERE, "ref"])
+    if _reference_source_present() and (force or not os.path.exists(ref)):
+        subprocess.check_call(["make", "-s", "-C", _HERE, "ref", "REFERENCE=" + REFERENCE])
 
 
 def _load(kind):
@@ -66,8 +83,7 @@ def _load(kind):
 
 
 def have_reference():
-    return os.path.exists(os.path.join(_HERE, "_ref", "libcocons_ref.so")) or os.path.exists(
-        "/root/reference/src/cocons_full.cpp")
+    return os.path.exists(os.path.join(_HERE, "_ref", "libcocons_ref.so")) or _reference_source_present()
 
 
 def _f(a):

@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE ONLY (oracle/): generates the committed fixtures under tests/golden/.
 
-Run once in the build container (needs /root/reference and oracle/_ref):
+Run once, with COCONS_REFERENCE naming the reference package's source tree (for its data/ and oracle/_ref):
     python -m oracle.make_golden            # everything
     python -m oracle.make_golden --quick    # skip the full-size holes / stripes values
 
@@ -13,6 +13,7 @@ Outputs
                                  nearest.dist patterns, objective and prediction values
   tests/golden/n2ll_cases.json   -2 loglik values: reference-compiled covariance + the literal
                                  numpy/LAPACK restatement of the R objectives (oracle/rmirror.py)
+  tests/golden/fresh_cases.npz   the reference's results on the seeded inputs of oracle/fresh_inputs.py
 """
 import argparse
 import json
@@ -21,12 +22,12 @@ import time
 
 import numpy as np
 
-from . import cov, rmirror
+from . import cov, fresh_inputs, rmirror
 from .rda import frame_to_matrix, read_rda
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = os.path.join(ROOT, "tests", "golden")
-REF = "/root/reference/data"
+REF = os.path.join(cov.REFERENCE, "data")
 KIND = "reference"  # oracle/_ref: the reference's src/cocons_full.cpp / cocons_taper.cpp compiled here
 
 
@@ -320,13 +321,29 @@ def n2ll_cases(d, quick):
     return cases
 
 
+def fresh_cases():
+    """The reference's result of every call of oracle/fresh_inputs.py, under the call's key."""
+    return {call[0]: np.asarray(fresh_inputs.run(call, KIND))
+            for call in list(fresh_inputs.dense_calls()) + list(fresh_inputs.taper_calls())}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--quick", action="store_true")
-    ap.add_argument("--only", choices=["datasets", "cov", "n2ll", "taper"], default=None)
+    ap.add_argument("--only", choices=["datasets", "cov", "n2ll", "taper", "fresh"], default=None)
     args = ap.parse_args()
+    if not cov._reference_source_present():
+        raise SystemExit("oracle.make_golden: no reference source under '%s' - set COCONS_REFERENCE to the cocons "
+                         "source tree" % cov.REFERENCE)
+    if args.only != "fresh" and not os.path.isdir(REF):
+        raise SystemExit("oracle.make_golden: the reference's data sets are not at '%s' - set COCONS_REFERENCE to the "
+                         "cocons source tree" % REF)
     os.makedirs(GOLD, exist_ok=True)
     cov.build(force=True)
+    if args.only in (None, "fresh"):
+        np.savez_compressed(os.path.join(GOLD, "fresh_cases.npz"), **fresh_cases())
+    if args.only == "fresh":
+        return
     d = load_datasets()
     if args.only in (None, "datasets"):
         np.savez_compressed(os.path.join(GOLD, "datasets.npz"), **d)

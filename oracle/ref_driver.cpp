@@ -1,9 +1,10 @@
 // TEST INFRASTRUCTURE ONLY (oracle/): C entry points around the REFERENCE's own
 // dense-covariance source, compiled from where it lies.
 //
-// `#include "cocons_full.cpp"` below resolves (via -I/root/reference/src in
-// oracle/Makefile) to /root/reference/src/cocons_full.cpp, which in turn pulls
-// src/cocons_types.h.  <Rcpp.h> and <boost/math/special_functions/bessel.hpp>
+// `#include "cocons_full.cpp"` below resolves (via -I$(REFERENCE)/src in
+// oracle/Makefile; REFERENCE is the reference's source tree, $COCONS_REFERENCE
+// or else BASELINE.json's reference_path) to the reference's
+// src/cocons_full.cpp, which in turn pulls src/cocons_types.h.  <Rcpp.h> and <boost/math/special_functions/bessel.hpp>
 // resolve to the stand-ins under oracle/shim/.  Nothing of the reference is
 // copied into this repository; the output (oracle/_ref/libcocons_ref.so) is
 // git-ignored and is only ever loaded by tests/, __graft_entry__.smoke() and

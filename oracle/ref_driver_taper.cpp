@@ -1,9 +1,10 @@
 // TEST INFRASTRUCTURE ONLY (oracle/): C entry points around the REFERENCE's own
 // sparse (tapered) covariance source, compiled from where it lies.
 //
-// `#include "cocons_taper.cpp"` resolves (via -I/root/reference/src in
-// oracle/Makefile) to /root/reference/src/cocons_taper.cpp.  <Rcpp.h> and the
-// Boost Bessel header resolve to the stand-ins under oracle/shim/.  Nothing of
+// `#include "cocons_taper.cpp"` resolves (via -I$(REFERENCE)/src in
+// oracle/Makefile, as in ref_driver.cpp) to the reference's
+// src/cocons_taper.cpp.  <Rcpp.h> and the Boost Bessel header resolve to the
+// stand-ins under oracle/shim/.  Nothing of
 // the reference is copied into this repository; the object is linked into
 // oracle/_ref/libcocons_ref.so (git-ignored), which only tests/,
 // __graft_entry__.smoke() and bench.py's CPU-baseline legs ever load.

@@ -15,7 +15,7 @@ import numpy as np
 import pytest
 
 from conftest import relerr, theta_dict
-from oracle import cov, rmirror
+from oracle import cov, fresh_inputs, rmirror
 
 
 def _run_square(case, kind):
@@ -39,34 +39,27 @@ def test_restatement_reproduces_reference_goldens_bit_for_bit(cov_cases):
         assert np.array_equal(got, case["out"]), name
 
 
-@pytest.mark.skipif(not cov.have_reference(), reason="oracle/_ref not built and /root/reference absent")
+@pytest.mark.skipif(not cov.have_reference(), reason="needs the reference's source (COCONS_REFERENCE)")
 def test_compiled_reference_reproduces_its_goldens(cov_cases):
     for name, case in cov_cases.items():
         assert np.array_equal(_run_case(case, "reference"), case["out"]), name
 
 
-@pytest.mark.skipif(not cov.have_reference(), reason="oracle/_ref not built and /root/reference absent")
+@pytest.mark.skipif(not cov.have_reference(), reason="needs the reference's source (COCONS_REFERENCE)")
 def test_restatement_equals_compiled_reference_on_fresh_inputs():
-    rng = np.random.default_rng(7)
-    for p, n in ((1, 40), (3, 90), (5, 61)):
-        locs = rng.uniform(-1, 1, (n, 2))
-        X = np.column_stack([np.ones(n), rng.standard_normal((n, p - 1))])
-        th = {k: 0.3 * rng.standard_normal(p) for k in cov.ASPECTS}
-        th["scale"][0] = -1.5
-        th["nugget"][0] = -3.0
-        a = cov.cov_rns(th, locs, X, [0.5, 2.5], "restatement")
-        b = cov.cov_rns(th, locs, X, [0.5, 2.5], "reference")
-        assert np.array_equal(a, b)
-        a = cov.cov_rns_classic(th, locs, X, "restatement")
-        b = cov.cov_rns_classic(th, locs, X, "reference")
-        assert np.array_equal(a, b)
-        lp = rng.uniform(-1, 1, (17, 2))
-        Xp = np.column_stack([np.ones(17), rng.standard_normal((17, p - 1))])
-        a = cov.cov_rns_pred(th, locs, lp, X, Xp, [0.5, 2.5], "restatement")
-        b = cov.cov_rns_pred(th, locs, lp, X, Xp, [0.5, 2.5], "reference")
-        assert np.array_equal(a, b)
-        x = rng.standard_normal(9) * np.array([1, 1e-5, 1, 1e-6, 0, 1, 1, 1e-4, 1])
-        assert cov.sumsmoothlone(x, 0.3) == cov.sumsmoothlone(x, 0.3, kind="reference")
+    for call in fresh_inputs.dense_calls():
+        assert np.array_equal(fresh_inputs.run(call, "restatement"), fresh_inputs.run(call, "reference")), call[0]
+
+
+FRESH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "fresh_cases.npz")
+
+
+@pytest.mark.skipif(not os.path.exists(FRESH), reason="tests/golden/fresh_cases.npz not generated "
+                                                      "(python -m oracle.make_golden --only fresh, needs the reference)")
+def test_restatement_reproduces_the_stored_reference_results_on_fresh_inputs():
+    stored = np.load(FRESH)
+    for call in list(fresh_inputs.dense_calls()) + list(fresh_inputs.taper_calls()):
+        assert np.array_equal(fresh_inputs.run(call, "restatement"), stored[call[0]]), call[0]
 
 
 def test_bessel_stand_in_against_mpmath():

@@ -8,7 +8,7 @@ import pytest
 
 import cocons_b200 as cb
 from conftest import theta_dict
-from oracle import cov, rmirror
+from oracle import cov, fresh_inputs, rmirror
 
 
 def _entries(case, kind):
@@ -31,34 +31,16 @@ def test_restatement_reproduces_reference_goldens_bit_for_bit(taper_cases):
         assert np.array_equal(_entries(case, "restatement"), case["out"]), name
 
 
-@pytest.mark.skipif(not cov.have_reference(), reason="oracle/_ref not built and /root/reference absent")
+@pytest.mark.skipif(not cov.have_reference(), reason="needs the reference's source (COCONS_REFERENCE)")
 def test_compiled_reference_reproduces_its_goldens(taper_cases):
     for name, case in _cov_cases(taper_cases).items():
         assert np.array_equal(_entries(case, "reference"), case["out"]), name
 
 
-@pytest.mark.skipif(not cov.have_reference(), reason="oracle/_ref not built and /root/reference absent")
+@pytest.mark.skipif(not cov.have_reference(), reason="needs the reference's source (COCONS_REFERENCE)")
 def test_restatement_equals_compiled_reference_on_fresh_inputs():
-    rng = np.random.default_rng(11)
-    for p, n, delta in ((1, 60, 0.5), (3, 150, 0.3), (5, 97, 0.4)):
-        locs = rng.uniform(-1, 1, (n, 2))
-        X = np.column_stack([np.ones(n), rng.standard_normal((n, p - 1))])
-        th = {k: 0.3 * rng.standard_normal(p) for k in cov.ASPECTS}
-        th["scale"][0], th["nugget"][0] = -2.0, -3.0
-        _, ci, rp = rmirror.nearest_dist(locs, delta=delta)
-        for lim in ([0.5, 2.5], [0.3, 0.9]):
-            assert np.array_equal(cov.cov_rns_taper(th, locs, X, ci, rp, lim, "restatement"),
-                                  cov.cov_rns_taper(th, locs, X, ci, rp, lim, "reference"))
-        th0 = dict(th, smooth=np.zeros(p))
-        for lim in ([0.5, 0.5], [1.5, 1.5], [2.5, 2.5], [1.0, 1.0]):
-            assert np.array_equal(cov.cov_rns_taper(th0, locs, X, ci, rp, lim, "restatement"),
-                                  cov.cov_rns_taper(th0, locs, X, ci, rp, lim, "reference"))
-        lp = rng.uniform(-1, 1, (23, 2))
-        lp[4] = locs[9]
-        Xp = np.column_stack([np.ones(23), rng.standard_normal((23, p - 1))])
-        _, cip, rpp = rmirror.nearest_dist(lp, locs, delta=delta)
-        assert np.array_equal(cov.cov_rns_taper_pred(th, locs, lp, X, Xp, cip, rpp, [0.5, 2.5], "restatement"),
-                              cov.cov_rns_taper_pred(th, locs, lp, X, Xp, cip, rpp, [0.5, 2.5], "reference"))
+    for call in fresh_inputs.taper_calls():
+        assert np.array_equal(fresh_inputs.run(call, "restatement"), fresh_inputs.run(call, "reference")), call[0]
 
 
 def test_tapered_family_is_the_isotropic_member_of_the_dense_one(taper_cases):
