@@ -588,6 +588,22 @@ static int finish_timings(cocons_ctx* c) {
   return 0;
 }
 
+// what ws.info < 0 means after a forward substitution (solve.cu): a dependency wait of the dataflow kernel ended
+// at its spin limit instead of hanging the device
+static const char* const kSolveGaveUp = "a dependency wait of the forward substitution gave up (COCONS_ERR_CUDA)";
+
+// after the substitutions on the kept factor (prediction, betas): report a wait that gave up, and clear it so that
+// the factor - still valid - can be used again
+static int solve_status(cocons_ctx* c, const char* who) {
+  COCONS_CUDA_TRY(cudaMemcpyAsync(c->hInfo, c->ws.info, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+  COCONS_CUDA_TRY(cudaStreamSynchronize(c->stream));
+  if (*c->hInfo >= 0) return 0;
+  const int rc = *c->hInfo;
+  COCONS_CUDA_TRY(cudaMemsetAsync(c->ws.info, 0, sizeof(int), c->stream));
+  set_error("%s: %s", who, kSolveGaveUp);
+  return rc;
+}
+
 static int n2ll_impl(cocons_ctx* c, int kind, const double* theta6, const double* limits, const double* mean_p,
                      double* logdet, double* quad, double* logdet_w, int* rank_x, bool taper) {
   if (!c || !theta6 || !limits || !logdet || !quad || kind < COCONS_ML || kind > COCONS_REML || c->r <= 0) {
@@ -638,7 +654,8 @@ static int n2ll_impl(cocons_ctx* c, int kind, const double* theta6, const double
       cudaEventRecord(c->ev[3], st);
       cudaStreamSynchronize(st);
       finish_timings(c);
-      return *c->hInfo;  // not positive definite
+      if (*c->hInfo < 0) set_error("n2ll: %s", kSolveGaveUp);
+      return *c->hInfo;  // > 0: not positive definite
     }
     *logdet = hG[kMaxRhs * kMaxRhs];
     if (qx == 0) {
@@ -855,7 +872,8 @@ int cocons_profile_betas(cocons_ctx* c, int kind, double* betas) {
   launch_gram(c->dRhs, c->n, np, k, c->dGram, st);
   double* hG = c->hStage + 7 * c->p;
   COCONS_CUDA_TRY(cudaMemcpyAsync(hG, c->dGram, sizeof(double) * k * k, cudaMemcpyDeviceToHost, st));
-  COCONS_CUDA_TRY(cudaStreamSynchronize(st));
+  int rc = solve_status(c, "profile_betas");
+  if (rc) return rc;
   std::vector<double> W((size_t)qx * qx);
   for (int a = 0; a < qx; ++a)
     for (int b = 0; b < qx; ++b) W[(size_t)a * qx + b] = hG[a * k + b];
@@ -1052,7 +1070,7 @@ static int predict_impl(cocons_ctx* c, int64_t m, const double* locs_pred, const
     }
   }
   cudaFree(dPart);
-  return 0;
+  return solve_status(c, "predict");
 }
 
 int cocons_predict(cocons_ctx* c, int64_t m, const double* locs_pred, const double* Xp, const double* resid,

@@ -9,6 +9,7 @@
 #include <cooperative_groups.h>
 
 #include <algorithm>
+#include <cstring>
 #include <vector>
 
 #include "../../include/cocons_b200.h"
@@ -526,7 +527,12 @@ __global__ void __launch_bounds__(256, (NR == 1) ? 2 : 1)
 #pragma unroll
       for (int c = 0; c < NR; ++c)
         if (c < nr) {
-          const double y = (rq[c][0][tid] + rq[c][1][tid]) + (rq[c][2][tid] + rq[c][3][tid]);
+          double y = (rq[c][0][tid] + rq[c][1][tid]) + (rq[c][2][tid] + rq[c][3][tid]);
+          // a NaN carried over from b (a NaN payload propagates) may have the 'unset' bits: the row-finishing units
+          // would wait for it until kSolveSpinLimit and give up, so publish it as the canonical quiet NaN
+          unsigned long long bits;
+          memcpy(&bits, &y, sizeof bits);
+          if (bits == kSolveUnset) y = __longlong_as_double(0x7FF8000000000000ll);
           Y[(int64_t)c * ldb + i0 + tid] = y;  // what the other units read
           B[(int64_t)c * ldb + i0 + tid] = y;  // the caller's result, in place of b_I
         }
