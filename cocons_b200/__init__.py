@@ -14,6 +14,7 @@ from .api import (  # noqa: F401
     GetNeg2loglikelihoodTaper,
     GetNeg2loglikelihoodTaperProfile,
     NotPositiveDefinite,
+    TaperedLikelihood,
     coco,
     cocoOptim,
     cocoPredict,

@@ -45,6 +45,9 @@ SIGNATURES = {
     "cocons_cov_rns_taper_pred": (ctypes.c_int, [_i64, _i64, _i64, _dp, _dp, _dp, _dp, _dp, _dp, _i32p, _i32p, _i64,
                                                  _dp]),
     "cocons_ctx_set_taper": (ctypes.c_int, [_vp, _i32p, _i32p, _dp, _i64]),
+    "cocons_ctx_create_taper_tiled": (ctypes.c_int, [ctypes.c_int, _i64, _i64, _i64, _dp, _dp, _dp, _i32p, _i32p, _dp,
+                                                     _i64, _vp, ctypes.POINTER(_vp)]),
+    "cocons_ctx_tile_stats": (ctypes.c_int, [_vp, _lp]),
     "cocons_n2ll_taper": (ctypes.c_int, [_vp, _dp, _dp, _dp, _dp, _dp]),
     "cocons_factor_taper": (ctypes.c_int, [_vp, _dp, _dp]),
     "cocons_predict_taper": (ctypes.c_int, [_vp, _i64, _dp, _dp, _i32p, _i32p, _dp, _i64, _dp, _dp, _dp]),

@@ -444,6 +444,33 @@ class DenseLikelihood:
                 "kernel_ms": kms.value, "kernel_flops": kfl.value}
 
 
+class TaperedLikelihood(DenseLikelihood):
+    """A context for the tapered model only (cocons_ctx_create_taper_tiled): the pattern of `ref_taper` (a `spam`,
+    n x n) is fixed at creation and only the tiles of the Cholesky factor that can be nonzero are stored on the
+    device - so n is bounded by the factor's fill, not by n^2.  terms_taper / factor_taper / get_factor /
+    factor_rows / set_z / timings work as on a DenseLikelihood (and so do GetNeg2loglikelihoodTaper{,Profile}
+    with ctx=); the dense objectives, prediction and simulation raise CoconsError.  At most 128 columns of z."""
+
+    def __init__(self, locs, x_covariates, z, ref_taper, device=0, stream=None):
+        self.locs, self.X = _lib.fmat(locs), _lib.fmat(x_covariates)
+        self.n, self.p = self.X.shape
+        self.z = _lib.fmat(z, rows=self.n)
+        self.r = self.z.shape[1]
+        assert ref_taper.dimension == (self.n, self.n)
+        self._h = _lib._vp()
+        _lib.check(_lib.lib().cocons_ctx_create_taper_tiled(
+            int(device), self.n, self.p, self.r, _lib.ptr(self.locs), _lib.ptr(self.X), _lib.ptr(self.z),
+            _lib.iptr(ref_taper.colindices), _lib.iptr(ref_taper.rowpointers), _lib.ptr(ref_taper.entries),
+            ref_taper.entries.shape[0], stream, self._h))
+        self.q = 0
+
+    def tile_stats(self):
+        """dict(tile_columns, stored_tiles, fill_tiles, tile_products) - see cocons_ctx_tile_stats."""
+        out = np.empty(4, dtype=np.int64)
+        _lib.check(_lib.lib().cocons_ctx_tile_stats(self._h, out.ctypes.data_as(_lib._lp)))
+        return dict(zip(("tile_columns", "stored_tiles", "fill_tiles", "tile_products"), (int(v) for v in out)))
+
+
 # --------------------------------------------------------------------------
 # objectives (R/neg2loglikelihood.R), one-shot: host buffers in, scalar out
 # --------------------------------------------------------------------------
@@ -768,12 +795,13 @@ def _cocoOptim_two_step(coco_object, boundaries, ncores, safe, optim_control, de
 
 
 def cocoOptim(coco_object, boundaries, ncores="auto", safe=True, optim_type="ml", optim_control=None, device=0,
-              forward=False, _first_step=None):
+              forward=False, _first_step=None, tiled=False):
     """R/optim.R:65-365 (dense) and :366-690 (sparse, see _cocoOptim_sparse).  L-BFGS-B (scipy) stands in for optimParallel's optimiser; its
     gradient is the same batched finite-difference scheme (fd_value_and_grad), whose independent
     objective evaluations run on the device-resident context of each rank - across all GPUs when
     launched with one process per GPU - instead of on forked R workers.
-    `boundaries` = dict(theta_init, theta_lower, theta_upper)."""
+    `boundaries` = dict(theta_init, theta_lower, theta_upper).  `tiled` (sparse objects only): evaluate on
+    TaperedLikelihood contexts, which store only the factor's nonzero tiles, instead of dense ones."""
     from scipy.optimize import minimize
 
     dm = getDesignMatrix(coco_object.model_list, coco_object.data)
@@ -803,7 +831,7 @@ def cocoOptim(coco_object, boundaries, ncores="auto", safe=True, optim_type="ml"
     if coco_object.type == "sparse":
         nc = max(1, min(8, int(4e9 // (8 * n * n)))) if ncores == "auto" else int(ncores)
         return _cocoOptim_sparse(coco_object, boundaries, dm, sc, mod_DM, init, lower, upper, ctrl, ndeps, forward,
-                                 nc, safe, optim_type, device)
+                                 nc, safe, optim_type, device, tiled)
     if optim_type in ("pml", "reml"):
         if not isinstance(par_pos["mean"], np.ndarray):
             raise ValueError("Profile ML or Restricted ML only available when considering covariates in the mean.")
@@ -849,7 +877,7 @@ def cocoOptim(coco_object, boundaries, ncores="auto", safe=True, optim_type="ml"
 
 
 def _cocoOptim_sparse(coco_object, boundaries, dm, sc, mod_DM, init, lower, upper, ctrl, ndeps, forward, ncores, safe,
-                      optim_type, device):
+                      optim_type, device, tiled=False):
     """R/optim.R:366-690: the tapered model.  "ml" (:480-531) and "pml" (:533-688, global variance profiled
     out and recovered after the fit).  The penalised two-step fit (:368-478) prunes the model through
     .cocons.update.coco.first.step - validation/UI code outside this path - and is not mirrored."""
@@ -877,8 +905,10 @@ def _cocoOptim_sparse(coco_object, boundaries, dm, sc, mod_DM, init, lower, uppe
         keep = np.arange(init.shape[0]) != first_sigma
         init, lower, upper = init[keep], lower[keep], upper[keep]
         fn_ref = GetNeg2loglikelihoodTaperProfile
-    with DenseLikelihoodPool(coco_object.locs, mod_DM, coco_object.z, size=ncores, device=device) as pool:
-        pool.set_taper(ref_taper)
+    kw = {"ctx_class": TaperedLikelihood, "ref_taper": ref_taper} if tiled else {}
+    with DenseLikelihoodPool(coco_object.locs, mod_DM, coco_object.z, size=ncores, device=device, **kw) as pool:
+        if not tiled:
+            pool.set_taper(ref_taper)
         ctx = pool.ctxs[0]
 
         def fn_on(c, theta):
@@ -1036,9 +1066,12 @@ class DenseLikelihoodPool:
     cannot fill a B200 (holes: 156 evaluations/s one at a time, 321 with 8 in flight) - and every value is
     bit-identical to a single context's (tests/test_gpu_repro.py); across GPUs use distributed.fan_out."""
 
-    def __init__(self, locs, x_covariates, z, size=4, device=0):
+    def __init__(self, locs, x_covariates, z, size=4, device=0, ctx_class=None, **ctx_kw):
+        """`ctx_class` (default DenseLikelihood) and `ctx_kw` make the contexts, e.g. TaperedLikelihood with
+        ref_taper=..."""
         from concurrent.futures import ThreadPoolExecutor
-        self.ctxs = [DenseLikelihood(locs, x_covariates, z, device=device) for _ in range(int(size))]
+        ctx_class = ctx_class or DenseLikelihood
+        self.ctxs = [ctx_class(locs, x_covariates, z, device=device, **ctx_kw) for _ in range(int(size))]
         self.exec = ThreadPoolExecutor(max_workers=len(self.ctxs))
         self.n, self.p, self.r = self.ctxs[0].n, self.ctxs[0].p, self.ctxs[0].r
 

@@ -2,7 +2,9 @@
 // O(n^2) and O(n^3) step is a kernel launch from assembly.cu / chol.cu /
 // solve.cu on the context's stream.  No CPU fallback exists: without a usable
 // CUDA device every computing entry point returns COCONS_ERR_NO_DEVICE.
+#include <algorithm>
 #include <atomic>
+#include <iterator>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -42,6 +44,12 @@ __global__ void residual_kernel(int64_t n, int64_t ld, int p, int nc, const doub
   if (i < n && mean)
     for (int k = 0; k < p; ++k) trend = fma(X[(int64_t)k * ld + i], mean[k], trend);
   for (int c = 0; c < nc; ++c) out[(int64_t)c * ld + i] = (i < n) ? Z[(int64_t)c * ld + i] - trend : 0.0;
+}
+
+static void launch_residual(int64_t n, int64_t ld, int p, int nc, const double* X, const double* Z, const double* mean,
+                            double* out, cudaStream_t st) {
+  note_launch();
+  residual_kernel<<<(unsigned)((ld + 255) / 256), 256, 0, st>>>(n, ld, p, nc, X, Z, mean, out);
 }
 
 // partial sums over a slice of columns k of T (m_pad x n, ld):
@@ -236,6 +244,20 @@ struct cocons_ctx {
   double* dTap = nullptr;
   int64_t tap_nnz = 0;
   bool factor_is_taper = false;
+  // tiled tapered context (cocons_ctx_create_taper_tiled): only the tiles of L that can be nonzero are stored.
+  // Column panel J stacks its tiles column-major: the diagonal tile, the tiles below it (pattern + fill, Morton
+  // order), then one right-hand-side tile holding (z - X mean)^T over the panel's columns, so that the factorisation
+  // carries the forward substitution along (see tiled_factor).
+  bool tiled = false;
+  int64_t T = 0, nstored = 0, nfill = 0, tile_products = 0, rhs_k = 0;
+  std::vector<int64_t> colptr, rows, base, ldp;  // column starts into rows; tile rows (diagonal first); panel layout
+  int64_t g_off = 0;                              // element offset of the Gram block (right-hand sides) in the pool
+  std::vector<int64_t> upd_at;                    // per panel: start of its update map in dMaps
+  int64_t scat_at = 0;                            // start of the right-hand-side scatter map in dMaps
+  double* dPool = nullptr;                        // the stored tiles
+  int64_t pool_elems = 0;
+  int64_t *dTiles = nullptr, *dMaps = nullptr;    // assembly tile map (TaperSink::tiles); update / scatter maps
+  double *dNegI = nullptr, *dLogPart = nullptr;   // -I (128 x rhs_k); log-determinant of each diagonal tile
   double* dCheck = nullptr;  // COCONS_DEBUG_CHECKSUM: 296 partials + [assembly, factor] sums
   double check[2] = {0, 0};
   SiteTable table() const { return SiteTable{dSite, n_pad, dOrig}; }
@@ -423,6 +445,7 @@ void cocons_ctx_destroy(cocons_ctx* c) {
   cudaFree(c->dX), cudaFree(c->dLocs), cudaFree(c->dZ), cudaFree(c->dXb), cudaFree(c->dTheta), cudaFree(c->dSite);
   cudaFree(c->dOrig), cudaFree(c->dA), cudaFree(c->dRhs);
   cudaFree(c->dTapCol), cudaFree(c->dTapRow), cudaFree(c->dInv), cudaFree(c->dTap), cudaFree(c->dCheck);
+  cudaFree(c->dPool), cudaFree(c->dTiles), cudaFree(c->dMaps), cudaFree(c->dNegI), cudaFree(c->dLogPart);
   solve_workspace_destroy(&c->ws);
   chol_workspace_destroy(&c->ws);
   cudaFree(c->dGram);
@@ -444,16 +467,13 @@ void cocons_ctx_destroy(cocons_ctx* c) {
     }                                                                                 \
   } while (0)
 
-int cocons_ctx_create(int device, int64_t n, int64_t p, int64_t r, const double* locs, const double* X,
-                      const double* z, void* stream, cocons_ctx** out) {
-  if (!out || n <= 0 || p <= 0 || r < 0 || !locs || !X || (r > 0 && !z)) {
-    set_error("ctx_create: bad argument");
-    return COCONS_ERR_ARG;
-  }
-  *out = nullptr;
+// tiled: no n_pad^2 matrix and no dense solve workspace (the tiled context allocates its tile pool itself)
+static int ctx_create(int device, int64_t n, int64_t p, int64_t r, const double* locs, const double* X,
+                      const double* z, void* stream, bool tiled, cocons_ctx** out) {
   int rc = check_device(device);
   if (rc) return rc;
   cocons_ctx* c = new cocons_ctx();
+  c->tiled = tiled;
   c->device = device;
   c->n = n, c->p = p, c->r = r;
   c->n_pad = round_up(n, kTile);
@@ -473,8 +493,8 @@ int cocons_ctx_create(int device, int64_t n, int64_t p, int64_t r, const double*
   CTX_TRY(cudaMalloc(&c->dTheta, sizeof(double) * 7 * p));
   CTX_TRY(cudaMalloc(&c->dSite, sizeof(double) * SF_COUNT * np));
   CTX_TRY(cudaMalloc(&c->dOrig, sizeof(int) * np));
-  CTX_TRY(cudaMalloc(&c->dA, sizeof(double) * np * np));
-  if (chol_workspace_create(np, &c->ws) != 0 || solve_workspace_create(np, &c->ws) != 0) {
+  if (!tiled) CTX_TRY(cudaMalloc(&c->dA, sizeof(double) * np * np));
+  if (chol_workspace_create(np, &c->ws) != 0 || (!tiled && solve_workspace_create(np, &c->ws) != 0)) {
     set_error("ctx_create: out of device memory for the factorisation workspace");
     cocons_ctx_destroy(c);
     return COCONS_ERR_ALLOC;
@@ -498,6 +518,24 @@ int cocons_ctx_create(int device, int64_t n, int64_t p, int64_t r, const double*
   return 0;
 }
 
+int cocons_ctx_create(int device, int64_t n, int64_t p, int64_t r, const double* locs, const double* X,
+                      const double* z, void* stream, cocons_ctx** out) {
+  if (!out || n <= 0 || p <= 0 || r < 0 || !locs || !X || (r > 0 && !z)) {
+    set_error("ctx_create: bad argument");
+    return COCONS_ERR_ARG;
+  }
+  *out = nullptr;
+  return ctx_create(device, n, p, r, locs, X, z, stream, false, out);
+}
+
+// the entries that need the dense matrix refuse a tiled context
+static int refuse_tiled(cocons_ctx* c, const char* who) {
+  if (!c || !c->tiled) return 0;
+  set_error("%s: not available on a tiled tapered context (cocons_ctx_create_taper_tiled); it supports "
+            "cocons_n2ll_taper, cocons_factor_taper, cocons_ctx_get_factor and cocons_ctx_factor_rows", who);
+  return COCONS_ERR_STATE;
+}
+
 int cocons_ctx_set_z(cocons_ctx* c, const double* z) {
   if (!c || !z || c->r <= 0) {
     set_error("ctx_set_z: bad argument");
@@ -508,6 +546,7 @@ int cocons_ctx_set_z(cocons_ctx* c, const double* z) {
 }
 
 int cocons_ctx_set_xbetas(cocons_ctx* c, int64_t q, const double* xb) {
+  if (int rc_ = refuse_tiled(c, "ctx_set_xbetas")) return rc_;
   if (!c || q <= 0 || !xb || q >= kMaxRhs) {
     set_error("ctx_set_xbetas: bad argument (q must be in 1..%d)", kMaxRhs - 1);
     return COCONS_ERR_ARG;
@@ -517,6 +556,133 @@ int cocons_ctx_set_xbetas(cocons_ctx* c, int64_t q, const double* xb) {
   COCONS_CUDA_TRY(cudaMalloc(&c->dXb, sizeof(double) * c->n_pad * q));
   c->q = q;
   return upload_sorted(c, xb, q, c->dXb);
+}
+
+// ---- tiled tapered context: layout and factorisation ----------------------------------------------------------
+
+// Tile-level symbolic Cholesky of the Morton-ordered pattern.  The pattern's lower tiles (entries i >= j of the
+// caller's pattern, as the assembly keeps them) give each tile column J its rows below the diagonal; eliminating J
+// adds its rows to those of its parent (the first of them), which yields every tile L can fill (the elimination tree).
+// Then the pool layout: panel J = [diagonal tile, rows below, right-hand-side tile], column-major, ld = 128 x its
+// tiles; the Gram block of the right-hand sides (128 x 128) closes the pool.
+static void tile_symbolic(cocons_ctx* c, const int32_t* colindices, const int32_t* rowpointers) {
+  const int64_t T = c->n_pad / kTile;
+  std::vector<int64_t> inv((size_t)c->n);
+  for (int64_t s = 0; s < c->n; ++s) inv[(size_t)c->perm[(size_t)s]] = s;
+  std::vector<std::vector<int64_t>> st((size_t)T);
+  std::vector<int64_t> keys;
+  for (int64_t i = 0; i < c->n; ++i) {  // one caller row at a time: its few distinct tile pairs
+    keys.clear();
+    const int64_t ti = inv[(size_t)i] / kTile;
+    for (int64_t e = rowpointers[i] - 1; e < rowpointers[i + 1] - 1; ++e) {
+      const int64_t j = colindices[e] - 1;
+      if (i < j) continue;
+      const int64_t tj = inv[(size_t)j] / kTile;
+      if (ti != tj) keys.push_back(std::min(ti, tj) * T + std::max(ti, tj));
+    }
+    std::sort(keys.begin(), keys.end());
+    keys.erase(std::unique(keys.begin(), keys.end()), keys.end());
+    for (int64_t k : keys) st[(size_t)(k / T)].push_back(k % T);
+  }
+  int64_t pattern = 0;
+  for (auto& v : st) {
+    std::sort(v.begin(), v.end());
+    v.erase(std::unique(v.begin(), v.end()), v.end());
+    pattern += (int64_t)v.size();
+  }
+  std::vector<int64_t> merged;
+  for (int64_t J = 0; J < T; ++J) {
+    const auto& v = st[(size_t)J];
+    if (v.empty()) continue;
+    auto& par = st[(size_t)v[0]];
+    merged.clear();
+    std::set_union(par.begin(), par.end(), v.begin() + 1, v.end(), std::back_inserter(merged));
+    par.swap(merged);
+  }
+  c->T = T;
+  c->colptr.assign((size_t)T + 1, 0);
+  c->rows.clear(), c->base.assign((size_t)T, 0), c->ldp.assign((size_t)T, 0);
+  c->tile_products = 0;
+  int64_t off = 0;
+  for (int64_t J = 0; J < T; ++J) {
+    const int64_t m = (int64_t)st[(size_t)J].size();
+    c->colptr[(size_t)J] = (int64_t)c->rows.size();
+    c->rows.push_back(J);
+    c->rows.insert(c->rows.end(), st[(size_t)J].begin(), st[(size_t)J].end());
+    c->tile_products += m * (m + 1) / 2;
+    c->ldp[(size_t)J] = (m + 2) * kTile;
+    c->base[(size_t)J] = off;
+    off += c->ldp[(size_t)J] * kTile;
+  }
+  c->colptr[(size_t)T] = (int64_t)c->rows.size();
+  c->nstored = (int64_t)c->rows.size();
+  c->nfill = c->nstored - T - pattern;
+  c->g_off = off;
+  c->pool_elems = off + (int64_t)kTile * kTile;
+}
+
+// position of tile row I inside panel J (0: diagonal, m_J + 1: the right-hand-side tile, I == T)
+static int64_t tile_pos(const cocons_ctx* c, int64_t I, int64_t J) {
+  const int64_t a = c->colptr[(size_t)J], b = c->colptr[(size_t)J + 1];
+  if (I == c->T) return b - a;
+  const auto it = std::lower_bound(c->rows.begin() + a, c->rows.begin() + b, I);
+  return (it != c->rows.begin() + b && *it == I) ? it - (c->rows.begin() + a) : -1;
+}
+
+// The maps of gemm_nt_tma_kernel's tile-mapped update (chol.cu): for panel J with rows B = [tiles below J, T] (T
+// stands for the right-hand-side tile), pair (a >= b) of B goes to tile (B[a], B[b]) - in panel B[b], or the Gram
+// block when both are right-hand sides.  The scatter map puts the 128 x T*128 block of right-hand sides (transposed)
+// into the right-hand-side tile of every panel.
+static void tile_maps(cocons_ctx* c, std::vector<int64_t>* maps) {
+  maps->clear();
+  c->upd_at.assign((size_t)c->T, 0);
+  for (int64_t J = 0; J < c->T; ++J) {
+    std::vector<int64_t> B(c->rows.begin() + c->colptr[(size_t)J] + 1, c->rows.begin() + c->colptr[(size_t)J + 1]);
+    B.push_back(c->T);
+    const int64_t mb = (int64_t)B.size();
+    c->upd_at[(size_t)J] = (int64_t)maps->size();
+    for (int64_t a = 0; a < mb; ++a)
+      for (int64_t b = 0; b <= a; ++b) {
+        if (B[(size_t)b] == c->T) {
+          maps->push_back(c->g_off);
+          continue;
+        }
+        const int64_t pos = tile_pos(c, B[(size_t)a], B[(size_t)b]);  // >= 0: the fill of the symbolic step
+        maps->push_back(c->base[(size_t)B[(size_t)b]] + pos * kTile);
+      }
+    for (int64_t b = 0; b < mb; ++b) maps->push_back(B[(size_t)b] == c->T ? kTile : c->ldp[(size_t)B[(size_t)b]]);
+  }
+  c->scat_at = (int64_t)maps->size();
+  for (int64_t J = 0; J < c->T; ++J) maps->push_back(c->base[(size_t)J] + c->ldp[(size_t)J] - kTile);
+  for (int64_t J = 0; J < c->T; ++J) maps->push_back(c->ldp[(size_t)J]);
+}
+
+// Right-looking factorisation over the column panels, in order, on the context's stream: every target tile receives
+// its updates in one fixed order (bitwise reproducible).  Per panel: POTRF + inverse of the diagonal tile (K3b), the
+// panel solve X = A W^T over the contiguous rows below it (K4), then ONE tile-mapped launch of C -= P P^T over the
+// lower pairs of its row tiles.  The right-hand-side tile rides along as the last row of every panel: its panel
+// solve gives y_J^T = (L^-1 (z - X mean))_J^T, its updates are the forward substitution, and the Gram block gathers
+// -sum_J y_J^T y_J.  The log-determinant of each diagonal tile goes to dLogPart[J].
+static void tiled_factor(cocons_ctx* c, bool rhs, cudaStream_t st) {
+  cudaMemsetAsync(c->ws.info, 0, sizeof(int), st);
+  const int64_t np = c->n_pad;
+  if (rhs) {
+    cudaMemsetAsync(c->dRhs, 0, sizeof(double) * np * c->rhs_k, st);
+    launch_residual(c->n, np, (int)c->p, (int)c->r, c->dX, c->dZ, c->dTheta + 6 * c->p, c->dRhs, st);
+    // 0 - (-I) R^T: the right-hand sides, transposed, into the right-hand-side tile of every panel (exact)
+    launch_gemm_nt(2, kTile, np, c->rhs_k, c->dNegI, kTile, c->dRhs, np, c->dPool,
+                   (int64_t)(uintptr_t)(c->dMaps + c->scat_at), 0, st);
+  }
+  for (int64_t J = 0; J < c->T; ++J) {
+    double* P = c->dPool + c->base[(size_t)J];
+    const int64_t ld = c->ldp[(size_t)J], below = ld - kTile;
+    double* W = c->ws.winv + J * (int64_t)kTile * kTile;
+    launch_potrf_tile(P, ld, W, c->ws.info, (int)(J * kTile), st);
+    launch_logdet(P, std::min<int64_t>(kTile, c->n - J * kTile), ld, c->dLogPart + J, st);
+    launch_gemm_nt(1, below, kTile, kTile, P + kTile, ld, W, kTile, P + kTile, ld, 0, st);
+    launch_gemm_nt(2, below, below, kTile, P + kTile, ld, P + kTile, ld, c->dPool,
+                   (int64_t)(uintptr_t)(c->dMaps + c->upd_at[(size_t)J]), 1, st);
+  }
 }
 
 // assembly + factorisation of the context's matrix; leaves events 0..2 recorded
@@ -534,7 +700,19 @@ static int assemble_and_factor(cocons_ctx* c, int par, const double* theta6, con
     std::memset(c->hStage + 6 * p, 0, sizeof(double) * p);
   COCONS_CUDA_TRY(cudaMemcpyAsync(c->dTheta, c->hStage, sizeof(double) * 7 * p, cudaMemcpyHostToDevice, c->stream));
   COCONS_CUDA_TRY(cudaEventRecord(c->ev[0], c->stream));
-  if (taper) {
+  if (c->tiled) {
+    // tiled tapered model: zero pool (fill tiles included), unit diagonal in the padding, taper[e] * cov[e] through
+    // the tile map
+    const int64_t last = c->T - 1;
+    launch_taper_site_stage(c->n, (int)p, c->dX, np, c->dLocs, np, c->dTheta, lim[0], lim[1], c->mode, 0,
+                            c->taper_table(), c->stream);
+    COCONS_CUDA_TRY(cudaMemsetAsync(c->dPool, 0, sizeof(double) * c->pool_elems, c->stream));
+    launch_taper_pad_diag(c->n - last * kTile, kTile, c->dPool + c->base[(size_t)last], c->ldp[(size_t)last],
+                          c->stream);
+    TaperSink S{TS_TILED, nullptr, c->dTap, c->dInv, c->dPool, c->T, c->nstored, c->dTiles};
+    launch_taper_entries(0, c->tap_nnz, c->n, c->dTapCol, c->dTapRow, c->taper_table(), c->taper_table(), 1, c->mode,
+                         c->nu_fixed, S, c->stream);
+  } else if (taper) {
     // tapered model: zero matrix, then taper[e] * cov[e] scattered onto the pattern (R/neg2loglikelihood.R:26-31)
     launch_taper_site_stage(c->n, (int)p, c->dX, np, c->dLocs, np, c->dTheta, lim[0], lim[1], c->mode, 0,
                             c->taper_table(), c->stream);
@@ -550,15 +728,18 @@ static int assemble_and_factor(cocons_ctx* c, int par, const double* theta6, con
   c->factor_is_taper = taper;
   static int debug_checksum = -1;
   if (debug_checksum < 0) debug_checksum = getenv("COCONS_DEBUG_CHECKSUM") ? 1 : 0;
-  if (debug_checksum) {
+  if (debug_checksum && !c->tiled) {
     if (!c->dCheck) COCONS_CUDA_TRY(cudaMalloc(&c->dCheck, sizeof(double) * 304));
     checksum_partial_kernel<<<296, 256, 0, c->stream>>>(c->dA, c->n, np, c->dCheck);
     checksum_final_kernel<<<1, 1, 0, c->stream>>>(c->dCheck, 296, c->dCheck + 300);
   }
   COCONS_CUDA_TRY(cudaEventRecord(c->ev[1], c->stream));
-  chol_factor(c->dA, np, np, c->ws, c->stream);
+  if (c->tiled)
+    tiled_factor(c, c->r > 0, c->stream);
+  else
+    chol_factor(c->dA, np, np, c->ws, c->stream);
   COCONS_CUDA_TRY(cudaEventRecord(c->ev[2], c->stream));
-  if (debug_checksum) {
+  if (debug_checksum && !c->tiled) {
     checksum_partial_kernel<<<296, 256, 0, c->stream>>>(c->dA, c->n, np, c->dCheck);
     checksum_final_kernel<<<1, 1, 0, c->stream>>>(c->dCheck, 296, c->dCheck + 301);
     COCONS_CUDA_TRY(cudaMemcpyAsync(c->check, c->dCheck + 300, sizeof(double) * 2, cudaMemcpyDeviceToHost, c->stream));
@@ -575,6 +756,7 @@ static int finish_timings(cocons_ctx* c) {
   COCONS_CUDA_TRY(cudaEventElapsedTime(&d, c->ev[2], c->ev[3]));
   c->ms[0] = a, c->ms[1] = b, c->ms[2] = d, c->ms[3] = a + b + d;
   c->kernel_ms = 0, c->kernel_flops = 0;
+  if (c->tiled) return 0;
   const int64_t outer = chol_outer(c->n_pad);
   const int64_t rest = c->n_pad - 2 * outer * kTile;  // rows/cols right of the first two outer panels
   if (rest > 0) {
@@ -637,10 +819,8 @@ static int n2ll_impl(cocons_ctx* c, int kind, const double* theta6, const double
   for (int64_t c0 = 0; c0 < c->r; c0 += chunk) {
     const int nc = (int)((c->r - c0 < chunk) ? c->r - c0 : chunk);
     double* rhs = c->dRhs + (int64_t)qx * np;
-    note_launch();
-    residual_kernel<<<(unsigned)((np + 255) / 256), 256, 0, st>>>(c->n, np, (int)p, nc, c->dX, c->dZ + c0 * np,
-                                                                  kind == COCONS_ML ? c->dTheta + 6 * p : nullptr,
-                                                                  rhs);
+    launch_residual(c->n, np, (int)p, nc, c->dX, c->dZ + c0 * np, kind == COCONS_ML ? c->dTheta + 6 * p : nullptr, rhs,
+                    st);
     forward_solve_ws(c->dA, np, np, c->ws, rhs, np, nc, st);
     const int k = qx + nc;
     launch_gram(c->dRhs, c->n, np, k, c->dGram, st);
@@ -699,6 +879,7 @@ static int n2ll_impl(cocons_ctx* c, int kind, const double* theta6, const double
 
 int cocons_n2ll(cocons_ctx* c, int kind, const double* theta6, const double* limits, const double* mean_p,
                 double* logdet, double* quad, double* logdet_w, int* rank_x) {
+  if (int rc_ = refuse_tiled(c, "n2ll")) return rc_;
   return n2ll_impl(c, kind, theta6, limits, mean_p, logdet, quad, logdet_w, rank_x, false);
 }
 
@@ -725,14 +906,8 @@ static int check_pattern(const char* who, const int32_t* colindices, const int32
   return 0;
 }
 
-int cocons_ctx_set_taper(cocons_ctx* c, const int32_t* colindices, const int32_t* rowpointers,
-                         const double* taper_entries, int64_t nnz) {
-  if (!c || !taper_entries) {
-    set_error("ctx_set_taper: bad argument");
-    return COCONS_ERR_ARG;
-  }
-  int rc = check_pattern("ctx_set_taper", colindices, rowpointers, c->n, c->n, nnz);
-  if (rc) return rc;
+static int attach_taper(cocons_ctx* c, const int32_t* colindices, const int32_t* rowpointers,
+                        const double* taper_entries, int64_t nnz) {
   cudaSetDevice(c->device);
   cudaFree(c->dTapCol), cudaFree(c->dTapRow), cudaFree(c->dTap);
   c->dTapCol = c->dTapRow = nullptr, c->dTap = nullptr, c->tap_nnz = 0;
@@ -752,12 +927,109 @@ int cocons_ctx_set_taper(cocons_ctx* c, const int32_t* colindices, const int32_t
   return 0;
 }
 
+int cocons_ctx_set_taper(cocons_ctx* c, const int32_t* colindices, const int32_t* rowpointers,
+                         const double* taper_entries, int64_t nnz) {
+  if (!c || !taper_entries) {
+    set_error("ctx_set_taper: bad argument");
+    return COCONS_ERR_ARG;
+  }
+  int rc = refuse_tiled(c, "ctx_set_taper");
+  if (rc || (rc = check_pattern("ctx_set_taper", colindices, rowpointers, c->n, c->n, nnz))) return rc;
+  return attach_taper(c, colindices, rowpointers, taper_entries, nnz);
+}
+
+int cocons_ctx_create_taper_tiled(int device, int64_t n, int64_t p, int64_t r, const double* locs, const double* X,
+                                  const double* z, const int32_t* colindices, const int32_t* rowpointers,
+                                  const double* taper_entries, int64_t nnz, void* stream, cocons_ctx** out) {
+  if (!out || n <= 0 || p <= 0 || r < 0 || r > kTile || !locs || !X || (r > 0 && !z) || !taper_entries) {
+    set_error("ctx_create_taper_tiled: bad argument (r must be in 0..%d)", kTile);
+    return COCONS_ERR_ARG;
+  }
+  *out = nullptr;
+  int rc = check_pattern("ctx_create_taper_tiled", colindices, rowpointers, n, n, nnz);
+  if (rc) return rc;
+  cocons_ctx* c = nullptr;
+  if ((rc = ctx_create(device, n, p, r, locs, X, z, stream, true, &c))) return rc;
+  if ((rc = attach_taper(c, colindices, rowpointers, taper_entries, nnz))) {
+    cocons_ctx_destroy(c);
+    return rc;
+  }
+  tile_symbolic(c, colindices, rowpointers);
+  std::vector<int64_t> tiles((size_t)(c->T + 1 + 2 * c->nstored + c->T)), maps;
+  for (int64_t J = 0; J < c->T; ++J) {
+    tiles[(size_t)(c->T + 1 + 2 * c->nstored + J)] = c->ldp[(size_t)J];
+    for (int64_t k = c->colptr[(size_t)J]; k < c->colptr[(size_t)J + 1]; ++k)
+      tiles[(size_t)(c->T + 1 + c->nstored + k)] = c->base[(size_t)J] + (k - c->colptr[(size_t)J]) * kTile;
+  }
+  std::copy(c->colptr.begin(), c->colptr.end(), tiles.begin());
+  std::copy(c->rows.begin(), c->rows.end(), tiles.begin() + c->T + 1);
+  tile_maps(c, &maps);
+  c->rhs_k = std::max<int64_t>(16, round_up(r, 16));
+  std::vector<double> negi((size_t)kTile * c->rhs_k, 0.0);
+  for (int64_t k = 0; k < c->rhs_k; ++k) negi[(size_t)(k * kTile + k)] = -1.0;
+  cudaFree(c->dRhs), c->dRhs = nullptr;
+  CTX_TRY(cudaMalloc(&c->dRhs, sizeof(double) * c->n_pad * c->rhs_k));
+  CTX_TRY(cudaMalloc(&c->dPool, sizeof(double) * c->pool_elems));
+  CTX_TRY(cudaMalloc(&c->dTiles, sizeof(int64_t) * tiles.size()));
+  CTX_TRY(cudaMalloc(&c->dMaps, sizeof(int64_t) * maps.size()));
+  CTX_TRY(cudaMalloc(&c->dNegI, sizeof(double) * negi.size()));
+  CTX_TRY(cudaMalloc(&c->dLogPart, sizeof(double) * c->T));
+  CTX_TRY(cudaMemcpy(c->dTiles, tiles.data(), sizeof(int64_t) * tiles.size(), cudaMemcpyHostToDevice));
+  CTX_TRY(cudaMemcpy(c->dMaps, maps.data(), sizeof(int64_t) * maps.size(), cudaMemcpyHostToDevice));
+  CTX_TRY(cudaMemcpy(c->dNegI, negi.data(), sizeof(double) * negi.size(), cudaMemcpyHostToDevice));
+  *out = c;
+  return 0;
+}
+
+int cocons_ctx_tile_stats(cocons_ctx* c, int64_t* stats4) {
+  if (!c || !stats4) {
+    set_error("ctx_tile_stats: bad argument");
+    return COCONS_ERR_ARG;
+  }
+  if (!c->tiled) {
+    set_error("ctx_tile_stats: the context is dense (tile statistics exist for cocons_ctx_create_taper_tiled)");
+    return COCONS_ERR_STATE;
+  }
+  stats4[0] = c->T, stats4[1] = c->nstored, stats4[2] = c->nfill, stats4[3] = c->tile_products;
+  return 0;
+}
+
+// GetNeg2loglikelihoodTaper on a tiled context: the factorisation already carried the substitution (tiled_factor);
+// what is left is reading the Gram block's diagonal and the diagonal tiles' log-determinants (summed in tile order)
+static int n2ll_tiled(cocons_ctx* c, const double* theta6, const double* limits, const double* mean_p, double* logdet,
+                      double* quad) {
+  if (!theta6 || !limits || !logdet || !quad || c->r <= 0) {
+    set_error("n2ll_taper: bad argument");
+    return COCONS_ERR_ARG;
+  }
+  cudaSetDevice(c->device);
+  int rc = assemble_and_factor(c, COCONS_PAR_DIFF, theta6, limits, mean_p, true);
+  if (rc) return rc;
+  cudaStream_t st = c->stream;
+  std::vector<double> part((size_t)c->T), g((size_t)kTile * c->r);
+  COCONS_CUDA_TRY(cudaMemcpyAsync(part.data(), c->dLogPart, sizeof(double) * c->T, cudaMemcpyDeviceToHost, st));
+  COCONS_CUDA_TRY(cudaMemcpyAsync(g.data(), c->dPool + c->g_off, sizeof(double) * g.size(), cudaMemcpyDeviceToHost,
+                                  st));
+  COCONS_CUDA_TRY(cudaMemcpyAsync(c->hInfo, c->ws.info, sizeof(int), cudaMemcpyDeviceToHost, st));
+  COCONS_CUDA_TRY(cudaEventRecord(c->ev[3], st));
+  COCONS_CUDA_TRY(cudaStreamSynchronize(st));
+  finish_timings(c);
+  if (*c->hInfo != 0) return *c->hInfo;  // > 0: not positive definite
+  double ld = 0.0;
+  for (double v : part) ld += v;
+  *logdet = ld;
+  for (int64_t j = 0; j < c->r; ++j) quad[j] = -g[(size_t)(j * kTile + j)];
+  c->factor_valid = true;
+  return 0;
+}
+
 int cocons_n2ll_taper(cocons_ctx* c, const double* theta6, const double* limits, const double* mean_p,
                       double* logdet, double* quad) {
   if (!c || !c->dTap) {
     set_error("n2ll_taper: cocons_ctx_set_taper first");
     return COCONS_ERR_STATE;
   }
+  if (c->tiled) return n2ll_tiled(c, theta6, limits, mean_p, logdet, quad);
   return n2ll_impl(c, COCONS_ML, theta6, limits, mean_p, logdet, quad, nullptr, nullptr, true);
 }
 
@@ -840,6 +1112,7 @@ int cocons_cov_rns_taper_pred(int64_t n, int64_t m, int64_t p, const double* loc
 }
 
 int cocons_profile_betas(cocons_ctx* c, int kind, double* betas) {
+  if (int rc_ = refuse_tiled(c, "profile_betas")) return rc_;
   if (!c || !betas || (kind != COCONS_PROFILE && kind != COCONS_REML)) {
     set_error("profile_betas: bad argument");
     return COCONS_ERR_ARG;
@@ -897,6 +1170,7 @@ int cocons_profile_betas(cocons_ctx* c, int kind, double* betas) {
 }
 
 int cocons_factor(cocons_ctx* c, int par, const double* theta6, const double* limits) {
+  if (int rc_ = refuse_tiled(c, "factor")) return rc_;
   if (!c || !theta6 || (par != COCONS_PAR_DIFF && par != COCONS_PAR_CLASSIC) || (par == COCONS_PAR_DIFF && !limits)) {
     set_error("factor: bad argument");
     return COCONS_ERR_ARG;
@@ -997,6 +1271,7 @@ static int refresh_table_for_pred(cocons_ctx* c) {
 
 static int predict_impl(cocons_ctx* c, int64_t m, const double* locs_pred, const double* Xp, const double* resid,
                         double* stochastic, double* explained, const TaperPred* tp) {
+  if (int rc_ = refuse_tiled(c, "predict")) return rc_;
   if (!c || m <= 0 || !locs_pred || !Xp || !resid || !stochastic) {
     set_error("predict: bad argument");
     return COCONS_ERR_ARG;
@@ -1102,6 +1377,7 @@ int cocons_factor_taper(cocons_ctx* c, const double* theta6, const double* limit
 int cocons_predict_taper(cocons_ctx* c, int64_t m, const double* locs_pred, const double* Xp,
                          const int32_t* colindices, const int32_t* rowpointers, const double* taper_entries,
                          int64_t nnz, const double* resid, double* stochastic, double* explained) {
+  if (int rc_ = refuse_tiled(c, "predict_taper")) return rc_;
   if (!c || m <= 0 || !taper_entries) {
     set_error("predict_taper: bad argument");
     return COCONS_ERR_ARG;
@@ -1122,6 +1398,7 @@ int cocons_predict_taper(cocons_ctx* c, int64_t m, const double* locs_pred, cons
 }
 
 int cocons_sim(cocons_ctx* c, int64_t k, const double* eps, double* out) {
+  if (int rc_ = refuse_tiled(c, "sim")) return rc_;
   if (!c || k <= 0 || !eps || !out) {
     set_error("sim: bad argument");
     return COCONS_ERR_ARG;
@@ -1161,6 +1438,7 @@ int cocons_sim(cocons_ctx* c, int64_t k, const double* eps, double* out) {
 
 int cocons_sim_cond(cocons_ctx* c, int64_t m, const double* locs_pred, const double* Xp, int64_t k, const double* eps,
                     double* out) {
+  if (int rc_ = refuse_tiled(c, "sim_cond")) return rc_;
   if (!c || m <= 0 || k <= 0 || !locs_pred || !Xp || !eps || !out) {
     set_error("sim_cond: bad argument");
     return COCONS_ERR_ARG;
@@ -1243,6 +1521,23 @@ int cocons_ctx_get_factor(cocons_ctx* c, double* L, int64_t* perm) {
   }
   cudaSetDevice(c->device);
   const int64_t np = c->n_pad, n = c->n;
+  if (c->tiled) {  // expand the stored tiles (meant for small n: the whole pool goes through the host)
+    std::vector<double> pool((size_t)c->pool_elems);
+    COCONS_CUDA_TRY(cudaMemcpy(pool.data(), c->dPool, sizeof(double) * pool.size(), cudaMemcpyDeviceToHost));
+    std::fill(L, L + (size_t)n * n, 0.0);
+    for (int64_t J = 0; J < c->T; ++J)
+      for (int64_t k = c->colptr[(size_t)J]; k < c->colptr[(size_t)J + 1]; ++k) {
+        const int64_t I = c->rows[(size_t)k];
+        const double* t = pool.data() + c->base[(size_t)J] + (k - c->colptr[(size_t)J]) * kTile;
+        for (int64_t jj = 0; jj < kTile && J * kTile + jj < n; ++jj)
+          for (int64_t ii = 0; ii < kTile && I * kTile + ii < n; ++ii)
+            if (I * kTile + ii >= J * kTile + jj)
+              L[(size_t)(J * kTile + jj) * n + I * kTile + ii] = t[jj * c->ldp[(size_t)J] + ii];
+      }
+    if (perm)
+      for (int64_t s = 0; s < n; ++s) perm[s] = c->perm[(size_t)s];
+    return 0;
+  }
   COCONS_CUDA_TRY(cudaMemcpy2D(L, sizeof(double) * n, c->dA, sizeof(double) * np, sizeof(double) * n, n,
                                cudaMemcpyDeviceToHost));
   for (int64_t j = 0; j < n; ++j)
@@ -1273,6 +1568,19 @@ int cocons_ctx_factor_rows(cocons_ctx* c, const int64_t* sites, int64_t m, doubl
     const int64_t i = inv[(size_t)sites[a]];
     pos[a] = i;
     double* out = rows + (size_t)a * n;
+    if (c->tiled) {  // row i crosses the stored tiles (I, J) of its tile row, J <= I
+      const int64_t I = i / kTile;
+      std::fill(out, out + n, 0.0);
+      for (int64_t J = 0; J <= I; ++J) {
+        const int64_t pos = tile_pos(c, I, J);
+        if (pos < 0) continue;
+        const int64_t w = std::min<int64_t>(kTile, std::min(i + 1, n) - J * kTile);
+        COCONS_CUDA_TRY(cudaMemcpy2D(out + J * kTile, sizeof(double), c->dPool + c->base[(size_t)J] + pos * kTile + i % kTile,
+                                     sizeof(double) * c->ldp[(size_t)J], sizeof(double), (size_t)w,
+                                     cudaMemcpyDeviceToHost));
+      }
+      continue;
+    }
     // row i of the column-major factor: one element per column, columns 0..i
     COCONS_CUDA_TRY(cudaMemcpy2D(out, sizeof(double), c->dA + i, sizeof(double) * np, sizeof(double), (size_t)(i + 1),
                                  cudaMemcpyDeviceToHost));
@@ -1303,12 +1611,14 @@ int cocons_ctx_timings(cocons_ctx* c, double* ms4) {
 }
 
 int cocons_ctx_debug_checksums(cocons_ctx* c, double* out2) {
+  if (int rc_ = refuse_tiled(c, "ctx_debug_checksums")) return rc_;
   if (!c || !out2) return COCONS_ERR_ARG;
   out2[0] = c->check[0], out2[1] = c->check[1];
   return 0;
 }
 
 int cocons_ctx_kernel_timing(cocons_ctx* c, double* ms, double* flops) {
+  if (int rc_ = refuse_tiled(c, "ctx_kernel_timing")) return rc_;
   if (!c || !ms || !flops) return COCONS_ERR_ARG;
   *ms = c->kernel_ms, *flops = c->kernel_flops;
   return 0;

@@ -35,6 +35,7 @@ namespace cocons {
 #endif
 constexpr int GBM = 128, GBK = 16, GSTAGES = 4;
 constexpr int GLDA = GBM + 4;  // padded leading dimension of a shared k-row (== 4 mod 16: conflict-free LDS.128)
+constexpr int kGemmMapped = 2;  // gemm_nt_tma_kernel's tile-mapped C -= A B^T (tiled factor, csrc/capi.cu)
 
 template <int BN, int NU = 2>
 struct GemmCfg {
@@ -225,6 +226,11 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
                : "memory");
 }
 
+// ASSIGN 0: C -= A B^T; 1: C = A B^T; 2 (kGemmMapped): C -= A B^T with every 128 x 128 block of C looked up in a
+// tile map, so that one launch updates tiles scattered over the panels of a tiled factor.  In that mode `ldc`
+// carries the device address of the map, int64: [pairs: element offset of the target block from C][128-column
+// blocks: leading dimension of the target], pair (bi, c) numbered bi (bi + 1) / 2 + c with lower_only, bi * nj / 2 + c
+// without (c = the 128-column block of the CTA's tile).
 template <int BN, int NU, int ASSIGN>
 __global__ void __launch_bounds__(GemmCfg<BN, NU>::kThreads, GemmCfg<BN, NU>::kMinBlocks)
     gemm_nt_tma_kernel(int ni, int nj, int64_t K, const double* A, int64_t lda, const double* B, int64_t ldb,
@@ -279,8 +285,18 @@ __global__ void __launch_bounds__(GemmCfg<BN, NU>::kThreads, GemmCfg<BN, NU>::kM
 #pragma unroll
     for (int b = 0; b < 2 * NU; ++b) acc[a][b][0] = acc[a][b][1] = 0.0;
 
+  if (ASSIGN == kGemmMapped) {  // C and ldc of the target block (BN = 64: two CTA tiles per 128-column block)
+    static_assert(ASSIGN != kGemmMapped || BN == 64, "the tile map is for 128 x 64 CTA tiles");
+    const int64_t* map = reinterpret_cast<const int64_t*>(ldc);
+    const int c = bj / 2;
+    const int64_t pair = lower_only ? (int64_t)bi * (bi + 1) / 2 + c : (int64_t)bi * (nj / 2) + c;
+    const int64_t npairs = lower_only ? (int64_t)ni * (ni + 1) / 2 : (int64_t)ni * (nj / 2);
+    ldc = map[npairs + c];
+    // shifted so that the addressing below, C + bj BN ldc + bi GBM, lands on the target block
+    C += map[pair] + (int64_t)(bj & 1) * BN * ldc - (int64_t)bj * BN * ldc - (int64_t)bi * GBM;
+  }
 #ifndef COCONS_GEMM_NO_PREFETCH
-  if (!ASSIGN) {  // pull the C tile towards L2 while the main loop runs
+  if (ASSIGN != 1) {  // pull the C tile towards L2 while the main loop runs
     const double* Cp = C + (int64_t)bj * BN * ldc + (int64_t)bi * GBM;
     for (int l = tid; l < BN * 8; l += Cfg::kThreads)
       asm volatile("prefetch.global.L2 [%0];" ::"l"(Cp + (int64_t)(l >> 3) * ldc + (l & 7) * 16));
@@ -349,7 +365,7 @@ __global__ void __launch_bounds__(GemmCfg<BN, NU>::kThreads, GemmCfg<BN, NU>::kM
       const int r0 = iw + 16 * u + 4 * c4;
       double2* p = reinterpret_cast<double2*>(Cg + (int64_t)j * ldc + r0);
       double2 lo, hi;
-      if (ASSIGN) {
+      if (ASSIGN == 1) {
         lo.x = acc[a][2 * u][0];
         lo.y = acc[a][2 * u + 1][0];
         hi.x = acc[a][2 * u][1];
@@ -364,7 +380,7 @@ __global__ void __launch_bounds__(GemmCfg<BN, NU>::kThreads, GemmCfg<BN, NU>::kM
         hi.x -= acc[a][2 * u][1];
         hi.y -= acc[a][2 * u + 1][1];
       }
-      if (ASSIGN) {
+      if (ASSIGN == 1) {
         p[0] = lo;
         p[1] = hi;
       } else {
@@ -385,6 +401,16 @@ static int debug_sync_mode() {
   return m;
 }
 
+// 128 x 64 tiles: C -= A B^T (EPI = 0) or the tile-mapped variant (EPI = kGemmMapped)
+template <int EPI>
+static void launch_gemm_64(int ni, int nj, int64_t K, const double* A, int64_t lda, const double* B, int64_t ldb,
+                           double* C, int64_t ldc, int lower_only, cudaStream_t st) {
+  const int64_t tiles = total_tiles<2>(ni, nj, lower_only);
+  gemm_nt_tma_kernel<64, 2, EPI><<<(unsigned)tiles, GemmCfg<64, 2>::kThreads, GemmCfg<64, 2>::kSmemBytes + 64, st>>>(
+      ni, nj, K, A, lda, B, ldb, C, ldc, lower_only);
+}
+
+// mode 2: as mode 0 with C addressed through a tile map whose device address is passed as ldc (see the kernel)
 void launch_gemm_nt(int mode, int64_t M, int64_t N, int64_t K, const double* A, int64_t lda, const double* B,
                     int64_t ldb, double* C, int64_t ldc, int lower_only, cudaStream_t st) {
   if (M <= 0 || N <= 0 || K <= 0) return;
@@ -397,6 +423,8 @@ void launch_gemm_nt(int mode, int64_t M, int64_t N, int64_t K, const double* A, 
                          GemmCfg<64, 2>::kSmemBytes + 64);
     cudaFuncSetAttribute(gemm_nt_tma_kernel<128, 2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                          GemmCfg<128, 2>::kSmemBytes + 64);
+    cudaFuncSetAttribute(gemm_nt_tma_kernel<64, 2, kGemmMapped>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                         GemmCfg<64, 2>::kSmemBytes + 64);
     attr_done[dev] = true;
   }
   const int ni = (int)(M / GBM);
@@ -406,11 +434,10 @@ void launch_gemm_nt(int mode, int64_t M, int64_t N, int64_t K, const double* A, 
     const int64_t tiles = total_tiles<1>(ni, nj, lower_only);
     gemm_nt_tma_kernel<128, 2, 1><<<(unsigned)tiles, GemmCfg<128, 2>::kThreads, GemmCfg<128, 2>::kSmemBytes + 64, st>>>(
         ni, nj, K, A, lda, B, ldb, C, ldc, lower_only);
+  } else if (mode == kGemmMapped) {
+    launch_gemm_64<kGemmMapped>(ni, (int)(N / 64), K, A, lda, B, ldb, C, ldc, lower_only, st);
   } else {
-    const int nj = (int)(N / 64);
-    const int64_t tiles = total_tiles<2>(ni, nj, lower_only);
-    gemm_nt_tma_kernel<64, 2, 0><<<(unsigned)tiles, GemmCfg<64, 2>::kThreads, GemmCfg<64, 2>::kSmemBytes + 64, st>>>(
-        ni, nj, K, A, lda, B, ldb, C, ldc, lower_only);
+    launch_gemm_64<0>(ni, (int)(N / 64), K, A, lda, B, ldb, C, ldc, lower_only, st);
   }
 }
 

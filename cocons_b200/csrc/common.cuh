@@ -88,16 +88,21 @@ struct TaperTable {
 void launch_taper_site_stage(int64_t n, int p, const double* dX, int64_t ldx, const double* dlocs, int64_t ldl,
                              const double* dtheta6, double lim0, double lim1, int mode, int pred_rows, TaperTable T,
                              cudaStream_t st);
-enum TaperSinkKind { TS_VECTOR = 0, TS_LOWER = 1, TS_ROWS = 2 };
+enum TaperSinkKind { TS_VECTOR = 0, TS_LOWER = 1, TS_ROWS = 2, TS_TILED = 3 };
 struct TaperSink {
   int kind;
   double* out;          // TS_VECTOR: nnz values in pattern order
-  const double* taper;  // TS_LOWER / TS_ROWS: taper values on the pattern, multiplied in
+  const double* taper;  // TS_LOWER / TS_ROWS / TS_TILED: taper values on the pattern, multiplied in
   const int* inv;       // caller index -> position in the context's ordering
-  double* A;            // dense sink
-  int64_t ld;
-  int64_t row0;         // TS_ROWS: first pattern row of the block
+  double* A;            // dense sink; TS_TILED: the tile pool
+  int64_t ld;           // TS_TILED: number of tile columns T
+  int64_t row0;         // TS_ROWS: first pattern row of the block; TS_TILED: number of stored tiles
+  // TS_TILED: the tile map, int64 [T + 1 column starts][stored tiles: tile row][stored tiles: element offset of the
+  // tile in the pool][T: leading dimension of column panel J]; the rows of a column are sorted, diagonal first
+  const int64_t* tiles;
 };
+// the tiled sink runs in instantiations of taper_entries_kernel<mode + kTaperTiled> of their own
+constexpr int kTaperTiled = 8;
 // entries [e0, e0 + count) of the pattern (nrows rows)
 void launch_taper_entries(int64_t e0, int64_t count, int64_t nrows, const int* dcol, const int* drow, TaperTable R,
                           TaperTable C, int square, int mode, double nu_fixed, TaperSink S, cudaStream_t st);
@@ -126,6 +131,9 @@ void factor_panel(double* A, int64_t n_pad, int64_t ld, const CholWorkspace& ws,
                   cudaStream_t st);
 int chol_factor(double* A, int64_t n_pad, int64_t ld, CholWorkspace ws, cudaStream_t st);
 int chol_outer(int64_t n_pad);  // tiles per outer panel of chol_factor
+// diagonal tile: Cholesky in place (leading dimension ld) and its explicit inverse into Winv (128 x 128); the first
+// failing pivot sets *info = first_index + its 1-based order
+void launch_potrf_tile(double* A, int64_t ld, double* Winv, int* info, int first_index, cudaStream_t st);
 void launch_gemm_nt(int mode, int64_t M, int64_t N, int64_t K, const double* A, int64_t lda, const double* B,
                     int64_t ldb, double* C, int64_t ldc, int lower_only, cudaStream_t st);
 

@@ -103,29 +103,48 @@ __device__ __forceinline__ int64_t taper_row_of(const int* __restrict__ rowpoint
 //   TS_LOWER    A[max(si,sj) + min(si,sj) ld] = taper[e] value  for the entries with i >= j, where
 //               si = inv[i] is the site's position in the context's (Morton) ordering
 //   TS_ROWS     A[(i - row0) + inv[j] ld] = taper[e] value      (a block of prediction rows x all sites)
+//   TS_TILED    as TS_LOWER, into the tile pool of a tiled context: tile (hi / 128, lo / 128) is found by a binary
+//               search over the stored tile rows of column lo / 128 (TaperSink::tiles).  Only the instantiations
+//               MODE = smoothness mode + kTaperTiled take this sink; the others compile exactly as before.
 template <int MODE>
 __global__ void __launch_bounds__(256) taper_entries_kernel(int64_t e0, int64_t count, int64_t nrows,
                                                             const int* __restrict__ colindices,
                                                             const int* __restrict__ rowpointers, TaperTable R,
                                                             TaperTable C, int square, double nu_fixed, TaperSink S) {
+  constexpr bool kTiled = MODE >= kTaperTiled;
+  constexpr int kMode = kTiled ? MODE - kTaperTiled : MODE;
   const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= count) return;
   const int64_t e = e0 + t;
   const int64_t i = taper_row_of(rowpointers, nrows, e);
   const int64_t j = (int64_t)colindices[e] - 1;
-  if (S.kind == TS_LOWER && i < j) return;  // the dense sink keeps the caller's lower triangle
+  if ((kTiled || S.kind == TS_LOWER) && i < j) return;  // the dense sink keeps the caller's lower triangle
   // table positions: the context's ordering for resident sites, block-local for prediction rows
-  const int64_t si = (S.kind == TS_LOWER) ? S.inv[i] : (S.kind == TS_ROWS ? i - S.row0 : i);
-  const int64_t sj = (S.kind == TS_VECTOR) ? j : S.inv[j];
+  const int64_t si = (kTiled || S.kind == TS_LOWER) ? S.inv[i] : (S.kind == TS_ROWS ? i - S.row0 : i);
+  const int64_t sj = (!kTiled && S.kind == TS_VECTOR) ? j : S.inv[j];
   const double xi = R.f(TF_X)[si], yi = R.f(TF_Y)[si];
   const double xj = C.f(TF_X)[sj], yj = C.f(TF_Y)[sj];
   double v = 0.0;
   bool same = square ? (i == j) : (xi == xj && yi == yj);
   if (!same)
-    v = taper_pair<MODE>(R.f(TF_R)[si], R.f(TF_SIG)[si], R.f(TF_NU)[si], C.f(TF_R)[sj], C.f(TF_SIG)[sj],
+    v = taper_pair<kMode>(R.f(TF_R)[si], R.f(TF_SIG)[si], R.f(TF_NU)[si], C.f(TF_R)[sj], C.f(TF_SIG)[sj],
                          C.f(TF_NU)[sj], __dsub_rn(xi, xj), __dsub_rn(yi, yj), nu_fixed, same);
   if (same) v = R.f(TF_DV)[si];
-  if (S.kind == TS_VECTOR) {
+  if (kTiled) {
+    const int64_t hi = si > sj ? si : sj, lo = si > sj ? sj : si;
+    const int64_t I = hi / kTile, J = lo / kTile, T = S.ld, nst = S.row0;
+    const int64_t* rows = S.tiles + T + 1;
+    int64_t a = S.tiles[J], b = S.tiles[J + 1] - 1;  // every tile of the pattern is stored: rows[a..b] holds I
+    while (a < b) {
+      const int64_t mid = (a + b) >> 1;
+      if (rows[mid] < I)
+        a = mid + 1;
+      else
+        b = mid;
+    }
+    const int64_t ld = S.tiles[T + 1 + 2 * nst + J];
+    S.A[rows[nst + a] + (lo % kTile) * ld + hi % kTile] = __dmul_rn(S.taper[e], v);
+  } else if (S.kind == TS_VECTOR) {
     S.out[e] = v;
   } else if (S.kind == TS_LOWER) {
     const int64_t hi = si > sj ? si : sj, lo = si > sj ? sj : si;
@@ -156,11 +175,16 @@ void launch_taper_entries(int64_t e0, int64_t count, int64_t nrows, const int* d
   note_launch();
 #define COCONS_TAPER_LAUNCH(M) \
   taper_entries_kernel<M><<<blocks, 256, 0, st>>>(e0, count, nrows, dcol, drow, R, C, square, nu_fixed, S)
-  switch (mode) {
+  switch (mode + (S.kind == TS_TILED ? kTaperTiled : 0)) {
     case SM_HALF: COCONS_TAPER_LAUNCH(SM_HALF); break;
     case SM_THREEHALF: COCONS_TAPER_LAUNCH(SM_THREEHALF); break;
     case SM_FIVEHALF: COCONS_TAPER_LAUNCH(SM_FIVEHALF); break;
     case SM_DEGENERATE: COCONS_TAPER_LAUNCH(SM_DEGENERATE); break;
+    case SM_HALF + kTaperTiled: COCONS_TAPER_LAUNCH(SM_HALF + kTaperTiled); break;
+    case SM_THREEHALF + kTaperTiled: COCONS_TAPER_LAUNCH(SM_THREEHALF + kTaperTiled); break;
+    case SM_FIVEHALF + kTaperTiled: COCONS_TAPER_LAUNCH(SM_FIVEHALF + kTaperTiled); break;
+    case SM_DEGENERATE + kTaperTiled: COCONS_TAPER_LAUNCH(SM_DEGENERATE + kTaperTiled); break;
+    case SM_GENERAL + kTaperTiled: COCONS_TAPER_LAUNCH(SM_GENERAL + kTaperTiled); break;
     default: COCONS_TAPER_LAUNCH(SM_GENERAL); break;
   }
 #undef COCONS_TAPER_LAUNCH

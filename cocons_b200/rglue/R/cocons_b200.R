@@ -90,7 +90,12 @@ GetNeg2loglikelihoodREML <- function(theta, par.pos, locs, x_covariates, x_betas
 # ---- tapered objectives (R/neg2loglikelihood.R:20-108) -----------------------------------
 # The tapered matrix is factored densely on the device instead of by spam's sparse Cholesky, so `cholS`
 # is accepted and unused.  A context per call keeps the closures drop-in; cocoOptim's sparse branch
-# (R/optim.R:480-531) can build it once, attach the taper once and pass it through `ctx`.
+# (R/optim.R:480-531) can build it once, attach the taper once and pass it through `ctx`.  For large n it can
+# build a tiled context instead, which stores only the tiles of the factor that can be nonzero (n = 200 000 fits
+# one GPU) and is passed through `ctx` the same way:
+#   ctx <- .Call(`_cocons_ctx_new_taper_tiled`, locs, as.matrix(x_covariates), as.matrix(z),
+#                ref_taper@colindices, ref_taper@rowpointers, ref_taper@entries, 0L)
+#   on.exit(.Call(`_cocons_ctx_free`, ctx))
 .cocons.n2ll.taper.device <- function(theta_list, ref_taper, locs, x_covariates, smooth.limits, z, ctx = NULL) {
   tryCatch({
     if (is.null(ctx)) {

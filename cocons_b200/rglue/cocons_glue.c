@@ -357,6 +357,29 @@ SEXP _cocons_ctx_set_taper(SEXP ptr, SEXP colS, SEXP rowS, SEXP entriesS) {
   return R_NilValue;
 }
 
+/* a context for the tapered model only, with ref_taper's pattern fixed: only the tiles of the Cholesky factor that can
+ * be nonzero are stored (cocons_ctx_create_taper_tiled).  Same external-pointer class as _cocons_ctx_new, so
+ * _cocons_ctx_n2ll_taper / _cocons_ctx_factor_taper / _cocons_ctx_set_z / _cocons_ctx_free take it as they are */
+SEXP _cocons_ctx_new_taper_tiled(SEXP locsS, SEXP xS, SEXP zS, SEXP colS, SEXP rowS, SEXP entriesS, SEXP deviceS) {
+  SEXP locs = PROTECT(as_real(locsS)), x = PROTECT(as_real(xS)), z = PROTECT(as_real(zS));
+  SEXP col = PROTECT(as_int(colS)), row = PROTECT(as_int(rowS)), ent = PROTECT(as_real(entriesS));
+  check_sites("ctx_new_taper_tiled", locs, x);
+  need(rows_of(z) == Rf_nrows(locs), "ctx_new_taper_tiled", "z must have nrow(locs) rows");
+  const int n = Rf_nrows(locs), p = Rf_ncols(x), r = Rf_isMatrix(z) ? Rf_ncols(z) : 1;
+  need(r <= 128, "ctx_new_taper_tiled", "z may have at most 128 columns");
+  need(XLENGTH(ent) == XLENGTH(col), "ctx_new_taper_tiled", "entries and colindices differ in length");
+  need(LENGTH(row) == n + 1, "ctx_new_taper_tiled", "rowpointers must have nrow(locs) + 1 elements");
+  cocons_ctx* c = NULL;
+  int rc = cocons_ctx_create_taper_tiled(Rf_asInteger(deviceS), n, p, r, REAL(locs), REAL(x), REAL(z), INTEGER(col),
+                                         INTEGER(row), REAL(ent), XLENGTH(col), NULL, &c);
+  UNPROTECT(6);
+  raise(rc);
+  SEXP ptr = PROTECT(R_MakeExternalPtr(c, R_NilValue, R_NilValue));
+  R_RegisterCFinalizerEx(ptr, ctx_finalizer, TRUE);
+  UNPROTECT(1);
+  return ptr;
+}
+
 /* c(status, logdet, quad...) of the tapered model (R/neg2loglikelihood.R:20-108) */
 SEXP _cocons_ctx_n2ll_taper(SEXP ptr, SEXP thetaS, SEXP pS, SEXP rS, SEXP limS, SEXP meanS) {
   const ctx_view v = view_of(ptr);
@@ -455,6 +478,7 @@ static const R_CallMethodDef CallEntries[] = {
     {"_cocons_ctx_profile_betas", (DL_FUNC)&_cocons_ctx_profile_betas, 3},
     {"_cocons_ctx_predict", (DL_FUNC)&_cocons_ctx_predict, 4},
     {"_cocons_ctx_set_taper", (DL_FUNC)&_cocons_ctx_set_taper, 4},
+    {"_cocons_ctx_new_taper_tiled", (DL_FUNC)&_cocons_ctx_new_taper_tiled, 7},
     {"_cocons_ctx_n2ll_taper", (DL_FUNC)&_cocons_ctx_n2ll_taper, 6},
     {"_cocons_ctx_factor_taper", (DL_FUNC)&_cocons_ctx_factor_taper, 4},
     {"_cocons_ctx_predict_taper", (DL_FUNC)&_cocons_ctx_predict_taper, 7},

@@ -135,6 +135,22 @@ int cocons_cov_rns_taper_pred(int64_t n, int64_t m, int64_t p, const double* loc
 int cocons_ctx_set_taper(cocons_ctx* ctx, const int32_t* colindices, const int32_t* rowpointers,
                          const double* taper_entries, int64_t nnz);
 
+/* A context for the tapered model only, with the pattern fixed at creation: only the tiles of L that can be nonzero
+ * (pattern + fill, Morton order) are stored, so n is bounded by the factor's fill, not by n_pad^2.  The pattern and
+ * taper entries are those of cocons_ctx_set_taper; 0 <= r <= 128.  On such a context cocons_n2ll_taper,
+ * cocons_factor_taper, cocons_ctx_get_factor (dense expansion, for small n), cocons_ctx_factor_rows,
+ * cocons_ctx_set_z, cocons_ctx_dims, cocons_ctx_timings and cocons_ctx_destroy work as on a dense context; every
+ * other context entry returns COCONS_ERR_STATE.  The factor differs from the dense path's in the last bits only. */
+int cocons_ctx_create_taper_tiled(int device, int64_t n, int64_t p, int64_t r, const double* locs,
+                                  const double* x_covariates, const double* z, const int32_t* colindices,
+                                  const int32_t* rowpointers, const double* taper_entries, int64_t nnz,
+                                  void* stream, cocons_ctx** out);
+/* {tile columns, stored tiles, stored tiles outside the pattern (fill), tile products per factorisation} of a tiled
+ * context: lower 128 x 128 tiles, diagonal included; a tile product is one 128 x 128 x 128 block of the trailing
+ * updates (sum over tile columns of m (m + 1) / 2, m = stored tiles below the diagonal).  COCONS_ERR_STATE on a dense
+ * context. */
+int cocons_ctx_tile_stats(cocons_ctx* ctx, int64_t* stats4);
+
 /* GetNeg2loglikelihoodTaper / ...TaperProfile (R/neg2loglikelihood.R:20-108):
  * taper * cov_rns_taper on the pattern -> Cholesky -> log-determinant and
  * |R^-T (z - X mean)|^2 per column of z.  Where the reference updates spam's
