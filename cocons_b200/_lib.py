@@ -83,6 +83,7 @@ SIGNATURES = {
     "cocons_dist_reduce_local": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vp, _vp]),
     "cocons_dist_perm": (ctypes.c_int, [_vp, _lp]),
     "cocons_bench_syrk": (ctypes.c_int, [ctypes.c_int, _i64, _i64, ctypes.c_int, _dp]),
+    "cocons_trailing_update": (ctypes.c_int, [ctypes.c_int, _i64, _dp, _dp, ctypes.c_int, ctypes.c_int, _dp]),
 }
 
 _lib = None

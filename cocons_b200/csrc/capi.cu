@@ -494,7 +494,7 @@ static int ctx_create(int device, int64_t n, int64_t p, int64_t r, const double*
   CTX_TRY(cudaMalloc(&c->dSite, sizeof(double) * SF_COUNT * np));
   CTX_TRY(cudaMalloc(&c->dOrig, sizeof(int) * np));
   if (!tiled) CTX_TRY(cudaMalloc(&c->dA, sizeof(double) * np * np));
-  if (chol_workspace_create(np, &c->ws) != 0 || (!tiled && solve_workspace_create(np, &c->ws) != 0)) {
+  if (chol_workspace_create(np, &c->ws, !tiled) != 0 || (!tiled && solve_workspace_create(np, &c->ws) != 0)) {
     set_error("ctx_create: out of device memory for the factorisation workspace");
     cocons_ctx_destroy(c);
     return COCONS_ERR_ALLOC;
@@ -1472,7 +1472,7 @@ int cocons_sim_cond(cocons_ctx* c, int64_t m, const double* locs_pred, const dou
       cudaMalloc(&blk.dC, sizeof(double) * mp * np) != cudaSuccess ||
       cudaMalloc(&dS, sizeof(double) * mp * mp) != cudaSuccess || cudaMalloc(&dE, sizeof(double) * mp * k) != cudaSuccess ||
       cudaMalloc(&dO, sizeof(double) * mp * k) != cudaSuccess ||
-      chol_workspace_create(mp, &ws2) != 0) {
+      chol_workspace_create(mp, &ws2, true) != 0) {
     cleanup();
     set_error("sim_cond: out of device memory");
     return COCONS_ERR_ALLOC;
@@ -1713,6 +1713,63 @@ int cocons_bench_syrk(int device, int64_t n, int64_t k, int reps, double* ms_per
     return COCONS_ERR_CUDA;
   }
   *ms_per_rep = ms / reps;
+  return 0;
+}
+
+int cocons_trailing_update(int device, int64_t m, const double* P, double* C, int path, int reps, double* ms_per_rep) {
+  int rc = check_device(device);
+  if (rc) return rc;
+  if (m <= 0 || m % kTile || (path != 0 && path != 1) || reps < 0 || (reps > 0 && !ms_per_rep) || (!P != !C)) {
+    set_error("trailing_update: m must be a positive multiple of 128, path 0 or 1, and P and C both given or both "
+              "null");
+    return COCONS_ERR_ARG;
+  }
+  if (path == 1 && !g_syrk_i8.update) {
+    set_error("trailing_update: this build of the library has no split-int8 update");
+    return COCONS_ERR_STATE;
+  }
+  const int64_t k = kSyrkI8K;
+  double *dC = nullptr, *dP = nullptr, *dS = nullptr;
+  int8_t* dQ = nullptr;
+  if (cudaMalloc(&dC, sizeof(double) * m * m) != cudaSuccess || cudaMalloc(&dP, sizeof(double) * m * k) != cudaSuccess ||
+      (path == 1 && (cudaMalloc(&dQ, (size_t)kSyrkI8BytesPerRow * m) != cudaSuccess ||
+                     cudaMalloc(&dS, sizeof(double) * m) != cudaSuccess))) {
+    cudaFree(dC), cudaFree(dP), cudaFree(dQ), cudaFree(dS);
+    set_error("trailing_update: out of device memory");
+    return COCONS_ERR_ALLOC;
+  }
+  if (P) {
+    cudaMemcpy(dP, P, sizeof(double) * m * k, cudaMemcpyHostToDevice);
+    cudaMemcpy(dC, C, sizeof(double) * m * m, cudaMemcpyHostToDevice);
+  } else {  // every double 0x3F3F3F3F3F3F3F3F (about 4.8e-4): the timing does not depend on the values
+    cudaMemsetAsync(dC, 0x3F, sizeof(double) * m * m, nullptr);
+    cudaMemsetAsync(dP, 0x3F, sizeof(double) * m * k, nullptr);
+  }
+  auto run = [&]() {
+    if (path == 1) {
+      g_syrk_i8.split(dP, m, m, dQ, dS, nullptr);
+      g_syrk_i8.update(m, m, dQ, dS, 0, 0, dC, m, 1, nullptr);
+    } else {
+      launch_gemm_nt(0, m, m, k, dP, m, dP, m, dC, m, 1, nullptr);
+    }
+  };
+  run();
+  if (C) cudaMemcpy(C, dC, sizeof(double) * m * m, cudaMemcpyDeviceToHost);
+  cudaEvent_t e0, e1;
+  cudaEventCreate(&e0), cudaEventCreate(&e1);
+  cudaEventRecord(e0);
+  for (int i = 0; i < reps; ++i) run();
+  cudaEventRecord(e1);
+  cudaError_t e = cudaEventSynchronize(e1);
+  float ms = 0;
+  cudaEventElapsedTime(&ms, e0, e1);
+  cudaEventDestroy(e0), cudaEventDestroy(e1);
+  cudaFree(dC), cudaFree(dP), cudaFree(dQ), cudaFree(dS);
+  if (e != cudaSuccess) {
+    set_error("trailing_update: %s", cudaGetErrorString(e));
+    return COCONS_ERR_CUDA;
+  }
+  if (reps > 0) *ms_per_rep = ms / reps;
   return 0;
 }
 

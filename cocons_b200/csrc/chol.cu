@@ -15,6 +15,7 @@
 
 #include "../../include/cocons_b200.h"
 #include "common.cuh"
+#include "tile_order.cuh"
 
 namespace cocons {
 
@@ -56,119 +57,6 @@ __device__ __forceinline__ void dmma884(double& d0, double& d1, double a, double
   asm("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
       : "+d"(d0), "+d"(d1)
       : "d"(a), "d"(b));
-}
-
-// Tile rasterisation.  Tiles are visited band by band (32 tile rows = 4096 matrix rows per band),
-// column by column inside a band, so that the ~300 tiles in flight at any time share one slab of A rows
-// (25 MB at K = 768, L2-resident) and a few B column tiles: the operand panel (300 MB at n = 50k, larger than
-// L2) is read from HBM once per band instead of once per tile column.  Band height 16 / 24 / 32 run at the
-// same speed (35.40 / 35.37 / 35.34 TFLOP/s, tensor-bound); the taller band re-reads the B tiles less often
-// (DRAM traffic of the largest launch 1.21x -> ~1.1x algorithmic; profiles/r02_gemm_ncu.md).
-//   ni tile rows of 128, njc tile columns of BN = 128 / W; with lower_only, tile (bi, c) exists when
-//   bi >= c / W (the matrix origin lies on the diagonal).
-#ifndef COCONS_GEMM_BAND
-#define COCONS_GEMM_BAND 32
-#endif
-constexpr int kBandRows = COCONS_GEMM_BAND;
-
-template <int W>
-__host__ __device__ __forceinline__ int64_t band_tiles(int r, int ni, int njc, int lower_only, int* full_cols_out) {
-  const int r0 = r * kBandRows;
-  const int h = (ni - r0 < kBandRows) ? ni - r0 : kBandRows;
-  if (!lower_only) {
-    *full_cols_out = njc;
-    return (int64_t)h * njc;
-  }
-  const int full_cols = (W * r0 < njc) ? W * r0 : njc;  // columns that see all h rows of the band
-  *full_cols_out = full_cols;
-  int64_t count = (int64_t)h * full_cols;
-  const int tri_end = (W * (r0 + h) < njc) ? W * (r0 + h) : njc;
-  if (tri_end == W * (r0 + h)) {
-    count += (int64_t)W * h * (h + 1) / 2;
-  } else {
-    for (int c = W * r0; c < tri_end; ++c) count += r0 + h - c / W;
-  }
-  return count;
-}
-
-template <int W>
-__host__ __device__ __forceinline__ int64_t total_tiles(int ni, int njc, int lower_only) {
-  int64_t total = 0;
-  int dummy;
-  for (int r = 0; r * kBandRows < ni; ++r) total += band_tiles<W>(r, ni, njc, lower_only, &dummy);
-  return total;
-}
-
-// O(1) inverse of the numbering above (a CTA decodes its tile once; a linear walk over the bands
-// would cost microseconds for the far-down tiles of a 1500-band-row update).
-//   bands [0, rt): complete triangle part      count(r) = W h^2 r + W h (h + 1) / 2   (h = kBandRows)
-//   band rt (at most one): triangle clipped by njc or by the last, shorter band - walked directly
-//   bands after it: rectangles of h x njc
-template <int W>
-__host__ __device__ __forceinline__ void tile_decode(int64_t t, int ni, int njc, int lower_only, int& bi, int& bj) {
-  const int nbands = (ni + kBandRows - 1) / kBandRows;
-  int r;
-  if (!lower_only) {
-    r = (int)(t / ((int64_t)kBandRows * njc));
-    if (r > nbands - 1) r = nbands - 1;
-    t -= (int64_t)r * kBandRows * njc;
-    const int r0 = r * kBandRows;
-    const int h = (ni - r0 < kBandRows) ? ni - r0 : kBandRows;
-    bj = (int)(t / h);
-    bi = r0 + (int)(t % h);
-    return;
-  }
-  // number of leading bands that are full height and whose triangle is not clipped by njc
-  int rt = njc / (kBandRows * W);
-  const int full_height = ni / kBandRows;
-  if (rt > full_height) rt = full_height;
-  // S(r) = per_a r (r - 1) + per_b r tiles before band r (h = kBandRows: W h^2 r + W h (h + 1) / 2 tiles in band r)
-  const int64_t per_a = (int64_t)W * kBandRows * kBandRows / 2, per_b = (int64_t)W * kBandRows * (kBandRows + 1) / 2;
-  auto before = [&](int rr) { return per_a * rr * (int64_t)(rr - 1) + per_b * rr; };
-  if (t < before(rt)) {
-    const double a = (double)per_a, b = (double)(per_b - per_a);
-    r = (int)((-b + sqrt(b * b + 4.0 * a * (double)t)) / (2.0 * a));
-    if (r < 0) r = 0;
-    while (r + 1 <= rt && before(r + 1) <= t) ++r;
-    while (before(r) > t) --r;
-    t -= before(r);
-  } else {
-    t -= before(rt);
-    r = rt;
-    int dummy;
-    for (;; ++r) {  // at most two irregular bands, then rectangles in closed form
-      const int64_t cnt = band_tiles<W>(r, ni, njc, 1, &dummy);
-      if (t < cnt) break;
-      t -= cnt;
-      const int r0n = (r + 1) * kBandRows;
-      if (W * r0n >= njc && ni - r0n >= kBandRows) {  // from here on: full-height rectangles h x njc
-        const int64_t rect = (int64_t)kBandRows * njc;
-        int skip = (int)(t / rect);
-        const int max_skip = (ni - r0n) / kBandRows - 1;  // keep the last (possibly shorter) band for the walk
-        if (skip > max_skip) skip = max_skip < 0 ? 0 : max_skip;
-        r += skip;
-        t -= (int64_t)skip * rect;
-      }
-    }
-  }
-  const int r0 = r * kBandRows;
-  const int h = (ni - r0 < kBandRows) ? ni - r0 : kBandRows;
-  const int full_cols = (W * r0 < njc) ? W * r0 : njc;
-  if (t < (int64_t)h * full_cols) {
-    bj = (int)(t / h);
-    bi = r0 + (int)(t % h);
-    return;
-  }
-  t -= (int64_t)h * full_cols;
-  for (int c = W * r0;; ++c) {  // at most W * h columns in the triangular part
-    const int rows = r0 + h - c / W;
-    if (t < rows) {
-      bj = c;
-      bi = c / W + (int)t;
-      return;
-    }
-    t -= rows;
-  }
 }
 
 // ---------------------------------------------------------------------------
@@ -888,9 +776,12 @@ void launch_potrf_tile(double* A, int64_t ld, double* Winv, int* info, int first
   potrf_tile_blocked_kernel<<<1, 256, kPotrfBlockedSmem, st>>>(A, ld, Winv, info, first_index);
 }
 
-int chol_workspace_create(int64_t n_pad, CholWorkspace* ws) {
+SyrkI8Ops g_syrk_i8 = {nullptr, nullptr};
+
+int chol_workspace_create(int64_t n_pad, CholWorkspace* ws, bool with_i8) {
   ws->winv = nullptr, ws->info = nullptr, ws->panel_stream = nullptr, ws->ev_a = nullptr, ws->ev_p = nullptr;
   ws->ev_k0 = nullptr, ws->ev_k1 = nullptr;
+  ws->i8_slices = nullptr, ws->i8_scale = nullptr;
   int lo = 0, hi = 0;
   cudaDeviceGetStreamPriorityRange(&lo, &hi);  // hi = greatest priority (numerically lowest)
   if (const char* e = getenv("COCONS_PANEL_PRIORITY"))  // 0: panel stream at default priority (bisection aid)
@@ -904,11 +795,20 @@ int chol_workspace_create(int64_t n_pad, CholWorkspace* ws) {
     chol_workspace_destroy(ws);
     return COCONS_ERR_ALLOC;
   }
+  if (with_i8 && g_syrk_i8.update && n_pad >= kSyrkI8MinPad &&
+      (cudaMalloc(&ws->i8_slices, (size_t)kSyrkI8BytesPerRow * n_pad) != cudaSuccess ||
+       cudaMalloc(&ws->i8_scale, sizeof(double) * n_pad) != cudaSuccess)) {
+    chol_workspace_destroy(ws);
+    return COCONS_ERR_ALLOC;
+  }
   return 0;
 }
 
 void chol_workspace_destroy(CholWorkspace* ws) {
   cudaFree(ws->winv), cudaFree(ws->info);
+  if (ws->i8_slices) cudaFree(ws->i8_slices);
+  if (ws->i8_scale) cudaFree(ws->i8_scale);
+  ws->i8_slices = nullptr, ws->i8_scale = nullptr;
   if (ws->panel_stream) cudaStreamDestroy(ws->panel_stream);
   if (ws->ev_a) cudaEventDestroy(ws->ev_a);
   if (ws->ev_p) cudaEventDestroy(ws->ev_p);
@@ -953,8 +853,20 @@ int chol_outer(int64_t n_pad) {
   return n_pad >= 16384 ? 6 : (n_pad >= 8192 ? 4 : 2);
 }
 
+// trailing updates with at least this many rows run as split-int8 products (syrk_i8.cu) when the workspace has
+// the slices; COCONS_SYRK_I8=0, read on every call, keeps every update on the DMMA GEMM.  Stand-alone lower-triangle
+// updates on B200 (tools/syrk_i8_bench.py): int8 / DMMA time 1.24 at 4096 rows, 1.02 at 8192, 0.96 at 16 384
+constexpr int64_t kSyrkI8MinRows = 16384;
+
+static bool syrk_i8_enabled(const CholWorkspace& ws) {
+  if (!g_syrk_i8.update || !ws.i8_slices) return false;
+  const char* e = getenv("COCONS_SYRK_I8");
+  return !(e && atoi(e) == 0);
+}
+
 int chol_factor(double* A, int64_t n_pad, int64_t ld, CholWorkspace ws, cudaStream_t st) {
   cudaMemsetAsync(ws.info, 0, sizeof(int), st);
+  const bool i8 = syrk_i8_enabled(ws);
   const int64_t nt = n_pad / kTile;
   const int64_t outer = chol_outer(n_pad);
   static int lookahead = -1;  // COCONS_CHOL_LOOKAHEAD=0: panel work on the main stream too (debugging knob)
@@ -972,18 +884,33 @@ int chol_factor(double* A, int64_t n_pad, int64_t ld, CholWorkspace ws, cudaStre
     const int64_t nb_next = std::min<int64_t>(outer, nt - (J0 + jb));
     const int64_t wnext = nb_next * kTile;
     const double* P = A + J0 * kTile * ld + done;  // rows [done, n_pad) of panel J
-    launch_gemm_nt(0, trail, wnext, jb * kTile, P, ld, P, ld, A + done * ld + done, ld, 1, st);  // (a)
+    const int64_t rest = trail - wnext;
+    const bool split = i8 && jb * kTile == kSyrkI8K && trail >= kSyrkI8MinRows;
+    if (split) {  // (a) from the slices of all rows of panel J; (b) re-uses them
+      g_syrk_i8.split(P, ld, trail, ws.i8_slices, ws.i8_scale, st);
+      g_syrk_i8.update(trail, wnext, ws.i8_slices, ws.i8_scale, 0, 0, A + done * ld + done, ld, 1, st);
+    } else {
+      launch_gemm_nt(0, trail, wnext, jb * kTile, P, ld, P, ld, A + done * ld + done, ld, 1, st);  // (a)
+    }
     cudaEventRecord(ws.ev_a, st);
     cudaStreamWaitEvent(ps, ws.ev_a, 0);
     factor_panel(A, n_pad, ld, ws, J0 + jb, nb_next, ps);
     cudaEventRecord(ws.ev_p, ps);
-    const int64_t rest = trail - wnext;
     if (rest > 0) {  // (b)
-      const double* P2 = P + wnext;
-      // the first (b) launch is the largest kernel of the factorisation: bracket it with events so
-      // that its own duration (measured inside the evaluation) is available for the roofline
+      double* C2 = A + (done + wnext) * ld + done + wnext;
+      // the first (b) update is the largest of the factorisation: bracket it with events so that its own
+      // duration (measured inside the evaluation) is available for the roofline.  On the int8 path the bracket
+      // holds what a stand-alone (b) costs, the split of its rows included: that split is repeated inside it
+      // (the same slices again, once per factorisation).
       if (J0 == 0) cudaEventRecord(ws.ev_k0, st);
-      launch_gemm_nt(0, rest, rest, jb * kTile, P2, ld, P2, ld, A + (done + wnext) * ld + done + wnext, ld, 1, st);
+      if (split) {
+        if (J0 == 0) g_syrk_i8.split(P + wnext, ld, rest, ws.i8_slices + wnext * kSyrkI8BytesPerRow,
+                                     ws.i8_scale + wnext, st);
+        g_syrk_i8.update(rest, rest, ws.i8_slices, ws.i8_scale, wnext, wnext, C2, ld, 1, st);
+      } else {
+        const double* P2 = P + wnext;
+        launch_gemm_nt(0, rest, rest, jb * kTile, P2, ld, P2, ld, C2, ld, 1, st);
+      }
       if (J0 == 0) cudaEventRecord(ws.ev_k1, st);
     }
     cudaStreamWaitEvent(st, ws.ev_p, 0);

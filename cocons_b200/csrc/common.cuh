@@ -120,10 +120,15 @@ struct CholWorkspace {
   int* solve_units;       // 4 ints per unit: tile row I, first tile column J0, end J1, chunk index
   double* solve_part;     // (I * solve_nchunks + chunk) * kSolveMaxRhs * kTile doubles
   int solve_nunits, solve_nchunks;
+  // split-int8 trailing update (syrk_i8.cu): int8 slices of the rows below one outer panel and their row scales;
+  // null when the library was built without syrk_i8.cu or the workspace was created without it
+  int8_t* i8_slices;
+  double* i8_scale;
 };
 constexpr int kSolveMaxRhs = 8;   // right-hand sides per launch of the substitution kernels
 constexpr int kSolveChunk = 16;   // tile columns per work unit (2 MB of L)
-int chol_workspace_create(int64_t n_pad, CholWorkspace* ws);
+// with_i8: also the slice workspace of the split-int8 trailing update, when n_pad reaches it (kSyrkI8MinPad)
+int chol_workspace_create(int64_t n_pad, CholWorkspace* ws, bool with_i8 = false);
 void chol_workspace_destroy(CholWorkspace* ws);
 // tiles [J0, J0+jb) of one outer panel (potrf + panel solve + in-panel update) on stream st; A is the
 // address element (0,0) of the full matrix would have (only columns of the panel are touched)
@@ -136,6 +141,22 @@ int chol_outer(int64_t n_pad);  // tiles per outer panel of chol_factor
 void launch_potrf_tile(double* A, int64_t ld, double* Winv, int* info, int first_index, cudaStream_t st);
 void launch_gemm_nt(int mode, int64_t M, int64_t N, int64_t K, const double* A, int64_t lda, const double* B,
                     int64_t ldb, double* C, int64_t ldc, int lower_only, cudaStream_t st);
+
+// ---- syrk_i8.cu: the K = 768 trailing update C -= P P^T as exact products of int8 slices on the tensor cores
+// (tcgen05, kind::i8), combined in FP64.  syrk_i8.cu fills g_syrk_i8 when it is linked in; a build of the sources
+// without it (the host emulation of the tests) leaves the entries null and chol_factor keeps to the DMMA GEMM.
+constexpr int kSyrkI8K = 768;                 // panel width the update is built for (chol_outer = 6 tiles)
+constexpr int64_t kSyrkI8MinPad = 16384;      // n_pad from which chol_factor runs K = 768 panels
+constexpr int64_t kSyrkI8BytesPerRow = 8 * kSyrkI8K;  // 8 int8 slices per row
+struct SyrkI8Ops {
+  // rows [0, m) of P (m x 768, column-major, m a multiple of 128) -> slices q and row scales
+  void (*split)(const double* P, int64_t ld, int64_t m, int8_t* q, double* scale, cudaStream_t st);
+  // C[M x N] -= P_a P_b^T over the lower 128 x 64 tiles (lower_only) or all of them, where P_a is rows
+  // [a_row0, a_row0 + M) of the split panel and P_b rows [b_row0, b_row0 + N); a_row0, b_row0 multiples of 128
+  void (*update)(int64_t M, int64_t N, const int8_t* q, const double* scale, int64_t a_row0, int64_t b_row0,
+                 double* C, int64_t ldc, int lower_only, cudaStream_t st);
+};
+extern SyrkI8Ops g_syrk_i8;
 
 // ---- solve.cu ------------------------------------------------------------
 void launch_logdet(const double* L, int64_t n, int64_t ld, double* out, cudaStream_t st);

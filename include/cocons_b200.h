@@ -272,6 +272,14 @@ int cocons_dist_perm(cocons_dist* ctx, int64_t* perm);
  * update kernel, timed with CUDA events; returns milliseconds per repetition.
  * Used to report the kernel's standalone FP64 rate next to cuBLAS dgemm. */
 int cocons_bench_syrk(int device, int64_t n, int64_t k, int reps, double* ms_per_rep);
+/* The K = 768 trailing update of the factorisation, C (m x m) -= P P' over the
+ * lower 128 x 64 tiles, with P m x 768, both column-major, m a multiple of 128.
+ * path 0: the DMMA kernel; 1: the split-int8 kernel (split of P included;
+ * COCONS_ERR_STATE if the library was built without it).  P and C given: C is
+ * updated once in place.  Both null: constant device data.  reps > 0: that
+ * many further updates are timed with CUDA events (ms per repetition). */
+int cocons_trailing_update(int device, int64_t m, const double* P, double* C, int path, int reps,
+                           double* ms_per_rep);
 
 #ifdef __cplusplus
 }
