@@ -770,9 +770,10 @@ static int finish_timings(cocons_ctx* c) {
   return 0;
 }
 
-// what ws.info < 0 means after a forward substitution (solve.cu): a dependency wait of the dataflow kernel ended
-// at its spin limit instead of hanging the device
-static const char* const kSolveGaveUp = "a dependency wait of the forward substitution gave up (COCONS_ERR_CUDA)";
+// what ws.info < 0 means after a factorisation or forward substitution: a dependency wait of the dataflow kernel
+// (solve.cu) or a barrier wait of the split-int8 update (syrk_i8.cu) ended at its limit instead of hanging the device
+static const char* const kSolveGaveUp =
+    "a device wait of the forward substitution or the split-int8 update gave up (COCONS_ERR_CUDA)";
 
 // after the substitutions on the kept factor (prediction, betas): report a wait that gave up, and clear it so that
 // the factor - still valid - can be used again
@@ -1731,13 +1732,16 @@ int cocons_trailing_update(int device, int64_t m, const double* P, double* C, in
   const int64_t k = kSyrkI8K;
   double *dC = nullptr, *dP = nullptr, *dS = nullptr;
   int8_t* dQ = nullptr;
+  int* dInfo = nullptr;
   if (cudaMalloc(&dC, sizeof(double) * m * m) != cudaSuccess || cudaMalloc(&dP, sizeof(double) * m * k) != cudaSuccess ||
       (path == 1 && (cudaMalloc(&dQ, (size_t)kSyrkI8BytesPerRow * m) != cudaSuccess ||
-                     cudaMalloc(&dS, sizeof(double) * m) != cudaSuccess))) {
-    cudaFree(dC), cudaFree(dP), cudaFree(dQ), cudaFree(dS);
+                     cudaMalloc(&dS, sizeof(double) * m) != cudaSuccess ||
+                     cudaMalloc(&dInfo, sizeof(int)) != cudaSuccess))) {
+    cudaFree(dC), cudaFree(dP), cudaFree(dQ), cudaFree(dS), cudaFree(dInfo);
     set_error("trailing_update: out of device memory");
     return COCONS_ERR_ALLOC;
   }
+  if (dInfo) cudaMemsetAsync(dInfo, 0, sizeof(int), nullptr);
   if (P) {
     cudaMemcpy(dP, P, sizeof(double) * m * k, cudaMemcpyHostToDevice);
     cudaMemcpy(dC, C, sizeof(double) * m * m, cudaMemcpyHostToDevice);
@@ -1748,7 +1752,7 @@ int cocons_trailing_update(int device, int64_t m, const double* P, double* C, in
   auto run = [&]() {
     if (path == 1) {
       g_syrk_i8.split(dP, m, m, dQ, dS, nullptr);
-      g_syrk_i8.update(m, m, dQ, dS, 0, 0, dC, m, 1, nullptr);
+      g_syrk_i8.update(m, m, dQ, dS, 0, 0, dC, m, 1, dInfo, nullptr);
     } else {
       launch_gemm_nt(0, m, m, k, dP, m, dP, m, dC, m, 1, nullptr);
     }
@@ -1764,9 +1768,15 @@ int cocons_trailing_update(int device, int64_t m, const double* P, double* C, in
   float ms = 0;
   cudaEventElapsedTime(&ms, e0, e1);
   cudaEventDestroy(e0), cudaEventDestroy(e1);
-  cudaFree(dC), cudaFree(dP), cudaFree(dQ), cudaFree(dS);
+  int info = 0;
+  if (dInfo && e == cudaSuccess) e = cudaMemcpy(&info, dInfo, sizeof(int), cudaMemcpyDeviceToHost);
+  cudaFree(dC), cudaFree(dP), cudaFree(dQ), cudaFree(dS), cudaFree(dInfo);
   if (e != cudaSuccess) {
     set_error("trailing_update: %s", cudaGetErrorString(e));
+    return COCONS_ERR_CUDA;
+  }
+  if (info != 0) {
+    set_error("trailing_update: a barrier wait of the split-int8 update gave up");
     return COCONS_ERR_CUDA;
   }
   if (reps > 0) *ms_per_rep = ms / reps;

@@ -888,7 +888,7 @@ int chol_factor(double* A, int64_t n_pad, int64_t ld, CholWorkspace ws, cudaStre
     const bool split = i8 && jb * kTile == kSyrkI8K && trail >= kSyrkI8MinRows;
     if (split) {  // (a) from the slices of all rows of panel J; (b) re-uses them
       g_syrk_i8.split(P, ld, trail, ws.i8_slices, ws.i8_scale, st);
-      g_syrk_i8.update(trail, wnext, ws.i8_slices, ws.i8_scale, 0, 0, A + done * ld + done, ld, 1, st);
+      g_syrk_i8.update(trail, wnext, ws.i8_slices, ws.i8_scale, 0, 0, A + done * ld + done, ld, 1, ws.info, st);
     } else {
       launch_gemm_nt(0, trail, wnext, jb * kTile, P, ld, P, ld, A + done * ld + done, ld, 1, st);  // (a)
     }
@@ -906,7 +906,7 @@ int chol_factor(double* A, int64_t n_pad, int64_t ld, CholWorkspace ws, cudaStre
       if (split) {
         if (J0 == 0) g_syrk_i8.split(P + wnext, ld, rest, ws.i8_slices + wnext * kSyrkI8BytesPerRow,
                                      ws.i8_scale + wnext, st);
-        g_syrk_i8.update(rest, rest, ws.i8_slices, ws.i8_scale, wnext, wnext, C2, ld, 1, st);
+        g_syrk_i8.update(rest, rest, ws.i8_slices, ws.i8_scale, wnext, wnext, C2, ld, 1, ws.info, st);
       } else {
         const double* P2 = P + wnext;
         launch_gemm_nt(0, rest, rest, jb * kTile, P2, ld, P2, ld, C2, ld, 1, st);

@@ -152,9 +152,10 @@ struct SyrkI8Ops {
   // rows [0, m) of P (m x 768, column-major, m a multiple of 128) -> slices q and row scales
   void (*split)(const double* P, int64_t ld, int64_t m, int8_t* q, double* scale, cudaStream_t st);
   // C[M x N] -= P_a P_b^T over the lower 128 x 64 tiles (lower_only) or all of them, where P_a is rows
-  // [a_row0, a_row0 + M) of the split panel and P_b rows [b_row0, b_row0 + N); a_row0, b_row0 multiples of 128
+  // [a_row0, a_row0 + M) of the split panel and P_b rows [b_row0, b_row0 + N); a_row0, b_row0 multiples of 128.
+  // A device wait that gave up (a bug) sets *info (device) to COCONS_ERR_CUDA if it was 0.
   void (*update)(int64_t M, int64_t N, const int8_t* q, const double* scale, int64_t a_row0, int64_t b_row0,
-                 double* C, int64_t ldc, int lower_only, cudaStream_t st);
+                 double* C, int64_t ldc, int lower_only, int* info, cudaStream_t st);
 };
 extern SyrkI8Ops g_syrk_i8;
 

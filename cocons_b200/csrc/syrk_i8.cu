@@ -13,8 +13,15 @@
 // Layout of the slices: for every 128-row tile r of P and every 32-column chunk c (24 of them), a 32 KB block of
 // the 8 slices, each 128 rows x 32 B in the UMMA K-major SWIZZLE_32B layout (row i at 32 i, 16-byte half h stored
 // at h ^ bit 2 of i).  One stage of the update is one chunk: A = the 32 KB block (one bulk copy), B = the 2 KB
-// halves of the 8 slices of its 64 rows.  A CTA computes one 128 x 64 tile of C: its 8 int32 accumulators of
-// 128 x 64 fill the 512 columns of tensor memory.
+// halves of the 8 slices of its 64 rows.  A tile of C is 128 x 64: its 8 int32 accumulators of 128 x 64 fill the
+// 512 columns of tensor memory.
+//
+// Update kernel: persistent, one CTA per SM, warp-specialised (warp 0 feeds the stages, warp 1 issues the MMAs,
+// warps 2-9 run the epilogue).  The epilogue drains the accumulators into registers and hands tensor memory back
+// before its read-modify-write of C, so that the products of the next tile run under it; the producer runs ahead
+// into the next tile's stages meanwhile.  CTAs can form clusters of kCM x kCN tiles (2 x 2: 256 rows x one 128-wide
+// block column) that share their operands: the A block of a tile row is multicast to the CTAs of that row, the B
+// halves of a tile column to the CTAs of that column, so each SM pulls half of a stage's 48 KB through L2.
 #include "../../include/cocons_b200.h"
 #include "common.cuh"
 #include "tile_order.cuh"
@@ -33,7 +40,9 @@ constexpr uint32_t kSliceBytesB = kRowsB * kChunk;                // 2 KB
 constexpr uint32_t kBlockBytes = kSlices * kSliceBytesA;          // 32 KB per (row tile, chunk)
 constexpr uint32_t kStageBytes = kSlices * (kSliceBytesA + kSliceBytesB);  // 48 KB
 constexpr int kStages = 4;
-constexpr int kThreads = 128;
+constexpr int kEpiWarps = 8;                       // two per tensor-memory lane quarter, each half of the columns
+constexpr int kThreads = 32 * (2 + kEpiWarps);     // producer warp, MMA warp, epilogue warps
+constexpr int kSplitThreads = 128;
 constexpr int kSmemBytes = kStages * kStageBytes + 1024;  // + alignment of the stages to 1 KB
 constexpr int kTmemCols = 512;
 static_assert(kWeights * kRowsB <= kTmemCols, "the accumulators must fit tensor memory");
@@ -45,23 +54,52 @@ __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
 __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
 }
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
+__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
+  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
+}
+__device__ __forceinline__ bool mbar_try(uint32_t bar, uint32_t parity) {
+  uint32_t ok;
   asm volatile(
       "{\n"
-      ".reg .pred P1;\n"
-      "LAB_WAIT:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n"
-      "@P1 bra DONE;\n"
-      "bra LAB_WAIT;\n"
-      "DONE:\n"
-      "}" ::"r"(bar),
-      "r"(parity)
+      ".reg .pred p;\n"
+      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
+      "selp.u32 %0, 1, 0, p;\n"
+      "}"
+      : "=r"(ok)
+      : "r"(bar), "r"(parity)
       : "memory");
+  return ok != 0;
+}
+__device__ __forceinline__ uint64_t globaltimer_ns() {
+  uint64_t t;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+  return t;
+}
+// a healthy wait ends within tens of microseconds; one that does not (an arrival or byte count that does not add up,
+// which would be a bug) sets *info = COCONS_ERR_CUDA and returns false, and the kernel ends instead of hanging
+constexpr uint64_t kWaitLimitNs = 2000000000ull;
+__device__ __noinline__ bool mbar_wait(uint32_t bar, uint32_t parity, int* info) {
+  if (mbar_try(bar, parity)) return true;
+  const uint64_t t0 = globaltimer_ns();
+  while (!mbar_try(bar, parity))
+    if (globaltimer_ns() - t0 > kWaitLimitNs) {
+      atomicCAS(info, 0, COCONS_ERR_CUDA);
+      return false;
+    }
+  return true;
 }
 __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
                "l"(src), "r"(bytes), "r"(bar)
                : "memory");
+}
+// the same bytes at the same offset in every CTA of the cluster named in mask, each signalling its own barrier at bar
+__device__ __forceinline__ void bulk_g2s_mc(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar, uint16_t mask) {
+  asm volatile(
+      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], "
+      "%4;" ::"r"(dst),
+      "l"(src), "r"(bytes), "r"(bar), "h"(mask)
+      : "memory");
 }
 
 // UMMA shared-memory descriptor, K-major SWIZZLE_32B: 8-row groups 256 B apart (SBO), LBO unused (1), version 1
@@ -74,41 +112,51 @@ __host__ __device__ constexpr uint32_t idesc_i8(int nblk) {
   return (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(nblk * kRowsB >> 3) << 17) | ((uint32_t)(kRowsA >> 4) << 24);
 }
 
-// D (+)= A B^T; the accumulators are cleared beforehand, so every MMA accumulates
-__device__ __forceinline__ void umma_i8(uint32_t dtmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc) {
+// D = A B^T (acc = 0) or D += A B^T
+__device__ __forceinline__ void umma_i8(uint32_t dtmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
   asm volatile(
       "{\n"
       ".reg .pred p;\n"
-      "setp.ne.b32 p, 1, 0;\n"
+      "setp.ne.b32 p, %4, 0;\n"
       "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n"
       "}" ::"r"(dtmem),
-      "l"(adesc), "l"(bdesc), "r"(idesc));
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc));
 }
 
 // The 36 slice products of a chunk in 12 MMAs.  An MMA costs about the same for N = 64 as for N = 256 (measured on
 // B200: 128 x 64 x 32 products ran at a quarter of the int8 rate), so the B slices u0 .. u0 + nblk - 1, which lie
 // one after the other in the stage (64 rows each), form one operand of N = 64 nblk, and the MMA of A_t writes it at
-// tensor-memory column 64 (t + u0 - 2): block u lands on the accumulator of its weight t + u.
+// tensor-memory column 64 (t + u0 - 2): block u lands on the accumulator of its weight t + u.  The first two MMAs
+// cover the 512 columns exactly once (weights 2-5 and 6-9), so in the first chunk of a tile they overwrite and
+// everything after them accumulates: the int32 sums are exact, and their order does not change a bit.
 struct SlicePairs {
   int t, u0, nblk;
 };
 constexpr int kMmas = 12;
 __host__ __device__ constexpr SlicePairs slice_pairs(int k) {
-  constexpr SlicePairs p[kMmas] = {{1, 1, 4}, {2, 1, 4}, {3, 1, 4}, {4, 1, 4}, {5, 1, 4}, {6, 1, 3},
-                                   {7, 1, 2}, {8, 1, 1}, {1, 5, 4}, {2, 5, 3}, {3, 5, 2}, {4, 5, 1}};
+  constexpr SlicePairs p[kMmas] = {{1, 1, 4}, {1, 5, 4}, {2, 1, 4}, {3, 1, 4}, {4, 1, 4}, {5, 1, 4},
+                                   {6, 1, 3}, {7, 1, 2}, {8, 1, 1}, {2, 5, 3}, {3, 5, 2}, {4, 5, 1}};
   return p[k];
 }
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
+// arrive on the barrier at bar in every CTA of the cluster named in mask once the MMAs issued so far have completed
+__device__ __forceinline__ void umma_commit_mc(uint32_t bar, uint16_t mask) {
+  asm volatile(
+      "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
+      "h"(mask)
+      : "memory");
+}
 
-#define TMEM_LD16(taddr, r)                                                                                      \
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, " \
-               "[%16];"                                                                                          \
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), \
-                 "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]),        \
-                 "=r"(r[15])                                                                                     \
+#define TMEM_LD8(taddr, r)                                                                                      \
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"                          \
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]) \
                : "r"(taddr))
+
+__device__ __forceinline__ void cluster_sync() {
+  asm volatile("barrier.cluster.arrive.release.aligned;\nbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
 
 // byte offset of (row i, byte b) inside one 128 x 32 B slice of a chunk block
 __host__ __device__ __forceinline__ uint32_t sw32_offset(int i, int b) {
@@ -119,7 +167,7 @@ __host__ __device__ __forceinline__ uint32_t sw32_offset(int i, int b) {
 }  // namespace
 
 // one thread per row, 128 rows (one tile) per block
-__global__ void __launch_bounds__(kThreads) syrk_i8_split_kernel(const double* __restrict__ P, int64_t ld,
+__global__ void __launch_bounds__(kSplitThreads) syrk_i8_split_kernel(const double* __restrict__ P, int64_t ld,
                                                                   int8_t* __restrict__ q, double* __restrict__ scale) {
   const int i = threadIdx.x;
   const int64_t tile = blockIdx.x, row = tile * kRowsA + i;
@@ -162,25 +210,70 @@ __global__ void __launch_bounds__(kThreads) syrk_i8_split_kernel(const double* _
   }
 }
 
-// one 128 x 64 tile of C per CTA; warp 0 lane 0 feeds the stages, warp 1 lane 0 issues the MMAs, all four warps
-// run the epilogue (warp w owns tensor-memory lanes, i.e. tile rows, 32 w .. 32 w + 31)
+namespace {
+
+// Cluster shape in tiles: kCM tile rows (A blocks) x kCN tile columns (B halves).  Measured on B200 (DESIGN.md §3
+// K5i): at full clock a tile costs the same ~42 k cycles per SM in every shape - the feed does not bound it - but
+// clusters of 4 leave 16 of the 148 SMs unused, and inside a factorisation, which runs at the power limit, sharing
+// the B halves (1 x 2) draws less power and keeps a higher clock than 1 x 1.  Other shapes build for comparison.
+#ifndef COCONS_I8_CLUSTER_M
+#define COCONS_I8_CLUSTER_M 1
+#endif
+#ifndef COCONS_I8_CLUSTER_N
+#define COCONS_I8_CLUSTER_N 2
+#endif
+constexpr int kCM = COCONS_I8_CLUSTER_M, kCN = COCONS_I8_CLUSTER_N, kCtas = kCM * kCN;
+static_assert((kCM == 1 || kCM == 2) && (kCN == 1 || kCN == 2), "clusters of 1 or 2 tile rows and columns");
+// super-tiles of 128 kCM rows x 64 kCN columns, numbered by tile_order.cuh: kW of their columns per row unit (with
+// lower_only, super-tile (R, C) exists when R >= C / kW, i.e. when it holds at least one lower tile), bands of
+// 4096 rows
+constexpr int kW = 2 * kCM / kCN, kBand = kBandRows / kCM;
+
+// Probe build (-DCOCONS_I8_PROBE, tools/syrk_i8_probe.py): per-CTA cycle counts summed over the launch
+#ifdef COCONS_I8_PROBE
+__device__ unsigned long long g_i8_probe[8];  // start->first MMA, MMA full waits, producer empty waits, epilogue,
+                                              // MMA waits for tensor memory, CTA cycles, tiles, CTAs
+#define I8_PROBE(...) __VA_ARGS__
+#else
+#define I8_PROBE(...)
+#endif
+
+__device__ __forceinline__ void super_tile(int64_t st, int ni, int nj, int lower_only, int rm, int cn, int& bi, int& bj,
+                                           bool& store) {
+  int R, Cc;
+  tile_decode<kW, kBand>(st, (ni + kCM - 1) / kCM, nj / kCN, lower_only, R, Cc);
+  bi = R * kCM + rm, bj = Cc * kCN + cn;
+  // a tile row past the last (odd ni), or a tile above the diagonal blocks of a diagonal super-tile, takes part in
+  // feeding its cluster but writes nothing
+  store = bi < ni && (!lower_only || bi >= bj / 2);
+}
+
+}  // namespace
+
 __global__ void __launch_bounds__(kThreads, 1)
     syrk_i8_update_kernel(int ni, int nj, int lower_only, const int8_t* __restrict__ qa, const double* __restrict__ sa,
-                          const int8_t* __restrict__ qb, const double* __restrict__ sb, double* C, int64_t ldc) {
+                          const int8_t* __restrict__ qb, const double* __restrict__ sb, double* C, int64_t ldc,
+                          int* info) {
   extern __shared__ uint8_t smem_raw[];
-  __shared__ __align__(8) uint64_t bars[2 * kStages + 1];
+  __shared__ __align__(8) uint64_t bars[2 * kStages + 2];
   __shared__ uint32_t tmem_slot;
+  I8_PROBE(const long long t_start = clock64();)
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  int bi, bj;
-  tile_decode<2>(blockIdx.x, ni, nj, lower_only, bi, bj);
+  const int rank = (int)(blockIdx.x % kCtas), rm = rank / kCN, cn = rank % kCN;
+  // the clusters (as many as fit the device at once) take the super-tiles in a stride over the banded numbering, so
+  // that the tiles in flight stay neighbours
+  const int64_t cluster = blockIdx.x / kCtas, nclusters = gridDim.x / kCtas;
+  const int64_t nsuper = total_tiles<kW, kBand>((ni + kCM - 1) / kCM, nj / kCN, lower_only);
   const uint32_t stage0 = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  const uint32_t full0 = smem_u32(bars), empty0 = full0 + 8 * kStages, done = full0 + 16 * kStages;
+  const uint32_t full0 = smem_u32(bars), empty0 = full0 + 8 * kStages;
+  const uint32_t tmem_full = full0 + 16 * kStages, tmem_empty = tmem_full + 8;
   if (tid == 0) {
     for (int s = 0; s < kStages; ++s) {
-      mbar_init(full0 + 8 * s, 1);
-      mbar_init(empty0 + 8 * s, 1);
+      mbar_init(full0 + 8 * s, 1);         // the local expect_tx; the bytes come from the CTAs that feed this one
+      mbar_init(empty0 + 8 * s, kCtas);    // one MMA commit from every CTA of the cluster
     }
-    mbar_init(done, 1);
+    mbar_init(tmem_full, 1);
+    mbar_init(tmem_empty, 32 * kEpiWarps);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   if (warp == 0) {
@@ -191,90 +284,163 @@ __global__ void __launch_bounds__(kThreads, 1)
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  if (kCtas > 1) cluster_sync();  // every barrier of the cluster is initialised before a multicast reaches it
   const uint32_t tmem = tmem_slot;
-  {  // clear the accumulators: warp w its 32 lanes, 32 columns per store
-    const uint32_t z = 0;
-    const uint32_t lane_base = tmem + ((uint32_t)(32 * warp) << 16);
-#pragma unroll 1
-    for (int col = 0; col < kTmemCols; col += 32)
-      asm volatile(
-          "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], {%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,"
-          "%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1};" ::"r"(lane_base + (uint32_t)col),
-          "r"(z)
-          : "memory");
-    asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  }
+  I8_PROBE(unsigned long long p_first = 0, p_full = 0, p_empty = 0, p_epi = 0, p_tmem = 0, p_tiles = 0;)
 
-  if (warp == 0 && lane == 0) {
-    const int8_t* a = qa + (int64_t)bi * kChunks * kBlockBytes;
-    const int8_t* b = qb + (int64_t)(bj >> 1) * kChunks * kBlockBytes + (bj & 1) * kSliceBytesB;
-    for (int c = 0; c < kChunks; ++c) {
-      const int slot = c % kStages;
-      if (c >= kStages) mbar_wait(empty0 + 8 * slot, (uint32_t)((c / kStages - 1) & 1));
-      const uint32_t fb = full0 + 8 * slot, da = stage0 + slot * kStageBytes, db = da + kSlices * kSliceBytesA;
-      mbar_expect_tx(fb, kStageBytes);
-      bulk_g2s(da, a + (int64_t)c * kBlockBytes, kBlockBytes, fb);
-#pragma unroll
-      for (int t = 0; t < kSlices; ++t)
-        bulk_g2s(db + t * kSliceBytesB, b + (int64_t)c * kBlockBytes + t * kSliceBytesA, kSliceBytesB, fb);
-    }
-  } else if (warp == 1 && lane == 0) {
-    for (int c = 0; c < kChunks; ++c) {
-      const int slot = c % kStages;
-      mbar_wait(full0 + 8 * slot, (uint32_t)((c / kStages) & 1));
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      const uint32_t da = stage0 + slot * kStageBytes, db = da + kSlices * kSliceBytesA;
-#pragma unroll
-      for (int k = 0; k < kMmas; ++k) {
-        const SlicePairs q = slice_pairs(k);
-        umma_i8(tmem + (uint32_t)(q.t + q.u0 - 2) * kRowsB, sw32_desc(da + (q.t - 1) * kSliceBytesA),
-                sw32_desc(db + (q.u0 - 1) * kSliceBytesB), idesc_i8(q.nblk));
+  if (warp == 0) {
+    if (lane == 0) {
+      constexpr uint16_t all = (uint16_t)((1u << kCtas) - 1);
+      uint16_t row_mask = 0, col_mask = 0;  // the CTAs that share this CTA's A block / B half
+      for (int r = 0; r < kCtas; ++r) {
+        if (r / kCN == rm) row_mask |= (uint16_t)(1u << r);
+        if (r % kCN == cn) col_mask |= (uint16_t)(1u << r);
       }
-      umma_commit(empty0 + 8 * slot);  // the stage is free once these MMAs have read it
+      (void)all;
+      uint32_t it = 0;
+      bool ok = true;
+      for (int64_t st = cluster; ok && st < nsuper; st += nclusters) {
+        int bi, bj;
+        bool store;
+        super_tile(st, ni, nj, lower_only, rm, cn, bi, bj, store);
+        // the missing tile row of an odd ni fetches the last real block, so that nothing is read past the slices
+        const int8_t* a = qa + (int64_t)(bi < ni ? bi : ni - 1) * kChunks * kBlockBytes + cn * (kBlockBytes / kCN);
+        const int8_t* b = qb + (int64_t)(bj >> 1) * kChunks * kBlockBytes + (bj & 1) * kSliceBytesB;
+        for (int c = 0; c < kChunks; ++c, ++it) {
+          const uint32_t slot = it % kStages;
+          if (it >= kStages) {
+            I8_PROBE(const long long t0 = clock64();)
+            if (!mbar_wait(empty0 + 8 * slot, ((it / kStages) - 1) & 1, info)) {
+              ok = false;
+              break;
+            }
+            I8_PROBE(p_empty += clock64() - t0;)
+          }
+          const uint32_t fb = full0 + 8 * slot, da = stage0 + slot * kStageBytes, db = da + kSlices * kSliceBytesA;
+          mbar_expect_tx(fb, kStageBytes);
+          const uint32_t aoff = cn * (kBlockBytes / kCN);
+          if (kCN > 1)
+            bulk_g2s_mc(da + aoff, a + (int64_t)c * kBlockBytes, kBlockBytes / kCN, fb, row_mask);
+          else
+            bulk_g2s(da + aoff, a + (int64_t)c * kBlockBytes, kBlockBytes / kCN, fb);
+#pragma unroll
+          for (int t = rm; t < kSlices; t += kCM) {
+            if (kCM > 1)
+              bulk_g2s_mc(db + t * kSliceBytesB, b + (int64_t)c * kBlockBytes + t * kSliceBytesA, kSliceBytesB, fb,
+                          col_mask);
+            else
+              bulk_g2s(db + t * kSliceBytesB, b + (int64_t)c * kBlockBytes + t * kSliceBytesA, kSliceBytesB, fb);
+          }
+        }
+      }
+      // the last commits of the cluster's MMAs arrive on this CTA's empty barriers: wait for them before it exits
+      for (uint32_t e = 0; ok && e < kStages; ++e, ++it)
+        if (it >= kStages) ok = mbar_wait(empty0 + 8 * (it % kStages), ((it / kStages) - 1) & 1, info);
     }
-    umma_commit(done);
+  } else if (warp == 1) {
+    if (lane == 0) {
+      constexpr uint16_t all = (uint16_t)((1u << kCtas) - 1);
+      uint32_t it = 0, tl = 0;
+      bool ok = true;
+      for (int64_t st = cluster; ok && st < nsuper; st += nclusters, ++tl) {
+        if (tl > 0) {  // the epilogue has drained the previous tile
+          I8_PROBE(const long long t0 = clock64();)
+          if (!mbar_wait(tmem_empty, (tl - 1) & 1, info)) break;
+          I8_PROBE(p_tmem += clock64() - t0;)
+          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        }
+        for (int c = 0; c < kChunks; ++c, ++it) {
+          const uint32_t slot = it % kStages;
+          I8_PROBE(const long long t0 = clock64();)
+          if (!mbar_wait(full0 + 8 * slot, (it / kStages) & 1, info)) {
+            ok = false;
+            break;
+          }
+          I8_PROBE(const long long t1 = clock64(); p_full += t1 - t0; if (it == 0) p_first = t1 - t_start;)
+          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          const uint32_t da = stage0 + slot * kStageBytes, db = da + kSlices * kSliceBytesA;
+#pragma unroll
+          for (int k = 0; k < kMmas; ++k) {
+            const SlicePairs q = slice_pairs(k);
+            umma_i8(tmem + (uint32_t)(q.t + q.u0 - 2) * kRowsB, sw32_desc(da + (q.t - 1) * kSliceBytesA),
+                    sw32_desc(db + (q.u0 - 1) * kSliceBytesB), idesc_i8(q.nblk), (c > 0 || k >= 2) ? 1u : 0u);
+          }
+          // the stage is free in every CTA that fed this one once these MMAs have read it
+          if (kCtas > 1)
+            umma_commit_mc(empty0 + 8 * slot, all);
+          else
+            umma_commit(empty0 + 8 * slot);
+        }
+        if (ok) umma_commit(tmem_full);
+        I8_PROBE(++p_tiles;)
+      }
+    }
+  } else {
+    // epilogue: C_ij -= ((hi 2^-35 + lo 2^-63) s_i) s_j.  Warp w reads tensor-memory lanes (tile rows) 32 (w % 4) ..,
+    // columns 32 h .. 32 h + 31 with h = (w - 2) / 4
+    const int quarter = warp & 3, h = (warp - 2) >> 2, r = 32 * quarter + lane;
+    const uint32_t trow = tmem + ((uint32_t)(32 * quarter) << 16) + (uint32_t)(32 * h);
+    uint32_t tl = 0;
+    for (int64_t st = cluster; st < nsuper; st += nclusters, ++tl) {
+      int bi, bj;
+      bool store;
+      super_tile(st, ni, nj, lower_only, rm, cn, bi, bj, store);
+      double* Cg = C + (int64_t)(bj * kRowsB + 32 * h) * ldc + (int64_t)bi * kRowsA + r;
+      if (store)
+#pragma unroll 4
+        for (int j = 0; j < 32; ++j) asm volatile("prefetch.global.L2 [%0];" ::"l"(Cg + (int64_t)j * ldc));
+      if (!mbar_wait(tmem_full, tl & 1, info)) break;
+      I8_PROBE(const long long t0 = clock64();)
+      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      double v[32];
+#pragma unroll
+      for (int j0 = 0; j0 < 32; j0 += 8) {
+        uint32_t acc[kWeights][8];
+#pragma unroll
+        for (int w = 0; w < kWeights; ++w) TMEM_LD8(trow + (uint32_t)(w * kRowsB + j0), acc[w]);
+        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+        for (int jj = 0; jj < 8; ++jj) {
+          int64_t hi = 0, lo = 0;
+#pragma unroll
+          for (int w = 0; w < kWeights; ++w) {
+            const int64_t s = (int64_t)(int32_t)acc[w][jj];
+            if (w + 2 <= kHiTop)
+              hi = hi * 128 + s;
+            else
+              lo = lo * 128 + s;
+          }
+          v[j0 + jj] = (double)hi * 0x1p-35 + (double)lo * 0x1p-63;
+        }
+      }
+      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+      mbar_arrive(tmem_empty);  // the next tile's products may overwrite the accumulators now
+      if (store) {
+        const double si = sa[(int64_t)bi * kRowsA + r];
+        const double* sbj = sb + (int64_t)bj * kRowsB + 32 * h;
+#pragma unroll
+        for (int j = 0; j < 32; ++j) {
+          double* p = Cg + (int64_t)j * ldc;
+          __stcs(p, __ldcs(p) - (v[j] * si) * sbj[j]);
+        }
+      }
+      I8_PROBE(if (tid == 64) p_epi += clock64() - t0;)
+    }
   }
   __syncwarp();
-
-  // epilogue: C_ij -= ((hi 2^-35 + lo 2^-63) s_i) s_j, 16 columns at a time
-  mbar_wait(done, 0);
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const int r = 32 * warp + lane;
-  const double si = sa[(int64_t)bi * kRowsA + r];
-  double* Cg = C + (int64_t)bj * kRowsB * ldc + (int64_t)bi * kRowsA + r;
-  const double* sbj = sb + (int64_t)bj * kRowsB;
-  const uint32_t trow = tmem + ((uint32_t)(32 * warp) << 16);
-#pragma unroll 1
-  for (int j0 = 0; j0 < kRowsB; j0 += 16) {
-    uint32_t acc[kWeights][16];
-#pragma unroll
-    for (int w = 0; w < kWeights; ++w) TMEM_LD16(trow + (uint32_t)(w * kRowsB + j0), acc[w]);
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-    for (int jj = 0; jj < 16; ++jj) {
-      int64_t hi = 0, lo = 0;
-#pragma unroll
-      for (int w = 0; w < kWeights; ++w) {
-        const int64_t s = (int64_t)(int32_t)acc[w][jj];
-        if (w + 2 <= kHiTop)
-          hi = hi * 128 + s;
-        else
-          lo = lo * 128 + s;
-      }
-      const double v = (double)hi * 0x1p-35 + (double)lo * 0x1p-63;
-      double* p = Cg + (int64_t)(j0 + jj) * ldc;
-      __stcs(p, __ldcs(p) - (v * si) * sbj[j0 + jj]);
-    }
-  }
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
+  if (kCtas > 1) cluster_sync();
   if (warp == 0) {
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(kTmemCols));
   }
+  I8_PROBE(if (tid == 32) {
+    atomicAdd(&g_i8_probe[0], p_first), atomicAdd(&g_i8_probe[1], p_full), atomicAdd(&g_i8_probe[4], p_tmem);
+    atomicAdd(&g_i8_probe[5], (unsigned long long)(clock64() - t_start)), atomicAdd(&g_i8_probe[6], p_tiles);
+    atomicAdd(&g_i8_probe[7], 1ull);
+  } if (tid == 0) atomicAdd(&g_i8_probe[2], p_empty);
+           if (tid == 64) atomicAdd(&g_i8_probe[3], p_epi);)
 }
 
 namespace {
@@ -284,26 +450,44 @@ static_assert(kHiTop == 5 && kSlices == 8, "the epilogue's 2^-35 and 2^-63 are f
 void split(const double* P, int64_t ld, int64_t m, int8_t* q, double* scale, cudaStream_t st) {
   if (m <= 0) return;
   note_launch();
-  syrk_i8_split_kernel<<<(unsigned)(m / kRowsA), kThreads, 0, st>>>(P, ld, q, scale);
+  syrk_i8_split_kernel<<<(unsigned)(m / kRowsA), kSplitThreads, 0, st>>>(P, ld, q, scale);
 }
 
 void update(int64_t M, int64_t N, const int8_t* q, const double* scale, int64_t a_row0, int64_t b_row0, double* C,
-            int64_t ldc, int lower_only, cudaStream_t st) {
+            int64_t ldc, int lower_only, int* info, cudaStream_t st) {
   if (M <= 0 || N <= 0) return;
-  static bool attr_done[16] = {};
+  cudaLaunchConfig_t cfg = {};
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = kCtas, attr[0].val.clusterDim.y = 1, attr[0].val.clusterDim.z = 1;
+  cfg.blockDim = dim3(kThreads);
+  cfg.dynamicSmemBytes = kSmemBytes;
+  cfg.stream = st;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  // persistent: as many clusters as fit the device at once (one CTA per SM), found once per device
+  static int max_clusters[16] = {};
   int dev = 0;
   cudaGetDevice(&dev);
-  if (dev < 16 && !attr_done[dev]) {
+  int clusters = dev < 16 ? max_clusters[dev] : 0;
+  if (clusters <= 0) {
     cudaFuncSetAttribute(syrk_i8_update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
-    attr_done[dev] = true;
+    cfg.gridDim = dim3(kCtas);
+    if (cudaOccupancyMaxActiveClusters(&clusters, syrk_i8_update_kernel, &cfg) != cudaSuccess || clusters <= 0) {
+      int sms = 0;
+      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+      clusters = sms / kCtas > 0 ? sms / kCtas : 1;
+    }
+    if (dev < 16) max_clusters[dev] = clusters;
   }
   const int ni = (int)(M / kRowsA), nj = (int)(N / kRowsB);
-  const int64_t tiles = total_tiles<2>(ni, nj, lower_only);
+  const int64_t nsuper = total_tiles<kW, kBand>((ni + kCM - 1) / kCM, nj / kCN, lower_only);
+  cfg.gridDim = dim3((unsigned)(kCtas * (nsuper < clusters ? nsuper : clusters)));
   const int8_t* qa = q + a_row0 / kRowsA * kChunks * (int64_t)kBlockBytes;
   const int8_t* qb = q + b_row0 / kRowsA * kChunks * (int64_t)kBlockBytes;
   note_launch();
-  syrk_i8_update_kernel<<<(unsigned)tiles, kThreads, kSmemBytes, st>>>(ni, nj, lower_only, qa, scale + a_row0, qb,
-                                                                       scale + b_row0, C, ldc);
+  cudaLaunchKernelEx(&cfg, syrk_i8_update_kernel, ni, nj, lower_only, qa, scale + a_row0, qb, scale + b_row0, C, ldc,
+                     info);
 }
 
 struct Register {
@@ -312,3 +496,12 @@ struct Register {
 
 }  // namespace
 }  // namespace cocons
+
+#ifdef COCONS_I8_PROBE
+// the probe sums of the launches since the last call, then zero (probe build only)
+extern "C" int cocons_i8_probe_read(unsigned long long* out) {
+  if (cudaMemcpyFromSymbol(out, cocons::g_i8_probe, sizeof(cocons::g_i8_probe)) != cudaSuccess) return -1;
+  const unsigned long long zero[8] = {};
+  return cudaMemcpyToSymbol(cocons::g_i8_probe, zero, sizeof(zero)) == cudaSuccess ? 0 : -1;
+}
+#endif

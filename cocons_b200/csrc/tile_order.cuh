@@ -15,16 +15,17 @@ namespace cocons {
 // same speed (35.40 / 35.37 / 35.34 TFLOP/s, tensor-bound); the taller band re-reads the B tiles less often
 // (DRAM traffic of the largest launch 1.21x -> ~1.1x algorithmic; profiles/r02_gemm_ncu.md).
 //   ni tile rows of 128, njc tile columns of BN = 128 / W; with lower_only, tile (bi, c) exists when
-//   bi >= c / W (the matrix origin lies on the diagonal).
+//   bi >= c / W (the matrix origin lies on the diagonal).  Band is the band height in tile rows; the split-int8
+//   update numbers super-tiles of 256 rows with Band = kBandRows / 2, so that its bands too are 4096 rows high.
 #ifndef COCONS_GEMM_BAND
 #define COCONS_GEMM_BAND 32
 #endif
 constexpr int kBandRows = COCONS_GEMM_BAND;
 
-template <int W>
+template <int W, int Band = kBandRows>
 __host__ __device__ __forceinline__ int64_t band_tiles(int r, int ni, int njc, int lower_only, int* full_cols_out) {
-  const int r0 = r * kBandRows;
-  const int h = (ni - r0 < kBandRows) ? ni - r0 : kBandRows;
+  const int r0 = r * Band;
+  const int h = (ni - r0 < Band) ? ni - r0 : Band;
   if (!lower_only) {
     *full_cols_out = njc;
     return (int64_t)h * njc;
@@ -41,39 +42,39 @@ __host__ __device__ __forceinline__ int64_t band_tiles(int r, int ni, int njc, i
   return count;
 }
 
-template <int W>
+template <int W, int Band = kBandRows>
 __host__ __device__ __forceinline__ int64_t total_tiles(int ni, int njc, int lower_only) {
   int64_t total = 0;
   int dummy;
-  for (int r = 0; r * kBandRows < ni; ++r) total += band_tiles<W>(r, ni, njc, lower_only, &dummy);
+  for (int r = 0; r * Band < ni; ++r) total += band_tiles<W, Band>(r, ni, njc, lower_only, &dummy);
   return total;
 }
 
 // O(1) inverse of the numbering above (a CTA decodes its tile once; a linear walk over the bands
 // would cost microseconds for the far-down tiles of a 1500-band-row update).
-//   bands [0, rt): complete triangle part      count(r) = W h^2 r + W h (h + 1) / 2   (h = kBandRows)
+//   bands [0, rt): complete triangle part      count(r) = W h^2 r + W h (h + 1) / 2   (h = Band)
 //   band rt (at most one): triangle clipped by njc or by the last, shorter band - walked directly
 //   bands after it: rectangles of h x njc
-template <int W>
+template <int W, int Band = kBandRows>
 __host__ __device__ __forceinline__ void tile_decode(int64_t t, int ni, int njc, int lower_only, int& bi, int& bj) {
-  const int nbands = (ni + kBandRows - 1) / kBandRows;
+  const int nbands = (ni + Band - 1) / Band;
   int r;
   if (!lower_only) {
-    r = (int)(t / ((int64_t)kBandRows * njc));
+    r = (int)(t / ((int64_t)Band * njc));
     if (r > nbands - 1) r = nbands - 1;
-    t -= (int64_t)r * kBandRows * njc;
-    const int r0 = r * kBandRows;
-    const int h = (ni - r0 < kBandRows) ? ni - r0 : kBandRows;
+    t -= (int64_t)r * Band * njc;
+    const int r0 = r * Band;
+    const int h = (ni - r0 < Band) ? ni - r0 : Band;
     bj = (int)(t / h);
     bi = r0 + (int)(t % h);
     return;
   }
   // number of leading bands that are full height and whose triangle is not clipped by njc
-  int rt = njc / (kBandRows * W);
-  const int full_height = ni / kBandRows;
+  int rt = njc / (Band * W);
+  const int full_height = ni / Band;
   if (rt > full_height) rt = full_height;
-  // S(r) = per_a r (r - 1) + per_b r tiles before band r (h = kBandRows: W h^2 r + W h (h + 1) / 2 tiles in band r)
-  const int64_t per_a = (int64_t)W * kBandRows * kBandRows / 2, per_b = (int64_t)W * kBandRows * (kBandRows + 1) / 2;
+  // S(r) = per_a r (r - 1) + per_b r tiles before band r (h = Band: W h^2 r + W h (h + 1) / 2 tiles in band r)
+  const int64_t per_a = (int64_t)W * Band * Band / 2, per_b = (int64_t)W * Band * (Band + 1) / 2;
   auto before = [&](int rr) { return per_a * rr * (int64_t)(rr - 1) + per_b * rr; };
   if (t < before(rt)) {
     const double a = (double)per_a, b = (double)(per_b - per_a);
@@ -87,22 +88,22 @@ __host__ __device__ __forceinline__ void tile_decode(int64_t t, int ni, int njc,
     r = rt;
     int dummy;
     for (;; ++r) {  // at most two irregular bands, then rectangles in closed form
-      const int64_t cnt = band_tiles<W>(r, ni, njc, 1, &dummy);
+      const int64_t cnt = band_tiles<W, Band>(r, ni, njc, 1, &dummy);
       if (t < cnt) break;
       t -= cnt;
-      const int r0n = (r + 1) * kBandRows;
-      if (W * r0n >= njc && ni - r0n >= kBandRows) {  // from here on: full-height rectangles h x njc
-        const int64_t rect = (int64_t)kBandRows * njc;
+      const int r0n = (r + 1) * Band;
+      if (W * r0n >= njc && ni - r0n >= Band) {  // from here on: full-height rectangles h x njc
+        const int64_t rect = (int64_t)Band * njc;
         int skip = (int)(t / rect);
-        const int max_skip = (ni - r0n) / kBandRows - 1;  // keep the last (possibly shorter) band for the walk
+        const int max_skip = (ni - r0n) / Band - 1;  // keep the last (possibly shorter) band for the walk
         if (skip > max_skip) skip = max_skip < 0 ? 0 : max_skip;
         r += skip;
         t -= (int64_t)skip * rect;
       }
     }
   }
-  const int r0 = r * kBandRows;
-  const int h = (ni - r0 < kBandRows) ? ni - r0 : kBandRows;
+  const int r0 = r * Band;
+  const int h = (ni - r0 < Band) ? ni - r0 : Band;
   const int full_cols = (W * r0 < njc) ? W * r0 : njc;
   if (t < (int64_t)h * full_cols) {
     bj = (int)(t / h);
