@@ -41,7 +41,13 @@ constexpr uint32_t kBlockBytes = kSlices * kSliceBytesA;          // 32 KB per (
 constexpr uint32_t kStageBytes = kSlices * (kSliceBytesA + kSliceBytesB);  // 48 KB
 constexpr int kStages = 4;
 constexpr int kEpiWarps = 8;                       // two per tensor-memory lane quarter, each half of the columns
-constexpr int kThreads = 32 * (2 + kEpiWarps);     // producer warp, MMA warp, epilogue warps
+constexpr int kEpiBatch = 16;                      // entries of C per thread read before the first of them is written
+#ifdef COCONS_I8_PROBE
+constexpr int kProbeWarps = 1;  // the probe build's observer of the stage refills
+#else
+constexpr int kProbeWarps = 0;
+#endif
+constexpr int kThreads = 32 * (2 + kEpiWarps + kProbeWarps);  // producer warp, MMA warp, epilogue warps (, observer)
 constexpr int kSplitThreads = 128;
 constexpr int kSmemBytes = kStages * kStageBytes + 1024;  // + alignment of the stages to 1 KB
 constexpr int kTmemCols = 512;
@@ -231,8 +237,8 @@ constexpr int kW = 2 * kCM / kCN, kBand = kBandRows / kCM;
 
 // Probe build (-DCOCONS_I8_PROBE, tools/syrk_i8_probe.py): per-CTA cycle counts summed over the launch
 #ifdef COCONS_I8_PROBE
-__device__ unsigned long long g_i8_probe[8];  // start->first MMA, MMA full waits, producer empty waits, epilogue,
-                                              // MMA waits for tensor memory, CTA cycles, tiles, CTAs
+__device__ unsigned long long g_i8_probe[9];  // start->first MMA, MMA full waits, producer empty waits, epilogue,
+                                              // MMA waits for tensor memory, CTA cycles, tiles, CTAs, stage refills
 #define I8_PROBE(...) __VA_ARGS__
 #else
 #define I8_PROBE(...)
@@ -257,6 +263,7 @@ __global__ void __launch_bounds__(kThreads, 1)
   extern __shared__ uint8_t smem_raw[];
   __shared__ __align__(8) uint64_t bars[2 * kStages + 2];
   __shared__ uint32_t tmem_slot;
+  I8_PROBE(__shared__ long long issue_t[kStages];)  // clock64 of each stage's copy issue
   I8_PROBE(const long long t_start = clock64();)
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int rank = (int)(blockIdx.x % kCtas), rm = rank / kCN, cn = rank % kCN;
@@ -286,7 +293,7 @@ __global__ void __launch_bounds__(kThreads, 1)
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   if (kCtas > 1) cluster_sync();  // every barrier of the cluster is initialised before a multicast reaches it
   const uint32_t tmem = tmem_slot;
-  I8_PROBE(unsigned long long p_first = 0, p_full = 0, p_empty = 0, p_epi = 0, p_tmem = 0, p_tiles = 0;)
+  I8_PROBE(unsigned long long p_first = 0, p_full = 0, p_empty = 0, p_epi = 0, p_tmem = 0, p_tiles = 0, p_refill = 0;)
 
   if (warp == 0) {
     if (lane == 0) {
@@ -317,6 +324,7 @@ __global__ void __launch_bounds__(kThreads, 1)
             I8_PROBE(p_empty += clock64() - t0;)
           }
           const uint32_t fb = full0 + 8 * slot, da = stage0 + slot * kStageBytes, db = da + kSlices * kSliceBytesA;
+          I8_PROBE(*(volatile long long*)&issue_t[slot] = clock64();)
           mbar_expect_tx(fb, kStageBytes);
           const uint32_t aoff = cn * (kBlockBytes / kCN);
           if (kCN > 1)
@@ -375,6 +383,21 @@ __global__ void __launch_bounds__(kThreads, 1)
         I8_PROBE(++p_tiles;)
       }
     }
+#ifdef COCONS_I8_PROBE
+  } else if (warp == 2 + kEpiWarps) {
+    // observer: the cycles from each stage's copy issue to its full barrier completing, whether or not the MMA thread
+    // is waiting for it then.  issue_t[slot] is rewritten only after the MMAs have read the stage, long after this
+    if (lane == 0) {
+      uint32_t it = 0;
+      bool ok = true;
+      for (int64_t st = cluster; ok && st < nsuper; st += nclusters)
+        for (int c = 0; ok && c < kChunks; ++c, ++it) {
+          const uint32_t slot = it % kStages;
+          ok = mbar_wait(full0 + 8 * slot, (it / kStages) & 1, info);
+          if (ok) p_refill += clock64() - *(volatile long long*)&issue_t[slot];
+        }
+    }
+#endif
   } else {
     // epilogue: C_ij -= ((hi 2^-35 + lo 2^-63) s_i) s_j.  Warp w reads tensor-memory lanes (tile rows) 32 (w % 4) ..,
     // columns 32 h .. 32 h + 31 with h = (w - 2) / 4
@@ -418,10 +441,15 @@ __global__ void __launch_bounds__(kThreads, 1)
       if (store) {
         const double si = sa[(int64_t)bi * kRowsA + r];
         const double* sbj = sb + (int64_t)bj * kRowsB + 32 * h;
+        // all loads of a batch before its first store: the compiler cannot move a load of C above a store to C (the
+        // addresses differ by the runtime ldc), so one load per store would cost one L2 round trip per entry
 #pragma unroll
-        for (int j = 0; j < 32; ++j) {
-          double* p = Cg + (int64_t)j * ldc;
-          __stcs(p, __ldcs(p) - (v[j] * si) * sbj[j]);
+        for (int j0 = 0; j0 < 32; j0 += kEpiBatch) {
+          double c[kEpiBatch], s[kEpiBatch];
+#pragma unroll
+          for (int j = 0; j < kEpiBatch; ++j) c[j] = __ldcs(Cg + (int64_t)(j0 + j) * ldc), s[j] = sbj[j0 + j];
+#pragma unroll
+          for (int j = 0; j < kEpiBatch; ++j) __stcs(Cg + (int64_t)(j0 + j) * ldc, c[j] - (v[j0 + j] * si) * s[j]);
         }
       }
       I8_PROBE(if (tid == 64) p_epi += clock64() - t0;)
@@ -440,7 +468,8 @@ __global__ void __launch_bounds__(kThreads, 1)
     atomicAdd(&g_i8_probe[5], (unsigned long long)(clock64() - t_start)), atomicAdd(&g_i8_probe[6], p_tiles);
     atomicAdd(&g_i8_probe[7], 1ull);
   } if (tid == 0) atomicAdd(&g_i8_probe[2], p_empty);
-           if (tid == 64) atomicAdd(&g_i8_probe[3], p_epi);)
+           if (tid == 64) atomicAdd(&g_i8_probe[3], p_epi);
+           if (tid == 32 * (2 + kEpiWarps)) atomicAdd(&g_i8_probe[8], p_refill);)
 }
 
 namespace {
@@ -501,7 +530,7 @@ struct Register {
 // the probe sums of the launches since the last call, then zero (probe build only)
 extern "C" int cocons_i8_probe_read(unsigned long long* out) {
   if (cudaMemcpyFromSymbol(out, cocons::g_i8_probe, sizeof(cocons::g_i8_probe)) != cudaSuccess) return -1;
-  const unsigned long long zero[8] = {};
+  const unsigned long long zero[9] = {};
   return cudaMemcpyToSymbol(cocons::g_i8_probe, zero, sizeof(zero)) == cudaSuccess ? 0 : -1;
 }
 #endif

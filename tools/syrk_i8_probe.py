@@ -11,6 +11,8 @@ Counters (clock64, SM cycles), all from the update kernel:
   producer_empty_wait the producer waiting for a stage to be freed (the tensor pipe is the limit)
   epilogue            per tile: the epilogue, from its accumulators being complete to its last store of C
   mma_tmem_wait       the MMA-issuing thread waiting for the epilogue to hand tensor memory back (epilogue exposed)
+  stage_refill        per stage: the producer issuing a stage's copies to the stage's full barrier completing (the
+                      refill latency; seen by an observer warp that only the probe build has)
 """
 import argparse
 import concurrent.futures
@@ -25,7 +27,8 @@ import tempfile
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 NAMES = ("start_to_first_mma", "mma_full_wait", "producer_empty_wait", "epilogue", "mma_tmem_wait", "cta_cycles",
-         "tiles", "ctas")
+         "tiles", "ctas", "stage_refill")
+CHUNKS = 24  # stages per tile (K = 768 in chunks of 32)
 
 
 def card():
@@ -61,7 +64,7 @@ def main():
     L.cocons_trailing_update.argtypes = [ctypes.c_int, ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int,
                                          ctypes.c_int, ctypes.POINTER(ctypes.c_double)]
     L.cocons_last_error.restype = ctypes.c_char_p
-    sums = (ctypes.c_ulonglong * 8)()
+    sums = (ctypes.c_ulonglong * len(NAMES))()
     before = card()
     ms = ctypes.c_double()
     if L.cocons_trailing_update(0, a.rows, None, None, 1, 1, ctypes.byref(ms)) != 0:  # warm-up
@@ -78,6 +81,7 @@ def main():
          "ctas_per_launch": ctas / (a.reps + 1), "tiles_per_launch": tiles / (a.reps + 1),
          "cycles_per_cta": {"start_to_first_mma": s["start_to_first_mma"] / ctas, "cta_cycles": s["cta_cycles"] / ctas},
          "cycles_per_tile": per_tile, "share_of_cta_cycles": {k: s[k] / s["cta_cycles"] for k in NAMES[:5]},
+         "stage_refill_cycles": s["stage_refill"] / (tiles * CHUNKS),
          "card": before, "card_after": card()}
     print(json.dumps(r, indent=1), flush=True)
     if a.out:
