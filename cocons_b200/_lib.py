@@ -55,6 +55,7 @@ SIGNATURES = {
     "cocons_factor": (ctypes.c_int, [_vp, ctypes.c_int, _dp, _dp]),
     "cocons_predict": (ctypes.c_int, [_vp, _i64, _dp, _dp, _dp, _dp, _dp]),
     "cocons_sim": (ctypes.c_int, [_vp, _i64, _dp, _dp]),
+    "cocons_sim_taper": (ctypes.c_int, [_vp, _i64, _dp, _dp]),
     "cocons_sim_cond": (ctypes.c_int, [_vp, _i64, _dp, _dp, _i64, _dp, _dp]),
     "cocons_ctx_get_factor": (ctypes.c_int, [_vp, _dp, _lp]),
     "cocons_ctx_factor_rows": (ctypes.c_int, [_vp, _lp, _i64, _dp, _lp]),

@@ -410,6 +410,14 @@ class DenseLikelihood:
         _lib.check(_lib.lib().cocons_sim(self._h, eps.shape[1], _lib.ptr(eps), _lib.ptr(out)))
         return out
 
+    def sim_taper(self, eps):
+        """L eps with the tapered factor kept by factor_taper / terms_taper (cocons_sim_taper); on a dense context
+        the same bits as sim()."""
+        eps = _lib.fmat(eps, rows=self.n)
+        out = np.empty_like(eps, order="F")
+        _lib.check(_lib.lib().cocons_sim_taper(self._h, eps.shape[1], _lib.ptr(eps), _lib.ptr(out)))
+        return out
+
     def sim_cond(self, locs_pred, x_covariates_pred, eps):
         lp, Xp = _lib.fmat(locs_pred), _lib.fmat(x_covariates_pred)
         m = Xp.shape[0]
@@ -447,9 +455,10 @@ class DenseLikelihood:
 class TaperedLikelihood(DenseLikelihood):
     """A context for the tapered model only (cocons_ctx_create_taper_tiled): the pattern of `ref_taper` (a `spam`,
     n x n) is fixed at creation and only the tiles of the Cholesky factor that can be nonzero are stored on the
-    device - so n is bounded by the factor's fill, not by n^2.  terms_taper / factor_taper / get_factor /
-    factor_rows / set_z / timings work as on a DenseLikelihood (and so do GetNeg2loglikelihoodTaper{,Profile}
-    with ctx=); the dense objectives, prediction and simulation raise CoconsError.  At most 128 columns of z."""
+    device - so n is bounded by the factor's fill, not by n^2.  terms_taper / factor_taper / predict_taper /
+    sim_taper / get_factor / factor_rows / set_z / timings work as on a DenseLikelihood (and so do
+    GetNeg2loglikelihoodTaper{,Profile} with ctx=); the dense objectives, set_taper, predict, sim and sim_cond raise
+    CoconsError.  At most 128 columns of z."""
 
     def __init__(self, locs, x_covariates, z, ref_taper, device=0, stream=None):
         self.locs, self.X = _lib.fmat(locs), _lib.fmat(x_covariates)
@@ -979,12 +988,15 @@ def getHessian(coco_object, ncores="auto", eps=np.finfo(float).eps ** 0.25, devi
     return H
 
 
-def cocoPredict(coco_object, newdataset, newlocs, type="mean", index_pred=0, device=0):
+def cocoPredict(coco_object, newdataset, newlocs, type="mean", index_pred=0, device=0, tiled=False):
     """R/predict.R:84-288: kriging mean and (type "pred") standard deviation, dense and sparse (tapered)
     branches.  The reference solves with LU (`solve`) / spam's sparse solve; here the Cholesky factor on the
-    device is used."""
+    device is used.  `tiled` (sparse objects only): factor and solve on a TaperedLikelihood, which stores only the
+    factor's nonzero tiles - for sizes whose dense matrix does not fit the device."""
     if not coco_object.output:
         raise ValueError("coco object has not yet been fitted.")
+    if tiled and coco_object.type != "sparse":
+        raise ValueError("tiled = True is for sparse coco objects.")
     dm = getDesignMatrix(coco_object.model_list, coco_object.data)
     eff = getModelLists(coco_object.output["par"], dm["par.pos"], "diff")
     X_std = getScale(dm["model.matrix"], coco_object.info["mean.vector"], coco_object.info["sd.vector"])["std.covs"]
@@ -992,9 +1004,14 @@ def cocoPredict(coco_object, newdataset, newlocs, type="mean", index_pred=0, dev
     X_pred = getScale(dmp["model.matrix"], coco_object.info["mean.vector"], coco_object.info["sd.vector"])["std.covs"]
     systematic = X_pred @ eff["mean"]
     resid = coco_object.z[:, index_pred] - X_std @ eff["mean"]
-    with DenseLikelihood(coco_object.locs, X_std, coco_object.z, device=device) as ctx:
+    if tiled:
+        ctx = TaperedLikelihood(coco_object.locs, X_std, coco_object.z, _ref_taper(coco_object), device=device)
+    else:
+        ctx = DenseLikelihood(coco_object.locs, X_std, coco_object.z, device=device)
+    with ctx:
         if coco_object.type == "sparse":  # R/predict.R:190-288: tapered Sigma and tapered cross-covariance
-            ctx.set_taper(_ref_taper(coco_object))
+            if not tiled:
+                ctx.set_taper(_ref_taper(coco_object))
             ctx.factor_taper(eff, coco_object.info["smooth.limits"])
             sto, expl = ctx.predict_taper(newlocs, X_pred, _ref_taper(coco_object, rows=newlocs), resid,
                                           want_explained=(type == "pred"))
@@ -1011,9 +1028,12 @@ def cocoPredict(coco_object, newdataset, newlocs, type="mean", index_pred=0, dev
 
 
 def cocoSim(coco_object, pars=None, n=1, seed=None, standardize=True, type="classic", sim_type=None, cond_info=None,
-            device=0, eps=None):
-    """R/sim.R:52-175, dense branch.  The N(0,1) draws come from numpy's legacy generator seeded
-    with `seed` (R's come from set.seed/rnorm; pass `eps` to supply R's own draws)."""
+            device=0, eps=None, tiled=False):
+    """R/sim.R:52-218, dense and sparse branches.  The N(0,1) draws come from numpy's legacy generator seeded
+    with `seed` (R's come from set.seed/rnorm; pass `eps` to supply R's own draws).  `tiled` (sparse objects,
+    marginal draws only): factor and draw on a TaperedLikelihood, which stores only the factor's nonzero tiles."""
+    if tiled and (coco_object.type != "sparse" or sim_type == "cond"):
+        raise ValueError("tiled = True is for the marginal draws of sparse coco objects.")
     if pars is None:
         pars, type = coco_object.output["par"], "diff"
     dm = getDesignMatrix(coco_object.model_list, coco_object.data)
@@ -1044,6 +1064,12 @@ def cocoSim(coco_object, pars=None, n=1, seed=None, standardize=True, type="clas
     nsites = std_coco.shape[0]
     if eps is None:
         eps = rng.standard_normal((nsites, n))
+    if tiled:
+        with TaperedLikelihood(coco_object.locs, std_coco, coco_object.z, _ref_taper(coco_object),
+                               device=device) as ctx:
+            ctx.factor_taper(theta_to_fit, coco_object.info["smooth.limits"])
+            draws = ctx.sim_taper(eps)
+        return draws + (std_coco @ theta_to_fit["mean"])[:, None]
     with DenseLikelihood(coco_object.locs, std_coco, coco_object.z, device=device) as ctx:
         if coco_object.type == "sparse":
             # R/sim.R:176-218.  The reference draws t(eps) %*% chol_spam(P Sigma P') un-permuted; any factor of

@@ -257,6 +257,7 @@ struct cocons_ctx {
   double* dPool = nullptr;                        // the stored tiles
   int64_t pool_elems = 0;
   int64_t *dTiles = nullptr, *dMaps = nullptr;    // assembly tile map (TaperSink::tiles); update / scatter maps
+  int64_t* dRowMap = nullptr;                     // the stored tiles by tile row (launch_tiled_forward / _product)
   double *dNegI = nullptr, *dLogPart = nullptr;   // -I (128 x rhs_k); log-determinant of each diagonal tile
   double* dCheck = nullptr;  // COCONS_DEBUG_CHECKSUM: 296 partials + [assembly, factor] sums
   double check[2] = {0, 0};
@@ -305,6 +306,21 @@ static int upload_sorted(cocons_ctx* c, const double* src, int64_t k, double* ds
   COCONS_CUDA_TRY(cudaStreamSynchronize(c->stream));
   return 0;
 }
+
+// device buffers of one call, freed on every way out
+struct CallBuffers {
+  std::vector<void*> held;
+  template <class T>
+  bool get(T** p, int64_t count) {
+    *p = nullptr;
+    if (cudaMalloc(p, sizeof(T) * (size_t)std::max<int64_t>(count, 1)) != cudaSuccess) return false;
+    held.push_back(*p);
+    return true;
+  }
+  ~CallBuffers() {
+    for (void* p : held) cudaFree(p);
+  }
+};
 
 extern "C" {
 
@@ -446,6 +462,7 @@ void cocons_ctx_destroy(cocons_ctx* c) {
   cudaFree(c->dOrig), cudaFree(c->dA), cudaFree(c->dRhs);
   cudaFree(c->dTapCol), cudaFree(c->dTapRow), cudaFree(c->dInv), cudaFree(c->dTap), cudaFree(c->dCheck);
   cudaFree(c->dPool), cudaFree(c->dTiles), cudaFree(c->dMaps), cudaFree(c->dNegI), cudaFree(c->dLogPart);
+  cudaFree(c->dRowMap);
   solve_workspace_destroy(&c->ws);
   chol_workspace_destroy(&c->ws);
   cudaFree(c->dGram);
@@ -532,7 +549,8 @@ int cocons_ctx_create(int device, int64_t n, int64_t p, int64_t r, const double*
 static int refuse_tiled(cocons_ctx* c, const char* who) {
   if (!c || !c->tiled) return 0;
   set_error("%s: not available on a tiled tapered context (cocons_ctx_create_taper_tiled); it supports "
-            "cocons_n2ll_taper, cocons_factor_taper, cocons_ctx_get_factor and cocons_ctx_factor_rows", who);
+            "cocons_n2ll_taper, cocons_factor_taper, cocons_predict_taper, cocons_sim_taper, cocons_ctx_get_factor "
+            "and cocons_ctx_factor_rows", who);
   return COCONS_ERR_STATE;
 }
 
@@ -655,6 +673,24 @@ static void tile_maps(cocons_ctx* c, std::vector<int64_t>* maps) {
   c->scat_at = (int64_t)maps->size();
   for (int64_t J = 0; J < c->T; ++J) maps->push_back(c->base[(size_t)J] + c->ldp[(size_t)J] - kTile);
   for (int64_t J = 0; J < c->T; ++J) maps->push_back(c->ldp[(size_t)J]);
+}
+
+// The stored tiles by tile row, for the substitutions and the product (common.cuh, launch_tiled_forward): columns are
+// visited in increasing J, so the entries of a row come in increasing J with the diagonal tile last.
+static std::vector<int64_t> tile_row_map(const cocons_ctx* c) {
+  const int64_t T = c->T, nst = c->nstored;
+  std::vector<int64_t> map((size_t)(T + 1 + 3 * nst), 0);
+  for (int64_t k = 0; k < nst; ++k) ++map[(size_t)c->rows[(size_t)k] + 1];
+  for (int64_t I = 0; I < T; ++I) map[(size_t)I + 1] += map[(size_t)I];
+  std::vector<int64_t> at(map.begin(), map.begin() + T);
+  for (int64_t J = 0; J < T; ++J)
+    for (int64_t k = c->colptr[(size_t)J]; k < c->colptr[(size_t)J + 1]; ++k) {
+      const int64_t e = at[(size_t)c->rows[(size_t)k]]++;
+      map[(size_t)(T + 1 + e)] = J;
+      map[(size_t)(T + 1 + nst + e)] = c->base[(size_t)J] + (k - c->colptr[(size_t)J]) * kTile;
+      map[(size_t)(T + 1 + 2 * nst + e)] = c->ldp[(size_t)J];
+    }
+  return map;
 }
 
 // Right-looking factorisation over the column panels, in order, on the context's stream: every target tile receives
@@ -965,6 +1001,7 @@ int cocons_ctx_create_taper_tiled(int device, int64_t n, int64_t p, int64_t r, c
   std::copy(c->colptr.begin(), c->colptr.end(), tiles.begin());
   std::copy(c->rows.begin(), c->rows.end(), tiles.begin() + c->T + 1);
   tile_maps(c, &maps);
+  const std::vector<int64_t> rmap = tile_row_map(c);
   c->rhs_k = std::max<int64_t>(16, round_up(r, 16));
   std::vector<double> negi((size_t)kTile * c->rhs_k, 0.0);
   for (int64_t k = 0; k < c->rhs_k; ++k) negi[(size_t)(k * kTile + k)] = -1.0;
@@ -975,6 +1012,8 @@ int cocons_ctx_create_taper_tiled(int device, int64_t n, int64_t p, int64_t r, c
   CTX_TRY(cudaMalloc(&c->dMaps, sizeof(int64_t) * maps.size()));
   CTX_TRY(cudaMalloc(&c->dNegI, sizeof(double) * negi.size()));
   CTX_TRY(cudaMalloc(&c->dLogPart, sizeof(double) * c->T));
+  CTX_TRY(cudaMalloc(&c->dRowMap, sizeof(int64_t) * rmap.size()));
+  CTX_TRY(cudaMemcpy(c->dRowMap, rmap.data(), sizeof(int64_t) * rmap.size(), cudaMemcpyHostToDevice));
   CTX_TRY(cudaMemcpy(c->dTiles, tiles.data(), sizeof(int64_t) * tiles.size(), cudaMemcpyHostToDevice));
   CTX_TRY(cudaMemcpy(c->dMaps, maps.data(), sizeof(int64_t) * maps.size(), cudaMemcpyHostToDevice));
   CTX_TRY(cudaMemcpy(c->dNegI, negi.data(), sizeof(double) * negi.size(), cudaMemcpyHostToDevice));
@@ -1222,6 +1261,9 @@ struct PredBlock {
 // the prediction pattern of the tapered model (pred_taper, R/predict.R:233-249): m rows x n columns
 struct TaperPred {
   const int32_t* rowpointers = nullptr;  // host, 1-based
+  const int32_t* colindices = nullptr;   // host
+  const double* taper = nullptr;         // host
+  int64_t nnz = 0;
   int *dCol = nullptr, *dRow = nullptr;
   double* dTap = nullptr;
   ~TaperPred() { cudaFree(dCol), cudaFree(dRow), cudaFree(dTap); }
@@ -1270,9 +1312,11 @@ static int refresh_table_for_pred(cocons_ctx* c) {
   return 0;
 }
 
+static int predict_tiled(cocons_ctx* c, int64_t m, const double* locs_pred, const double* Xp, const double* resid,
+                         double* stochastic, double* explained, const TaperPred& tp);
+
 static int predict_impl(cocons_ctx* c, int64_t m, const double* locs_pred, const double* Xp, const double* resid,
                         double* stochastic, double* explained, const TaperPred* tp) {
-  if (int rc_ = refuse_tiled(c, "predict")) return rc_;
   if (!c || m <= 0 || !locs_pred || !Xp || !resid || !stochastic) {
     set_error("predict: bad argument");
     return COCONS_ERR_ARG;
@@ -1296,6 +1340,7 @@ static int predict_impl(cocons_ctx* c, int64_t m, const double* locs_pred, const
     // cov_rns_taper_pred always takes the smoothness through the logistic, for both site sets (:54-70)
     launch_taper_site_stage(c->n, (int)c->p, c->dX, c->n_pad, c->dLocs, c->n_pad, c->dTheta, c->lim[0], c->lim[1],
                             SM_GENERAL, 0, c->taper_table(), c->stream);
+    if (c->tiled) return predict_tiled(c, m, locs_pred, Xp, resid, stochastic, explained, *tp);
   } else if ((rc = refresh_table_for_pred(c))) {
     return rc;
   }
@@ -1351,6 +1396,7 @@ static int predict_impl(cocons_ctx* c, int64_t m, const double* locs_pred, const
 
 int cocons_predict(cocons_ctx* c, int64_t m, const double* locs_pred, const double* Xp, const double* resid,
                    double* stochastic, double* explained) {
+  if (int rc_ = refuse_tiled(c, "predict")) return rc_;
   return predict_impl(c, m, locs_pred, Xp, resid, stochastic, explained, nullptr);
 }
 
@@ -1378,7 +1424,6 @@ int cocons_factor_taper(cocons_ctx* c, const double* theta6, const double* limit
 int cocons_predict_taper(cocons_ctx* c, int64_t m, const double* locs_pred, const double* Xp,
                          const int32_t* colindices, const int32_t* rowpointers, const double* taper_entries,
                          int64_t nnz, const double* resid, double* stochastic, double* explained) {
-  if (int rc_ = refuse_tiled(c, "predict_taper")) return rc_;
   if (!c || m <= 0 || !taper_entries) {
     set_error("predict_taper: bad argument");
     return COCONS_ERR_ARG;
@@ -1387,7 +1432,7 @@ int cocons_predict_taper(cocons_ctx* c, int64_t m, const double* locs_pred, cons
   if (rc) return rc;
   cudaSetDevice(c->device);
   TaperPred tp;
-  tp.rowpointers = rowpointers;
+  tp.rowpointers = rowpointers, tp.colindices = colindices, tp.taper = taper_entries, tp.nnz = nnz;
   const int64_t nz = std::max<int64_t>(nnz, 1);
   COCONS_CUDA_TRY(cudaMalloc(&tp.dCol, sizeof(int) * nz));
   COCONS_CUDA_TRY(cudaMalloc(&tp.dRow, sizeof(int) * (m + 1)));
@@ -1398,17 +1443,8 @@ int cocons_predict_taper(cocons_ctx* c, int64_t m, const double* locs_pred, cons
   return predict_impl(c, m, locs_pred, Xp, resid, stochastic, explained, &tp);
 }
 
-int cocons_sim(cocons_ctx* c, int64_t k, const double* eps, double* out) {
-  if (int rc_ = refuse_tiled(c, "sim")) return rc_;
-  if (!c || k <= 0 || !eps || !out) {
-    set_error("sim: bad argument");
-    return COCONS_ERR_ARG;
-  }
-  if (!c->factor_valid) {
-    set_error("sim: no factor kept (call cocons_factor first)");
-    return COCONS_ERR_STATE;
-  }
-  cudaSetDevice(c->device);
+// out = L eps with the dense context's factor (R/sim.R:172)
+static int sim_dense(cocons_ctx* c, int64_t k, const double* eps, double* out) {
   const int64_t np = c->n_pad;
   cudaStream_t st = c->stream;
   double *dE = nullptr, *dO = nullptr;
@@ -1435,6 +1471,167 @@ int cocons_sim(cocons_ctx* c, int64_t k, const double* eps, double* out) {
   for (int64_t col = 0; col < k; ++col)
     for (int64_t s = 0; s < c->n; ++s) out[(size_t)col * c->n + c->perm[(size_t)s]] = h[(size_t)col * np + s];
   return 0;
+}
+
+static int sim_tiled(cocons_ctx* c, int64_t k, const double* eps, double* out);
+
+int cocons_sim(cocons_ctx* c, int64_t k, const double* eps, double* out) {
+  if (int rc_ = refuse_tiled(c, "sim")) return rc_;
+  if (!c || k <= 0 || !eps || !out) {
+    set_error("sim: bad argument");
+    return COCONS_ERR_ARG;
+  }
+  if (!c->factor_valid) {
+    set_error("sim: no factor kept (call cocons_factor first)");
+    return COCONS_ERR_STATE;
+  }
+  cudaSetDevice(c->device);
+  return sim_dense(c, k, eps, out);
+}
+
+int cocons_sim_taper(cocons_ctx* c, int64_t k, const double* eps, double* out) {
+  if (!c || k <= 0 || !eps || !out) {
+    set_error("sim_taper: bad argument");
+    return COCONS_ERR_ARG;
+  }
+  if (!c->factor_valid || !c->factor_is_taper) {
+    set_error("sim_taper: no tapered factor kept (call cocons_factor_taper first)");
+    return COCONS_ERR_STATE;
+  }
+  cudaSetDevice(c->device);
+  return c->tiled ? sim_tiled(c, k, eps, out) : sim_dense(c, k, eps, out);
+}
+
+static TiledArgs tiled_args(const cocons_ctx* c, int64_t ldb) {
+  TiledArgs a{};
+  a.pool = c->dPool, a.rmap = c->dRowMap, a.tiles = c->dTiles, a.winv = c->ws.winv;
+  a.T = c->T, a.ldb = ldb, a.info = c->ws.info;
+  return a;
+}
+
+// out = L eps through the stored tiles (K8c); eps goes up row-major (n_pad x round_up(k, 8)) in the context's order
+static int sim_tiled(cocons_ctx* c, int64_t k, const double* eps, double* out) {
+  const int64_t np = c->n_pad, ldb = round_up(k, 8);
+  cudaStream_t st = c->stream;
+  CallBuffers buf;
+  double *dE, *dO;
+  TiledArgs* dArgs;
+  if (!buf.get(&dE, np * ldb) || !buf.get(&dO, np * ldb) || !buf.get(&dArgs, 1)) {
+    set_error("sim_taper: out of device memory");
+    return COCONS_ERR_ALLOC;
+  }
+  std::vector<double> h((size_t)(np * ldb), 0.0);
+  for (int64_t s = 0; s < c->n; ++s)
+    for (int64_t col = 0; col < k; ++col) h[(size_t)(s * ldb + col)] = eps[(size_t)col * c->n + c->perm[(size_t)s]];
+  COCONS_CUDA_TRY(cudaMemcpyAsync(dE, h.data(), sizeof(double) * h.size(), cudaMemcpyHostToDevice, st));
+  TiledArgs a = tiled_args(c, ldb);
+  a.E = dE, a.B = dO;
+  launch_tiled_product(a, dArgs, st);
+  COCONS_CUDA_TRY(cudaGetLastError());
+  COCONS_CUDA_TRY(cudaMemcpyAsync(h.data(), dO, sizeof(double) * h.size(), cudaMemcpyDeviceToHost, st));
+  COCONS_CUDA_TRY(cudaStreamSynchronize(st));
+  for (int64_t s = 0; s < c->n; ++s)
+    for (int64_t col = 0; col < k; ++col) out[(size_t)col * c->n + c->perm[(size_t)s]] = h[(size_t)(s * ldb + col)];
+  return 0;
+}
+
+// cocons_predict_taper on a tiled context (the training table already carries the logistic smoothness).  No m x n_pad
+// block is formed:
+//   stochastic = C w with w = L^-T L^-1 resid (K8a + K8b on one column), over the pattern entries of C only;
+//   explained_i = |L^-1 c_i|^2: the sites with pattern entries, ordered by their first neighbour in the context's
+//   order, go in blocks of 128 columns; each block's C' is written by the TS_ROWS sink into a row-major n_pad x 128
+//   block and forward-substituted (K8a) from the tile row of that first neighbour on - the rows above stay zero.
+static int predict_tiled(cocons_ctx* c, int64_t m, const double* locs_pred, const double* Xp, const double* resid,
+                         double* stochastic, double* explained, const TaperPred& tp) {
+  constexpr int64_t kb = kTile;  // prediction sites per explained block
+  const int64_t np = c->n_pad, n = c->n, p = c->p, T = c->T, nnz = tp.nnz;
+  cudaStream_t st = c->stream;
+  CallBuffers buf;
+  double *dXp, *dLp, *dSp, *dY, *dW, *dSto;
+  unsigned* dCtrl;
+  TiledArgs* dArgs;  // rewritten before every launch, in stream order
+  if (!buf.get(&dXp, m * p) || !buf.get(&dLp, m * 2) || !buf.get(&dSp, TF_COUNT * m) || !buf.get(&dY, np * 8) ||
+      !buf.get(&dW, np) || !buf.get(&dSto, m) || !buf.get(&dCtrl, 3 + T * (kb / 32)) ||
+      !buf.get(&dArgs, 1)) {
+    set_error("predict_taper: out of device memory");
+    return COCONS_ERR_ALLOC;
+  }
+  COCONS_CUDA_TRY(cudaMemcpyAsync(dXp, Xp, sizeof(double) * m * p, cudaMemcpyHostToDevice, st));
+  COCONS_CUDA_TRY(cudaMemcpyAsync(dLp, locs_pred, sizeof(double) * m * 2, cudaMemcpyHostToDevice, st));
+  const TaperTable P{dSp, m};
+  launch_taper_site_stage(m, (int)p, dXp, m, dLp, m, c->dTheta, c->lim[0], c->lim[1], SM_GENERAL, 1, P, st);
+  // w = L^-T L^-1 resid
+  std::vector<double> hr((size_t)(np * 8), 0.0);
+  for (int64_t s = 0; s < n; ++s) hr[(size_t)(s * 8)] = resid[c->perm[(size_t)s]];
+  COCONS_CUDA_TRY(cudaMemcpyAsync(dY, hr.data(), sizeof(double) * hr.size(), cudaMemcpyHostToDevice, st));
+  TiledArgs a = tiled_args(c, 8);
+  a.B = dY, a.ctrl = dCtrl;
+  launch_tiled_forward(a, dArgs, st);
+  a.E = dY, a.B = dW;
+  launch_tiled_backward(a, dArgs, st);
+  // stochastic = C w over the pattern, one thread per prediction row
+  launch_taper_entries(0, m, m, tp.dCol, tp.dRow, P, c->taper_table(), 0, SM_GENERAL, 0.0,
+                       TaperSink{TS_ROWDOT, dSto, tp.dTap, c->dInv, dW, 0, 0, nullptr}, st);
+  COCONS_CUDA_TRY(cudaGetLastError());
+  COCONS_CUDA_TRY(cudaMemcpyAsync(stochastic, dSto, sizeof(double) * m, cudaMemcpyDeviceToHost, st));
+  COCONS_CUDA_TRY(cudaStreamSynchronize(st));  // hr goes out of scope
+  if (explained) {
+    std::fill(explained, explained + m, 0.0);  // a site without pattern entries explains nothing
+    std::vector<int64_t> inv((size_t)n), first((size_t)m, INT64_MAX), order;
+    for (int64_t s = 0; s < n; ++s) inv[(size_t)c->perm[(size_t)s]] = s;
+    for (int64_t i = 0; i < m; ++i) {
+      for (int64_t e = tp.rowpointers[i] - 1; e < tp.rowpointers[i + 1] - 1; ++e)
+        first[(size_t)i] = std::min(first[(size_t)i], inv[(size_t)tp.colindices[e] - 1]);
+      if (first[(size_t)i] < INT64_MAX) order.push_back(i);
+    }
+    std::stable_sort(order.begin(), order.end(), [&](int64_t a, int64_t b) { return first[(size_t)a] < first[(size_t)b]; });
+    // the pattern, the design and the locations of those sites in that order
+    const int64_t ms = (int64_t)order.size();
+    std::vector<int32_t> rps((size_t)ms + 1, 1), cols;
+    std::vector<double> taps, xs((size_t)(ms * p)), ls((size_t)(ms * 2));
+    cols.reserve((size_t)nnz), taps.reserve((size_t)nnz);
+    for (int64_t a = 0; a < ms; ++a) {
+      const int64_t i = order[(size_t)a];
+      for (int64_t e = tp.rowpointers[i] - 1; e < tp.rowpointers[i + 1] - 1; ++e)
+        cols.push_back(tp.colindices[e]), taps.push_back(tp.taper[e]);
+      rps[(size_t)a + 1] = (int32_t)(cols.size() + 1);
+      for (int64_t k = 0; k < p; ++k) xs[(size_t)(k * ms + a)] = Xp[(size_t)(k * m + i)];
+      for (int64_t k = 0; k < 2; ++k) ls[(size_t)(k * ms + a)] = locs_pred[(size_t)(k * m + i)];
+    }
+    double *dXs, *dLs, *dSs, *dTs, *dB, *dSq, *dEx;
+    int *dCs, *dRs;
+    if (!buf.get(&dXs, ms * p) || !buf.get(&dLs, ms * 2) || !buf.get(&dSs, TF_COUNT * ms) ||
+        !buf.get(&dTs, (int64_t)taps.size()) || !buf.get(&dCs, (int64_t)cols.size()) || !buf.get(&dRs, ms + 1) ||
+        !buf.get(&dB, np * kb) || !buf.get(&dSq, T * kb) || !buf.get(&dEx, ms)) {
+      set_error("predict_taper: out of device memory");
+      return COCONS_ERR_ALLOC;
+    }
+    if (ms > 0) {
+      COCONS_CUDA_TRY(cudaMemcpyAsync(dXs, xs.data(), sizeof(double) * xs.size(), cudaMemcpyHostToDevice, st));
+      COCONS_CUDA_TRY(cudaMemcpyAsync(dLs, ls.data(), sizeof(double) * ls.size(), cudaMemcpyHostToDevice, st));
+      COCONS_CUDA_TRY(cudaMemcpyAsync(dTs, taps.data(), sizeof(double) * taps.size(), cudaMemcpyHostToDevice, st));
+      COCONS_CUDA_TRY(cudaMemcpyAsync(dCs, cols.data(), sizeof(int32_t) * cols.size(), cudaMemcpyHostToDevice, st));
+      COCONS_CUDA_TRY(cudaMemcpyAsync(dRs, rps.data(), sizeof(int32_t) * rps.size(), cudaMemcpyHostToDevice, st));
+      launch_taper_site_stage(ms, (int)p, dXs, ms, dLs, ms, c->dTheta, c->lim[0], c->lim[1], SM_GENERAL, 1,
+                              TaperTable{dSs, ms}, st);
+    }
+    for (int64_t i0 = 0; i0 < ms; i0 += kb) {
+      const int64_t cnt = std::min(kb, ms - i0), I0 = first[(size_t)order[(size_t)i0]] / kTile;
+      COCONS_CUDA_TRY(cudaMemsetAsync(dB + I0 * kTile * kb, 0, sizeof(double) * (np - I0 * kTile) * kb, st));
+      launch_taper_entries(rps[(size_t)i0] - 1, rps[(size_t)(i0 + cnt)] - rps[(size_t)i0], ms, dCs, dRs,
+                           TaperTable{dSs + i0, ms}, c->taper_table(), 0, SM_GENERAL, 0.0,
+                           TaperSink{TS_ROWS, nullptr, dTs, c->dInv, dB, kb, i0, nullptr}, st);
+      TiledArgs f = tiled_args(c, kb);
+      f.B = dB, f.I0 = I0, f.ctrl = dCtrl, f.sumsq = dSq, f.out = dEx + i0, f.count = cnt;
+      launch_tiled_forward(f, dArgs, st);
+    }
+    COCONS_CUDA_TRY(cudaGetLastError());
+    std::vector<double> he((size_t)ms);
+    COCONS_CUDA_TRY(cudaMemcpyAsync(he.data(), dEx, sizeof(double) * ms, cudaMemcpyDeviceToHost, st));
+    COCONS_CUDA_TRY(cudaStreamSynchronize(st));
+    for (int64_t a = 0; a < ms; ++a) explained[order[(size_t)a]] = he[(size_t)a];
+  }
+  return solve_status(c, "predict_taper");
 }
 
 int cocons_sim_cond(cocons_ctx* c, int64_t m, const double* locs_pred, const double* Xp, int64_t k, const double* eps,

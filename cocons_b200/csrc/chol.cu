@@ -114,6 +114,255 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
                : "memory");
 }
 
+// ---------------------------------------------------------------------------
+// Tiled tapered context (capi.cu, cocons_ctx_create_taper_tiled): the solves and the product with the factor through
+// its stored tiles, for prediction and simulation.  They run in instantiations gemm_nt_tma_kernel<64, 2, op> of their
+// own (op = kTiledFwd8 ... kTiledTrmm32, see the kernel), on its 256 threads and dynamic shared memory, and reuse its
+// DMMA fragment; the other instantiations compile exactly as before.  Arguments: one TiledArgs in device memory.
+// Right-hand sides are row-major (n_pad x ldb, element (s, c) at s ldb + c), which is what taper_entries_kernel's
+// TS_ROWS sink writes for a block of ldb prediction rows.
+//   K8a forward   L Y = B in place, work unit = (tile row, slice of 8 NT columns), one dataflow launch
+//   K8b backward  L^T x = y for one column
+//   K8c product   O = L E
+// Every sum runs in a fixed order (tiles in increasing J, k inside a tile in mma order), whatever the schedule.
+// ---------------------------------------------------------------------------
+constexpr int kTiledFwd8 = 3, kTiledFwd32 = 4, kTiledBwd = 5, kTiledTrmm8 = 6, kTiledTrmm32 = 7;
+constexpr unsigned kTiledSpinLimit = 1u << 25;  // ~seconds; a healthy wait ends within microseconds
+
+// acc[mt][nt] += L_tile (rows r0 + 8 mt + g) x Y (128 x 8 NT, row-major, ldb), k = 0..127; diag: only L's lower
+// triangle (the stored diagonal tile holds update leftovers above it)
+template <int NT>
+__device__ __forceinline__ void tiled_tile_mma(double (&acc)[2][NT][2], const double* __restrict__ Lt, int64_t ld,
+                                               const double* Y, int64_t ldb, int r0, int g, int c4, bool diag) {
+#pragma unroll 8
+  for (int kk = 0; kk < kTile / 4; ++kk) {
+    const int k = 4 * kk + c4;
+    double a[2], b[NT];
+#pragma unroll
+    for (int mt = 0; mt < 2; ++mt) {
+      const int row = r0 + 8 * mt + g;
+      a[mt] = __ldg(Lt + (int64_t)k * ld + row);
+      if (diag && k > row) a[mt] = 0.0;
+    }
+#pragma unroll
+    for (int nt = 0; nt < NT; ++nt) b[nt] = __ldcg(Y + (int64_t)k * ldb + 8 * nt + g);
+#pragma unroll
+    for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+      for (int nt = 0; nt < NT; ++nt) dmma884(acc[mt][nt][0], acc[mt][nt][1], a[mt], b[nt]);
+  }
+}
+
+// thread 0 polls *flag until it is set; false = gave up (error raised for everybody)
+__device__ __forceinline__ bool tiled_wait(unsigned* flag, unsigned* ctrl, int* info, int* s_bad) {
+  if (threadIdx.x == 0) {
+    unsigned spins = 0;
+    int bad = 0;
+    while (atomicAdd(flag, 0u) == 0u) {
+      if (++spins > 64) __nanosleep(64);
+      if ((spins & 1023u) == 0 && (spins > kTiledSpinLimit || atomicAdd(ctrl + 1, 0u) != 0u)) {
+        bad = 1;
+        atomicExch(ctrl + 1, 1u);
+        atomicCAS(info, 0, COCONS_ERR_CUDA);
+        break;
+      }
+    }
+    __threadfence();
+    *s_bad = bad;
+  }
+  __syncthreads();
+  const bool ok = (*s_bad == 0);
+  __syncthreads();
+  return ok;
+}
+
+// the next work unit from the ticket counter ctrl[0], broadcast to the CTA
+__device__ __forceinline__ unsigned tiled_ticket(unsigned* ctrl, unsigned* s_u) {
+  if (threadIdx.x == 0) *s_u = atomicAdd(ctrl, 1u);
+  __syncthreads();
+  const unsigned u = *s_u;
+  __syncthreads();
+  return u;
+}
+
+// K8a.  Work unit u = (tile row I = I0 + u / nsl, column slice s = u % nsl), handed out in that order, so a unit waits
+// only for units of earlier rows - no deadlock whatever is resident.
+//   t = B_I - sum_{J stored, I0 <= J < I} L_IJ Y_J   (J ascending; Y_J for J < I0 is zero: B is zero above row I0)
+//   Y_I = W_I t  over B_I;  flag (I, s) = ctrl[2 + I nsl + s] released
+// With a.sumsq: sumsq[I ldb + c] = sum over tile row I of Y(., c)^2 in row order, and the unit that finishes last
+// (counter ctrl[2 + T nsl]) writes out[c] = sum_{I >= I0} sumsq[I ldb + c], c < count, in tile-row order.
+template <int NT>
+__device__ void tiled_forward(const TiledArgs& a, double* smem) {
+  constexpr int NC = 8 * NT;
+  double(*tsm)[NC + 1] = reinterpret_cast<double(*)[NC + 1]>(smem);
+  unsigned* s_u = reinterpret_cast<unsigned*>(smem + kTile * (NC + 1));
+  int* s_bad = reinterpret_cast<int*>(s_u + 1);
+  const int tid = threadIdx.x, lane = tid & 31, g = lane >> 2, c4 = lane & 3, r0 = (tid >> 5) * 16;
+  const int64_t T = a.T, I0 = a.I0, ldb = a.ldb, nsl = ldb / NC;
+  const int64_t nent = a.rmap[T];
+  const int64_t *rp = a.rmap, *ej = rp + T + 1, *eoff = ej + nent, *eld = eoff + nent;
+  unsigned* ctrl = a.ctrl;
+  const unsigned nunits = (unsigned)((T - I0) * nsl);
+  for (;;) {
+    const unsigned u = tiled_ticket(ctrl, s_u);
+    if (u >= nunits) break;
+    const int64_t I = I0 + u / nsl;
+    const int s = (int)(u % nsl), c0 = s * NC;
+    double acc[2][NT][2];
+#pragma unroll
+    for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+      for (int nt = 0; nt < NT; ++nt) acc[mt][nt][0] = acc[mt][nt][1] = 0.0;
+    for (int64_t e = rp[I]; e < rp[I + 1] - 1; ++e) {
+      const int64_t J = ej[e];
+      if (J < I0) continue;
+      if (!tiled_wait(ctrl + 2 + J * nsl + s, ctrl, a.info, s_bad)) return;
+      tiled_tile_mma<NT>(acc, a.pool + eoff[e], eld[e], a.B + J * kTile * ldb + c0, ldb, r0, g, c4, false);
+    }
+    double* BI = a.B + I * kTile * ldb + c0;
+#pragma unroll
+    for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+      for (int nt = 0; nt < NT; ++nt)
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          const int row = r0 + 8 * mt + g, col = 8 * nt + 2 * c4 + h;
+          tsm[row][col] = BI[(int64_t)row * ldb + col] - acc[mt][nt][h];
+          acc[mt][nt][h] = 0.0;
+        }
+    __syncthreads();
+    const double* W = a.winv + I * (int64_t)kTile * kTile;  // explicit zeros above the diagonal
+#pragma unroll 8
+    for (int kk = 0; kk < kTile / 4; ++kk) {
+      const int k = 4 * kk + c4;
+      double av[2], bv[NT];
+#pragma unroll
+      for (int mt = 0; mt < 2; ++mt) av[mt] = __ldg(W + (int64_t)k * kTile + r0 + 8 * mt + g);
+#pragma unroll
+      for (int nt = 0; nt < NT; ++nt) bv[nt] = tsm[k][8 * nt + g];
+#pragma unroll
+      for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+        for (int nt = 0; nt < NT; ++nt) dmma884(acc[mt][nt][0], acc[mt][nt][1], av[mt], bv[nt]);
+    }
+    __syncthreads();  // every read of t is done
+#pragma unroll
+    for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+      for (int nt = 0; nt < NT; ++nt)
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          const int row = r0 + 8 * mt + g, col = 8 * nt + 2 * c4 + h;
+          BI[(int64_t)row * ldb + col] = acc[mt][nt][h];
+          tsm[row][col] = acc[mt][nt][h];
+        }
+    __threadfence();
+    __syncthreads();
+    if (tid == 0) atomicExch(ctrl + 2 + I * nsl + s, 1u);
+    if (a.sumsq) {
+      if (tid < NC) {
+        double q = 0.0;
+        for (int r = 0; r < kTile; ++r) q = fma(tsm[r][tid], tsm[r][tid], q);
+        a.sumsq[I * ldb + c0 + tid] = q;
+      }
+      __threadfence();
+      __syncthreads();
+      if (tid == 0) *s_u = atomicAdd(ctrl + 2 + T * nsl, 1u);
+      __syncthreads();
+      if (*s_u == nunits - 1) {  // every unit's sums are out: the column totals
+        __threadfence();
+        for (int64_t c = tid; c < a.count; c += blockDim.x) {
+          double t = 0.0;
+          for (int64_t J = I0; J < T; ++J) t += __ldcg(a.sumsq + J * ldb + c);
+          a.out[c] = t;
+        }
+      }
+    }
+    __syncthreads();  // tsm and s_u are rewritten by the next unit
+  }
+}
+
+// K8b.  Work unit u = tile column J = T - 1 - u (ticket order), waiting only for later columns:
+//   x_J = W_J^T (y_J - sum_{I stored below J} L_IJ^T x_I)   (I ascending), flag J = ctrl[2 + J]
+// Warp w owns the 16 columns 16 w .. 16 w + 15 of the tile; lane l sums rows l, l + 32, l + 64, l + 96 of each over
+// all I, then the lanes are reduced in a fixed butterfly.  y = a.E with stride a.ldb, x = a.B contiguous.
+__device__ void tiled_backward(const TiledArgs& a, double* smem) {
+  double *xs = smem, *ts = smem + kTile;
+  unsigned* s_u = reinterpret_cast<unsigned*>(smem + 2 * kTile);
+  int* s_bad = reinterpret_cast<int*>(s_u + 1);
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+  const int64_t T = a.T, nst = a.tiles[T];
+  const int64_t *cp = a.tiles, *rows = cp + T + 1, *offs = rows + nst, *ldp = offs + nst;
+  auto reduce = [&](double v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_sync(0xffffffffu, v, lane ^ o);
+    return v;
+  };
+  for (;;) {
+    const unsigned u = tiled_ticket(a.ctrl, s_u);
+    if (u >= (unsigned)T) break;
+    const int64_t J = T - 1 - u, ld = ldp[J];
+    double p[16];
+#pragma unroll
+    for (int c = 0; c < 16; ++c) p[c] = 0.0;
+    for (int64_t k = cp[J] + 1; k < cp[J + 1]; ++k) {
+      const int64_t I = rows[k];
+      if (!tiled_wait(a.ctrl + 2 + I, a.ctrl, a.info, s_bad)) return;
+      if (tid < kTile) xs[tid] = __ldcg(a.B + I * kTile + tid);
+      __syncthreads();
+      const double* Lt = a.pool + offs[k] + (int64_t)(16 * w) * ld;
+#pragma unroll
+      for (int c = 0; c < 16; ++c)
+#pragma unroll
+        for (int q = 0; q < 4; ++q) p[c] = fma(__ldg(Lt + (int64_t)c * ld + lane + 32 * q), xs[lane + 32 * q], p[c]);
+      __syncthreads();
+    }
+#pragma unroll
+    for (int c = 0; c < 16; ++c) {
+      const double v = reduce(p[c]);
+      if (lane == 0) ts[16 * w + c] = a.E[(J * kTile + 16 * w + c) * a.ldb] - v;
+    }
+    __syncthreads();
+    const double* W = a.winv + J * (int64_t)kTile * kTile + (int64_t)(16 * w) * kTile;  // (W^T t)_jj = W(:, jj) . t
+#pragma unroll
+    for (int c = 0; c < 16; ++c) {
+      double v = 0.0;
+#pragma unroll
+      for (int q = 0; q < 4; ++q) v = fma(__ldg(W + (int64_t)c * kTile + lane + 32 * q), ts[lane + 32 * q], v);
+      v = reduce(v);
+      if (lane == 0) a.B[J * kTile + 16 * w + c] = v;
+    }
+    __threadfence();
+    __syncthreads();
+    if (tid == 0) atomicExch(a.ctrl + 2 + J, 1u);
+  }
+}
+
+// K8c.  CTA b = (tile row I = b / nsl, column slice b % nsl): O_I = sum_{J stored, J <= I} L_IJ E_J (J ascending, the
+// diagonal last); O = a.B
+template <int NT>
+__device__ void tiled_product(const TiledArgs& a) {
+  const int tid = threadIdx.x, lane = tid & 31, g = lane >> 2, c4 = lane & 3, r0 = (tid >> 5) * 16;
+  const int64_t T = a.T, ldb = a.ldb, nsl = ldb / (8 * NT);
+  const int64_t I = blockIdx.x / nsl, c0 = (int64_t)(blockIdx.x % nsl) * 8 * NT;
+  const int64_t nent = a.rmap[T];
+  const int64_t *rp = a.rmap, *ej = rp + T + 1, *eoff = ej + nent, *eld = eoff + nent;
+  double acc[2][NT][2];
+#pragma unroll
+  for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+    for (int nt = 0; nt < NT; ++nt) acc[mt][nt][0] = acc[mt][nt][1] = 0.0;
+  for (int64_t e = rp[I]; e < rp[I + 1]; ++e)
+    tiled_tile_mma<NT>(acc, a.pool + eoff[e], eld[e], a.E + ej[e] * kTile * ldb + c0, ldb, r0, g, c4, ej[e] == I);
+#pragma unroll
+  for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+    for (int nt = 0; nt < NT; ++nt)
+#pragma unroll
+      for (int h = 0; h < 2; ++h)
+        a.B[(I * kTile + r0 + 8 * mt + g) * ldb + c0 + 8 * nt + 2 * c4 + h] = acc[mt][nt][h];
+}
+
 // ASSIGN 0: C -= A B^T; 1: C = A B^T; 2 (kGemmMapped): C -= A B^T with every 128 x 128 block of C looked up in a
 // tile map, so that one launch updates tiles scattered over the panels of a tiled factor.  In that mode `ldc`
 // carries the device address of the map, int64: [pairs: element offset of the target block from C][128-column
@@ -127,6 +376,15 @@ __global__ void __launch_bounds__(GemmCfg<BN, NU>::kThreads, GemmCfg<BN, NU>::kM
   constexpr int kWarps = Cfg::kThreads / 32;
   constexpr uint32_t kStageBytes = GBK * (GBM + BN) * (uint32_t)sizeof(double);
   extern __shared__ __align__(16) double smem[];
+  if constexpr (ASSIGN >= kTiledFwd8) {  // the tiled context's solves and product (see above), ldc = &TiledArgs
+    const TiledArgs& ta = *reinterpret_cast<const TiledArgs*>(ldc);
+    if constexpr (ASSIGN == kTiledFwd8) tiled_forward<1>(ta, smem);
+    if constexpr (ASSIGN == kTiledFwd32) tiled_forward<4>(ta, smem);
+    if constexpr (ASSIGN == kTiledBwd) tiled_backward(ta, smem);
+    if constexpr (ASSIGN == kTiledTrmm8) tiled_product<1>(ta);
+    if constexpr (ASSIGN == kTiledTrmm32) tiled_product<4>(ta);
+    return;
+  }
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (size_t)GSTAGES * Cfg::kStageDoubles);
   const int tid = threadIdx.x;
   const int warp = tid >> 5, lane = tid & 31;
@@ -916,6 +1174,56 @@ int chol_factor(double* A, int64_t n_pad, int64_t ld, CholWorkspace ws, cudaStre
     cudaStreamWaitEvent(st, ws.ev_p, 0);
   }
   return 0;
+}
+
+// ---- launches of the tiled context's solves and product: one TiledArgs goes up to `slot` (device) first ----------
+
+template <int OP>
+static void launch_tiled_op(const TiledArgs& a, TiledArgs* slot, int64_t grid, cudaStream_t st) {
+  static bool attr_done[16] = {};
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (dev < 16 && !attr_done[dev]) {
+    cudaFuncSetAttribute(gemm_nt_tma_kernel<64, 2, OP>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                         GemmCfg<64, 2>::kSmemBytes + 64);
+    attr_done[dev] = true;
+  }
+  // a pageable source is staged before cudaMemcpyAsync returns: `a` may go out of scope right after
+  cudaMemcpyAsync(slot, &a, sizeof(TiledArgs), cudaMemcpyHostToDevice, st);
+  note_launch();
+  launch_gemm_64<OP>((int)grid, 1, 0, nullptr, 0, nullptr, 0, nullptr, (int64_t)(uintptr_t)slot, 0, st);
+}
+
+static int64_t resident_ctas() {  // two CTAs of the GEMM's shape per SM
+  static int sms[16] = {};
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (dev < 16 && sms[dev] == 0) cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev);
+  return 2 * (int64_t)((dev < 16 && sms[dev] > 0) ? sms[dev] : 148);
+}
+
+void launch_tiled_forward(const TiledArgs& a, TiledArgs* slot, cudaStream_t st) {
+  if (a.I0 >= a.T) return;
+  const bool wide = a.ldb % 32 == 0;
+  const int64_t nsl = a.ldb / (wide ? 32 : 8), nunits = (a.T - a.I0) * nsl;
+  cudaMemsetAsync(a.ctrl, 0, sizeof(unsigned) * (size_t)(3 + a.T * nsl), st);
+  const int64_t grid = std::min(nunits, resident_ctas());
+  if (wide)
+    launch_tiled_op<kTiledFwd32>(a, slot, grid, st);
+  else
+    launch_tiled_op<kTiledFwd8>(a, slot, grid, st);
+}
+
+void launch_tiled_backward(const TiledArgs& a, TiledArgs* slot, cudaStream_t st) {
+  cudaMemsetAsync(a.ctrl, 0, sizeof(unsigned) * (size_t)(2 + a.T), st);
+  launch_tiled_op<kTiledBwd>(a, slot, std::min(a.T, resident_ctas()), st);
+}
+
+void launch_tiled_product(const TiledArgs& a, TiledArgs* slot, cudaStream_t st) {
+  if (a.ldb % 32 == 0)
+    launch_tiled_op<kTiledTrmm32>(a, slot, a.T * (a.ldb / 32), st);
+  else
+    launch_tiled_op<kTiledTrmm8>(a, slot, a.T * (a.ldb / 8), st);
 }
 
 }  // namespace cocons

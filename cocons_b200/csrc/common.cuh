@@ -88,13 +88,13 @@ struct TaperTable {
 void launch_taper_site_stage(int64_t n, int p, const double* dX, int64_t ldx, const double* dlocs, int64_t ldl,
                              const double* dtheta6, double lim0, double lim1, int mode, int pred_rows, TaperTable T,
                              cudaStream_t st);
-enum TaperSinkKind { TS_VECTOR = 0, TS_LOWER = 1, TS_ROWS = 2, TS_TILED = 3 };
+enum TaperSinkKind { TS_VECTOR = 0, TS_LOWER = 1, TS_ROWS = 2, TS_TILED = 3, TS_ROWDOT = 4 };
 struct TaperSink {
   int kind;
-  double* out;          // TS_VECTOR: nnz values in pattern order
-  const double* taper;  // TS_LOWER / TS_ROWS / TS_TILED: taper values on the pattern, multiplied in
+  double* out;          // TS_VECTOR: nnz values in pattern order; TS_ROWDOT: one value per pattern row
+  const double* taper;  // TS_LOWER / TS_ROWS / TS_TILED / TS_ROWDOT: taper values on the pattern, multiplied in
   const int* inv;       // caller index -> position in the context's ordering
-  double* A;            // dense sink; TS_TILED: the tile pool
+  double* A;            // dense sink; TS_TILED: the tile pool; TS_ROWDOT: the vector w (context order)
   int64_t ld;           // TS_TILED: number of tile columns T
   int64_t row0;         // TS_ROWS: first pattern row of the block; TS_TILED: number of stored tiles
   // TS_TILED: the tile map, int64 [T + 1 column starts][stored tiles: tile row][stored tiles: element offset of the
@@ -103,6 +103,8 @@ struct TaperSink {
 };
 // the tiled sink runs in instantiations of taper_entries_kernel<mode + kTaperTiled> of their own
 constexpr int kTaperTiled = 8;
+// ... and the row-dot sink (TS_ROWDOT, general smoothness only) in taper_entries_kernel<SM_GENERAL + kTaperRowDot>
+constexpr int kTaperRowDot = 16;
 // entries [e0, e0 + count) of the pattern (nrows rows)
 void launch_taper_entries(int64_t e0, int64_t count, int64_t nrows, const int* dcol, const int* drow, TaperTable R,
                           TaperTable C, int square, int mode, double nu_fixed, TaperSink S, cudaStream_t st);
@@ -141,6 +143,27 @@ int chol_outer(int64_t n_pad);  // tiles per outer panel of chol_factor
 void launch_potrf_tile(double* A, int64_t ld, double* Winv, int* info, int first_index, cudaStream_t st);
 void launch_gemm_nt(int mode, int64_t M, int64_t N, int64_t K, const double* A, int64_t lda, const double* B,
                     int64_t ldb, double* C, int64_t ldc, int lower_only, cudaStream_t st);
+// Tiled tapered context (K8a-c in chol.cu, run by gemm_nt_tma_kernel instantiations of their own).  Right-hand sides
+// are row-major n_pad x ldb, ldb a multiple of 8.  A dependency wait that does not end (a bug) sets *info =
+// COCONS_ERR_CUDA instead of hanging.  Each launch first copies its TiledArgs to `slot` (device memory).
+struct TiledArgs {
+  const double* pool;    // the stored tiles
+  const int64_t* rmap;   // by tile row: int64 [T + 1 row starts][entries: J][entries: pool offset][entries: ld], J
+                         // increasing inside a row, the diagonal tile last
+  const int64_t* tiles;  // by tile column: TaperSink::tiles
+  const double* winv;    // inverted diagonal tiles
+  int64_t T, I0, ldb;    // tile rows; first tile row of the forward sweep (B is zero above it); row stride
+  double* B;             // forward: B, solved in place; backward: x (contiguous); product: the output
+  const double* E;       // backward: y (stride ldb); product: the input
+  unsigned* ctrl;        // scratch: 3 + T * ldb / 8 words
+  double* sumsq;         // forward, or null: T x ldb per-tile-row sums of squares of Y ...
+  double* out;           // ... and their column totals from row I0 on, `count` of them
+  int64_t count;
+  int* info;
+};
+void launch_tiled_forward(const TiledArgs& a, TiledArgs* slot, cudaStream_t st);   // L Y = B
+void launch_tiled_backward(const TiledArgs& a, TiledArgs* slot, cudaStream_t st);  // L^T x = y, one column
+void launch_tiled_product(const TiledArgs& a, TiledArgs* slot, cudaStream_t st);   // O = L E
 
 // ---- syrk_i8.cu: the K = 768 trailing update C -= P P^T as exact products of int8 slices on the tensor cores
 // (tcgen05, kind::i8), combined in FP64.  syrk_i8.cu fills g_syrk_i8 when it is linked in; a build of the sources

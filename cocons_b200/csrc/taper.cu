@@ -106,15 +106,36 @@ __device__ __forceinline__ int64_t taper_row_of(const int* __restrict__ rowpoint
 //   TS_TILED    as TS_LOWER, into the tile pool of a tiled context: tile (hi / 128, lo / 128) is found by a binary
 //               search over the stored tile rows of column lo / 128 (TaperSink::tiles).  Only the instantiations
 //               MODE = smoothness mode + kTaperTiled take this sink; the others compile exactly as before.
+//   TS_ROWDOT   ONE THREAD PER PATTERN ROW i (count = nrows, e0 = 0): out[i] = sum_e taper[e] value_e A[inv[j_e]] over
+//               the row's entries in pattern order (rows from table R at i, columns at inv[j] of the context's table
+//               C): the kriging mean C w of the tiled context, w = Sigma^-1 resid.  Instantiation
+//               SM_GENERAL + kTaperRowDot of its own.
 template <int MODE>
 __global__ void __launch_bounds__(256) taper_entries_kernel(int64_t e0, int64_t count, int64_t nrows,
                                                             const int* __restrict__ colindices,
                                                             const int* __restrict__ rowpointers, TaperTable R,
                                                             TaperTable C, int square, double nu_fixed, TaperSink S) {
-  constexpr bool kTiled = MODE >= kTaperTiled;
-  constexpr int kMode = kTiled ? MODE - kTaperTiled : MODE;
+  constexpr bool kRowDot = MODE >= kTaperRowDot;
+  constexpr bool kTiled = MODE >= kTaperTiled && !kRowDot;
+  constexpr int kMode = kRowDot ? MODE - kTaperRowDot : (kTiled ? MODE - kTaperTiled : MODE);
   const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= count) return;
+  if constexpr (kRowDot) {
+    double s = 0.0;
+    for (int64_t e = rowpointers[t] - 1; e < rowpointers[t + 1] - 1; ++e) {
+      const int64_t sj = S.inv[colindices[e] - 1];
+      const double xi = R.f(TF_X)[t], yi = R.f(TF_Y)[t], xj = C.f(TF_X)[sj], yj = C.f(TF_Y)[sj];
+      bool same = (xi == xj && yi == yj);
+      double v = 0.0;
+      if (!same)
+        v = taper_pair<kMode>(R.f(TF_R)[t], R.f(TF_SIG)[t], R.f(TF_NU)[t], C.f(TF_R)[sj], C.f(TF_SIG)[sj],
+                              C.f(TF_NU)[sj], __dsub_rn(xi, xj), __dsub_rn(yi, yj), nu_fixed, same);
+      if (same) v = R.f(TF_DV)[t];
+      s = fma(__dmul_rn(S.taper[e], v), S.A[sj], s);
+    }
+    S.out[t] = s;
+    return;
+  }
   const int64_t e = e0 + t;
   const int64_t i = taper_row_of(rowpointers, nrows, e);
   const int64_t j = (int64_t)colindices[e] - 1;
@@ -175,7 +196,7 @@ void launch_taper_entries(int64_t e0, int64_t count, int64_t nrows, const int* d
   note_launch();
 #define COCONS_TAPER_LAUNCH(M) \
   taper_entries_kernel<M><<<blocks, 256, 0, st>>>(e0, count, nrows, dcol, drow, R, C, square, nu_fixed, S)
-  switch (mode + (S.kind == TS_TILED ? kTaperTiled : 0)) {
+  switch (mode + (S.kind == TS_TILED ? kTaperTiled : (S.kind == TS_ROWDOT ? kTaperRowDot : 0))) {
     case SM_HALF: COCONS_TAPER_LAUNCH(SM_HALF); break;
     case SM_THREEHALF: COCONS_TAPER_LAUNCH(SM_THREEHALF); break;
     case SM_FIVEHALF: COCONS_TAPER_LAUNCH(SM_FIVEHALF); break;
@@ -185,6 +206,7 @@ void launch_taper_entries(int64_t e0, int64_t count, int64_t nrows, const int* d
     case SM_FIVEHALF + kTaperTiled: COCONS_TAPER_LAUNCH(SM_FIVEHALF + kTaperTiled); break;
     case SM_DEGENERATE + kTaperTiled: COCONS_TAPER_LAUNCH(SM_DEGENERATE + kTaperTiled); break;
     case SM_GENERAL + kTaperTiled: COCONS_TAPER_LAUNCH(SM_GENERAL + kTaperTiled); break;
+    case SM_GENERAL + kTaperRowDot: COCONS_TAPER_LAUNCH(SM_GENERAL + kTaperRowDot); break;
     default: COCONS_TAPER_LAUNCH(SM_GENERAL); break;
   }
 #undef COCONS_TAPER_LAUNCH

@@ -146,4 +146,10 @@ GetNeg2loglikelihoodTaperProfile <- function(theta, par.pos, ref_taper, locs, x_
 #   pr <- .Call(`_cocons_ctx_predict_taper`, ctx, newlocs, X_pred_std$std.covs, pred_taper@colindices,
 #               pred_taper@rowpointers, pred_taper@entries, coco.resid)
 #   stochastic_part <- pr[[1]];  spam::rowSums(pred_taper * t(inv_cov)) == pr[[2]]   (:259, :274)
-# and `_cocons_ctx_sim` for the marginal draws (same distribution as t(iiderrors) %*% cholS un-permuted).
+# and `_cocons_ctx_sim_taper` (or `_cocons_ctx_sim`) for the marginal draws (same distribution as
+# t(iiderrors) %*% cholS un-permuted).  At sizes whose dense matrix does not fit, the same sequence runs on a tiled
+# context, which takes no `_cocons_ctx_set_taper` (its pattern is fixed at creation):
+#   ctx <- .Call(`_cocons_ctx_new_taper_tiled`, locs, X_std$std.covs, as.matrix(z), taper_two@colindices,
+#                taper_two@rowpointers, taper_two@entries, 0L)
+#   .Call(`_cocons_ctx_factor_taper`, ctx, ...);  pr <- .Call(`_cocons_ctx_predict_taper`, ctx, ...)
+#   draws <- .Call(`_cocons_ctx_sim_taper`, ctx, iiderrors)

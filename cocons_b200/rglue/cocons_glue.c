@@ -445,6 +445,19 @@ SEXP _cocons_ctx_sim(SEXP ptr, SEXP epsS) {
   return out;
 }
 
+/* n x k draws L eps with the kept tapered factor, dense or tiled context (sparse cocoSim, R/sim.R:193-218) */
+SEXP _cocons_ctx_sim_taper(SEXP ptr, SEXP epsS) {
+  const ctx_view v = view_of(ptr);
+  SEXP eps = PROTECT(as_real(epsS));
+  need(Rf_isMatrix(eps) && Rf_nrows(eps) == v.n, "ctx_sim_taper", "eps must be an n x k matrix");
+  const int n = Rf_nrows(eps), k = Rf_ncols(eps);
+  SEXP out = PROTECT(Rf_allocMatrix(REALSXP, n, k));
+  int rc = cocons_sim_taper(v.c, k, REAL(eps), REAL(out));
+  UNPROTECT(2);
+  raise(rc);
+  return out;
+}
+
 /* m x k conditional draws (R/sim.R:87-121) */
 SEXP _cocons_ctx_sim_cond(SEXP ptr, SEXP locsPredS, SEXP xPredS, SEXP epsS) {
   const ctx_view v = view_of(ptr);
@@ -483,6 +496,7 @@ static const R_CallMethodDef CallEntries[] = {
     {"_cocons_ctx_factor_taper", (DL_FUNC)&_cocons_ctx_factor_taper, 4},
     {"_cocons_ctx_predict_taper", (DL_FUNC)&_cocons_ctx_predict_taper, 7},
     {"_cocons_ctx_sim", (DL_FUNC)&_cocons_ctx_sim, 2},
+    {"_cocons_ctx_sim_taper", (DL_FUNC)&_cocons_ctx_sim_taper, 2},
     {"_cocons_ctx_sim_cond", (DL_FUNC)&_cocons_ctx_sim_cond, 4},
     {NULL, NULL, 0}};
 

@@ -138,9 +138,9 @@ int cocons_ctx_set_taper(cocons_ctx* ctx, const int32_t* colindices, const int32
 /* A context for the tapered model only, with the pattern fixed at creation: only the tiles of L that can be nonzero
  * (pattern + fill, Morton order) are stored, so n is bounded by the factor's fill, not by n_pad^2.  The pattern and
  * taper entries are those of cocons_ctx_set_taper; 0 <= r <= 128.  On such a context cocons_n2ll_taper,
- * cocons_factor_taper, cocons_ctx_get_factor (dense expansion, for small n), cocons_ctx_factor_rows,
- * cocons_ctx_set_z, cocons_ctx_dims, cocons_ctx_timings and cocons_ctx_destroy work as on a dense context; every
- * other context entry returns COCONS_ERR_STATE.  The factor differs from the dense path's in the last bits only. */
+ * cocons_factor_taper, cocons_predict_taper, cocons_sim_taper, cocons_ctx_get_factor (dense expansion, for small n),
+ * cocons_ctx_factor_rows, cocons_ctx_set_z, cocons_ctx_dims, cocons_ctx_timings and cocons_ctx_destroy work as on a
+ * dense context; every other context entry returns COCONS_ERR_STATE.  The factor differs from the dense path's in the last bits only. */
 int cocons_ctx_create_taper_tiled(int device, int64_t n, int64_t p, int64_t r, const double* locs,
                                   const double* x_covariates, const double* z, const int32_t* colindices,
                                   const int32_t* rowpointers, const double* taper_entries, int64_t nnz,
@@ -170,7 +170,10 @@ int cocons_factor_taper(cocons_ctx* ctx, const double* theta6, const double* smo
  * are those of `pred_taper` before its entries are multiplied by
  * cov_rns_taper_pred - that product is formed on the device.  Outputs as
  * cocons_predict: stochastic = resid' Sigma^-1 C' (:259),
- * explained = rowSums(C * t(Sigma^-1 C')) (:274; NULL to skip). */
+ * explained = rowSums(C * t(Sigma^-1 C')) (:274; NULL to skip).
+ * Works on a dense context and on a tiled one (cocons_ctx_create_taper_tiled).  On a tiled context no m x n block
+ * is formed: stochastic = C (Sigma^-1 resid) over the pattern entries, and explained_i = |L^-1 c_i|^2 through the
+ * stored tiles, 128 prediction sites at a time.  A prediction row without pattern entries gives exactly 0 for both. */
 int cocons_predict_taper(cocons_ctx* ctx, int64_t m, const double* locs_pred, const double* x_covariates_pred,
                          const int32_t* colindices, const int32_t* rowpointers, const double* taper_entries,
                          int64_t nnz, const double* resid, double* stochastic, double* explained);
@@ -195,6 +198,11 @@ int cocons_predict(cocons_ctx* ctx, int64_t m, const double* locs_pred, const do
 /* cocoSim marginal branch (R/sim.R:162-172): out (n x k) = t(t(eps) %*% chol(Sigma)),
  * i.e. L eps, eps n x k standard normal draws made by the caller (R's RNG). */
 int cocons_sim(cocons_ctx* ctx, int64_t k, const double* eps, double* out);
+
+/* cocoSim sparse branch (R/sim.R:193-218): out (n x k) = L eps with the tapered factor kept by cocons_factor_taper
+ * (or cocons_n2ll_taper).  On a tiled context the product runs through the stored tiles; on a dense context it is
+ * cocons_sim's own product (the same bits).  COCONS_ERR_STATE when no tapered factor is kept. */
+int cocons_sim_taper(cocons_ctx* ctx, int64_t k, const double* eps, double* out);
 
 /* cocoSim conditional branch (R/sim.R:87-121): Schur complement of the
  * prediction sites given the kept factor, its Cholesky factor applied to eps
