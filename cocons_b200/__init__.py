@@ -7,6 +7,7 @@ reference's R interface; see api.py.
 from .api import (  # noqa: F401
     CoconsError,
     DenseLikelihood,
+    DenseLikelihoodBatch,
     DenseLikelihoodPool,
     GetNeg2loglikelihood,
     GetNeg2loglikelihoodProfile,

@@ -41,6 +41,9 @@ SIGNATURES = {
     "cocons_ctx_set_z": (ctypes.c_int, [_vp, _dp]),
     "cocons_ctx_set_xbetas": (ctypes.c_int, [_vp, _i64, _dp]),
     "cocons_n2ll": (ctypes.c_int, [_vp, ctypes.c_int, _dp, _dp, _dp, _dp, _dp, _dp, _ip]),
+    "cocons_ctx_create_batch": (ctypes.c_int, [ctypes.c_int, _i64, _i64, _i64, _dp, _dp, _dp, _i64, _vp,
+                                               ctypes.POINTER(_vp)]),
+    "cocons_n2ll_batch": (ctypes.c_int, [_vp, ctypes.c_int, _i64, _dp, _dp, _dp, _dp, _dp, _dp, _ip, _ip]),
     "cocons_cov_rns_taper": (ctypes.c_int, [_i64, _i64, _dp, _dp, _dp, _dp, _i32p, _i32p, _i64, _dp]),
     "cocons_cov_rns_taper_pred": (ctypes.c_int, [_i64, _i64, _i64, _dp, _dp, _dp, _dp, _dp, _dp, _i32p, _i32p, _i64,
                                                  _dp]),

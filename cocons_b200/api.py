@@ -452,6 +452,62 @@ class DenseLikelihood:
                 "kernel_ms": kms.value, "kernel_flops": kfl.value}
 
 
+class DenseLikelihoodBatch:
+    """`batch` matrices over the same data on one GPU (cocons_ctx_create_batch): terms_batch evaluates many points per
+    call, up to `batch` of them with one launch per step of the assembly and the factorisation.  Each point's terms are
+    bit for bit those of DenseLikelihood.terms.  For n_pad = ceil(n / 128) * 128 < 16 384 only (CoconsError above)."""
+
+    def __init__(self, locs, x_covariates, z, batch, device=0, stream=None):
+        self.locs, self.X = _lib.fmat(locs), _lib.fmat(x_covariates)
+        self.n, self.p = self.X.shape
+        self.z = _lib.fmat(z, rows=self.n)
+        self.r = self.z.shape[1]
+        self.batch = int(batch)
+        self._h = _lib._vp()
+        _lib.check(_lib.lib().cocons_ctx_create_batch(int(device), self.n, self.p, self.r, _lib.ptr(self.locs),
+                                                      _lib.ptr(self.X), _lib.ptr(self.z), self.batch, stream, self._h))
+        self.q = 0
+
+    close = DenseLikelihood.close
+    __del__ = close
+    __enter__ = DenseLikelihood.__enter__
+    __exit__ = DenseLikelihood.__exit__
+    set_z = DenseLikelihood.set_z
+    set_xbetas = DenseLikelihood.set_xbetas
+
+    def terms_batch(self, kind, theta_lists, smooth_limits, means=None):
+        """[terms of point i] for the named theta lists: per point the dict DenseLikelihood.terms returns, or that
+        point's NotPositiveDefinite (returned, not raised).  `means`: one mean vector per point, or None."""
+        k = len(theta_lists)
+        th = np.asfortranarray(np.stack([_lib.pack_theta(t, self.p).reshape(-1) for t in theta_lists], axis=1))
+        lim = np.ascontiguousarray(np.asarray(smooth_limits, dtype=np.float64))
+        mean_m = None if means is None else np.asfortranarray(
+            np.stack([np.asarray(m, dtype=np.float64).reshape(self.p) for m in means], axis=1))
+        logdet, ldw = np.zeros(k), np.zeros(k)
+        quad = np.zeros((self.r, k), order="F")
+        rank = _lib.ctypes.c_int()
+        status = np.zeros(k, dtype=np.int32)
+        _lib.check(_lib.lib().cocons_n2ll_batch(self._h, int(kind), k, _lib.ptr(th), _lib.ptr(lim), _lib.ptr(mean_m),
+                                                _lib.ptr(logdet), _lib.ptr(quad), _lib.ptr(ldw),
+                                                _lib.ctypes.byref(rank),
+                                                status.ctypes.data_as(_lib.ctypes.POINTER(_lib.ctypes.c_int))))
+        out = []
+        for i in range(k):
+            if status[i] > 0:
+                out.append(NotPositiveDefinite(int(status[i])))
+            else:
+                _lib.check(int(status[i]))
+                out.append({"logdet": float(logdet[i]), "quad": quad[:, i].copy(), "logdet_w": float(ldw[i]),
+                            "rank": rank.value})
+        return out
+
+    def timings(self):
+        """phase times of the last terms_batch call, added up over its groups of `batch` points"""
+        ms = np.empty(4)
+        _lib.check(_lib.lib().cocons_ctx_timings(self._h, _lib.ptr(ms)))
+        return {"assembly_ms": ms[0], "factor_ms": ms[1], "solve_ms": ms[2], "total_ms": ms[3]}
+
+
 class TaperedLikelihood(DenseLikelihood):
     """A context for the tapered model only (cocons_ctx_create_taper_tiled): the pattern of `ref_taper` (a `spam`,
     n x n) is fixed at creation and only the tiles of the Cholesky factor that can be nonzero are stored on the
@@ -525,6 +581,21 @@ def _objective(kind, theta, par_pos, locs, x_covariates, smooth_limits, z, n, la
             return 1e6  # R/neg2loglikelihood.R:138-142, 202-206, 261-265
         raise ArithmeticError("Cholesky error")
     return _combine(kind, t, n, r, lambda_, theta_list, smooth_limits)
+
+
+def _objectives_batch(kind, thetas, par_pos, smooth_limits, n, lambda_, safe, bctx):
+    """_objective at every point of `thetas` through one DenseLikelihoodBatch.terms_batch call: the same values, bit for
+    bit; with safe=False the first point that is not PD, in point order, raises"""
+    lists = [getModelLists(t, par_pos, "diff") for t in thetas]
+    out = []
+    for tl, t in zip(lists, bctx.terms_batch(kind, lists, smooth_limits, [tl["mean"] for tl in lists])):
+        if isinstance(t, NotPositiveDefinite):
+            if not safe:
+                raise ArithmeticError("Cholesky error")
+            out.append(1e6)
+        else:
+            out.append(_combine(kind, t, n, bctx.r, lambda_, tl, smooth_limits))
+    return out
 
 
 def GetNeg2loglikelihood(theta, par_pos, locs, x_covariates, smooth_limits, z, n, lambda_, safe=True, ctx=None):

@@ -24,10 +24,16 @@ namespace cocons {
 // ---------------------------------------------------------------------------
 __device__ __forceinline__ double link_exp(double eta) { return __ddiv_rn(1.0, exp(-eta)); }
 
+// BATCH = 1: blockIdx.y is the point of a batch, with its own theta (7 p apart) and site table (SF_COUNT tables apart)
+template <int BATCH>
 __global__ void __launch_bounds__(128) site_stage_kernel(int64_t n, int64_t n_fill, int p, const double* __restrict__ X,
                                                          int64_t ldx, const double* __restrict__ locs, int64_t ldl,
                                                          const double* __restrict__ theta6, double lim0, double lim1,
                                                          int mode, SiteTable T) {
+  if constexpr (BATCH) {
+    theta6 += (int64_t)blockIdx.y * 7 * p;
+    T.base += (int64_t)blockIdx.y * SF_COUNT * T.stride;
+  }
   const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (s >= n_fill) return;
   if (s >= n) {  // padding sites: never used by a real pair
@@ -181,11 +187,20 @@ __device__ __forceinline__ void tri_decode(int64_t t, int& tr, int& tc) {
 #ifndef COCONS_ASM_MINBLOCKS
 #define COCONS_ASM_MINBLOCKS 8
 #endif
-template <int MODE>
+// KMODE = mode + kAsmBatch: the lower triangle of matrix blockIdx.y of a batch (launch_assemble_lower_batch); `ld`
+// carries the device address of the batch's global ranges, the matrices are T.stride x T.stride
+template <int KMODE>
 __global__ void __launch_bounds__(kAsmTile, COCONS_ASM_MINBLOCKS) assemble_lower_kernel(int64_t n, int64_t n_out, SiteTable T,
                                                                   double global_range, double nu_fixed,
                                                                   double* __restrict__ C, int64_t ld, int col_tile0,
                                                                   int slab) {
+  constexpr int MODE = KMODE % kAsmBatch;
+  if constexpr (KMODE >= kAsmBatch) {
+    global_range = reinterpret_cast<const double*>(ld)[blockIdx.y];
+    ld = T.stride;
+    T.base += (int64_t)blockIdx.y * SF_COUNT * T.stride;
+    C += (int64_t)blockIdx.y * ld * ld;
+  }
   // slab == 0: C is the whole matrix, blockIdx.x runs over its lower-triangle tiles.
   // slab == 1: C holds only the tile columns [col_tile0, col_tile0 + gridDim.y) (a column panel of a
   //            distributed matrix); blockIdx.x runs over the tile rows from col_tile0 down.
@@ -399,31 +414,56 @@ int smooth_mode_for(int par, int p, const double* theta6, const double* limits, 
   return SM_GENERAL;
 }
 
+template <int BATCH>
+static void launch_site_stage_k(dim3 grid, int64_t n, int64_t n_fill, int p, const double* dX, int64_t ldx,
+                                const double* dlocs, int64_t ldl, const double* dtheta6, double lim0, double lim1,
+                                int mode, SiteTable T, cudaStream_t st) {
+  site_stage_kernel<BATCH><<<grid, 128, 0, st>>>(n, n_fill, p, dX, ldx, dlocs, ldl, dtheta6, lim0, lim1, mode, T);
+}
+
 void launch_site_stage(int64_t n, int64_t n_fill, int p, const double* dX, int64_t ldx, const double* dlocs,
                        int64_t ldl, const double* dtheta6, double lim0, double lim1, int mode, SiteTable T,
-                       cudaStream_t st) {
+                       cudaStream_t st, int batch) {
   const int threads = 128;
   const unsigned blocks = (unsigned)((n_fill + threads - 1) / threads);
   // the degenerate mode leaves smooth_vector at zero, exactly as the reference does
   note_launch();
-  site_stage_kernel<<<blocks, threads, 0, st>>>(n, n_fill, p, dX, ldx, dlocs, ldl, dtheta6, lim0, lim1, mode, T);
+  if (batch > 0)
+    launch_site_stage_k<1>(dim3(blocks, (unsigned)batch), n, n_fill, p, dX, ldx, dlocs, ldl, dtheta6, lim0, lim1, mode,
+                           T, st);
+  else
+    launch_site_stage_k<0>(dim3(blocks), n, n_fill, p, dX, ldx, dlocs, ldl, dtheta6, lim0, lim1, mode, T, st);
 }
 
+template <int OFF>
 static void launch_assemble_any(int64_t n, int64_t n_out, SiteTable T, double global_range, double nu_fixed, int mode,
                                 double* C, int64_t ld, int col_tile0, int slab, dim3 grid, cudaStream_t st);
 
-void launch_assemble_lower(int64_t n, int64_t n_out, SiteTable T, double global_range, double nu_fixed, int mode,
-                           double* C, int64_t ld, cudaStream_t st) {
-  const int64_t nt = (n_out + kAsmTile - 1) / kAsmTile;
-  const int64_t tiles = nt * (nt + 1) / 2;
-  // ~1200 CTAs fit the GPU at once; measured: holes (990 tiles) 2 / 4 / 8 / 16 / 32 slices -> 1.15 / 0.99 / 0.91 /
-  // 0.87 / 0.89 ms, stripes (4465 tiles) -> 3.58 / 3.45 / 3.41 / 3.46 / 3.59 ms
+// ~1200 CTAs fit the GPU at once; measured: holes (990 tiles) 2 / 4 / 8 / 16 / 32 slices -> 1.15 / 0.99 / 0.91 /
+// 0.87 / 0.89 ms, stripes (4465 tiles) -> 3.58 / 3.45 / 3.41 / 3.46 / 3.59 ms
+static unsigned assemble_slices(int64_t tiles) {
   unsigned slices = tiles < 1500 ? 16u : (tiles < 6000 ? 8u : (tiles < 9600 ? 4u : 1u));
   if (const char* e = getenv("COCONS_ASM_SLICES")) {  // experiment knob: 1, 2, 4, 8, 16, 32
     const int v = atoi(e);
     if (v >= 1 && v <= 32 && (v & (v - 1)) == 0) slices = (unsigned)v;
   }
-  launch_assemble_any(n, n_out, T, global_range, nu_fixed, mode, C, ld, 0, 0, dim3((unsigned)tiles, 1, slices), st);
+  return slices;
+}
+
+void launch_assemble_lower(int64_t n, int64_t n_out, SiteTable T, double global_range, double nu_fixed, int mode,
+                           double* C, int64_t ld, cudaStream_t st) {
+  const int64_t nt = (n_out + kAsmTile - 1) / kAsmTile;
+  const int64_t tiles = nt * (nt + 1) / 2;
+  launch_assemble_any<0>(n, n_out, T, global_range, nu_fixed, mode, C, ld, 0, 0,
+                         dim3((unsigned)tiles, 1, assemble_slices(tiles)), st);
+}
+
+void launch_assemble_lower_batch(int64_t n, int64_t n_out, SiteTable T, const double* dranges, double nu_fixed,
+                                 int mode, double* C, int batch, cudaStream_t st) {
+  const int64_t nt = (n_out + kAsmTile - 1) / kAsmTile;
+  const int64_t tiles = nt * (nt + 1) / 2;
+  launch_assemble_any<kAsmBatch>(n, n_out, T, 0.0, nu_fixed, mode, C, (int64_t)(uintptr_t)dranges, 0, 0,
+                                 dim3((unsigned)tiles, (unsigned)batch, assemble_slices(tiles)), st);
 }
 
 // column panel [col_tile0, col_tile0 + ncol_tiles) of the lower triangle into a slab whose first
@@ -431,7 +471,7 @@ void launch_assemble_lower(int64_t n, int64_t n_out, SiteTable T, double global_
 void launch_assemble_panel(int64_t n, int64_t n_out, SiteTable T, double global_range, double nu_fixed, int mode,
                            double* slab, int64_t ld, int col_tile0, int ncol_tiles, cudaStream_t st) {
   const int64_t nt = (n_out + kAsmTile - 1) / kAsmTile;
-  launch_assemble_any(n, n_out, T, global_range, nu_fixed, mode, slab, ld, col_tile0, 1,
+  launch_assemble_any<0>(n, n_out, T, global_range, nu_fixed, mode, slab, ld, col_tile0, 1,
                       dim3((unsigned)(nt - col_tile0), (unsigned)ncol_tiles), st);
 }
 
@@ -440,16 +480,19 @@ void launch_assemble_cyclic(int64_t n, int64_t n_out, SiteTable T, double global
                             double* slab, int64_t ld, int world, int rank, int64_t nlocal, cudaStream_t st) {
   const int64_t nt = (n_out + kAsmTile - 1) / kAsmTile;
   if (nlocal <= 0 || world > 63) return;
-  launch_assemble_any(n, n_out, T, global_range, nu_fixed, mode, slab, ld, 0, 2 | (world << 4) | (rank << 10),
+  launch_assemble_any<0>(n, n_out, T, global_range, nu_fixed, mode, slab, ld, 0, 2 | (world << 4) | (rank << 10),
                       dim3((unsigned)nt, (unsigned)(nlocal * 4)), st);
 }
 
+// OFF = kAsmBatch: the batched instantiations
+template <int OFF>
 static void launch_assemble_any(int64_t n, int64_t n_out, SiteTable T, double global_range, double nu_fixed, int mode,
                                 double* C, int64_t ld, int col_tile0, int slab, dim3 grid, cudaStream_t st) {
   note_launch();
 #define COCONS_ASM_CASE(M)                                                                          \
   case M:                                                                                           \
-    assemble_lower_kernel<M><<<grid, kAsmTile, 0, st>>>(n, n_out, T, global_range, nu_fixed, C, ld, col_tile0, slab); \
+    assemble_lower_kernel<M + OFF><<<grid, kAsmTile, 0, st>>>(n, n_out, T, global_range, nu_fixed, C, ld, col_tile0, \
+                                                              slab);                                 \
     break;
   switch (mode) {
     COCONS_ASM_CASE(SM_GENERAL)

@@ -261,6 +261,12 @@ struct cocons_ctx {
   double *dNegI = nullptr, *dLogPart = nullptr;   // -I (128 x rhs_k); log-determinant of each diagonal tile
   double* dCheck = nullptr;  // COCONS_DEBUG_CHECKSUM: 296 partials + [assembly, factor] sums
   double check[2] = {0, 0};
+  // batch context (cocons_ctx_create_batch): `batch` matrices back to back in dA, each with its own theta + mean in
+  // dTheta (7p apart), site table in dSite, inverted tiles and info word in ws, global range in dRange and
+  // log-determinant in dLogdetB; hInfo holds `batch` ints, hDown the Gram blocks of a group on their way to the host
+  int64_t batch = 0;
+  double *dRange = nullptr, *dLogdetB = nullptr, *hDown = nullptr;
+  int64_t down_cap = 0;
   SiteTable table() const { return SiteTable{dSite, n_pad, dOrig}; }
   TaperTable taper_table() const { return TaperTable{dSite, n_pad}; }  // shares the per-site buffer
 };
@@ -462,7 +468,8 @@ void cocons_ctx_destroy(cocons_ctx* c) {
   cudaFree(c->dOrig), cudaFree(c->dA), cudaFree(c->dRhs);
   cudaFree(c->dTapCol), cudaFree(c->dTapRow), cudaFree(c->dInv), cudaFree(c->dTap), cudaFree(c->dCheck);
   cudaFree(c->dPool), cudaFree(c->dTiles), cudaFree(c->dMaps), cudaFree(c->dNegI), cudaFree(c->dLogPart);
-  cudaFree(c->dRowMap);
+  cudaFree(c->dRowMap), cudaFree(c->dRange), cudaFree(c->dLogdetB);
+  if (c->hDown) cudaFreeHost(c->hDown);
   solve_workspace_destroy(&c->ws);
   chol_workspace_destroy(&c->ws);
   cudaFree(c->dGram);
@@ -484,13 +491,16 @@ void cocons_ctx_destroy(cocons_ctx* c) {
     }                                                                                 \
   } while (0)
 
-// tiled: no n_pad^2 matrix and no dense solve workspace (the tiled context allocates its tile pool itself)
+// tiled: no n_pad^2 matrix and no dense solve workspace (the tiled context allocates its tile pool itself);
+// batch > 0: a batch context with that many matrices
 static int ctx_create(int device, int64_t n, int64_t p, int64_t r, const double* locs, const double* X,
-                      const double* z, void* stream, bool tiled, cocons_ctx** out) {
+                      const double* z, void* stream, bool tiled, cocons_ctx** out, int64_t batch = 0) {
   int rc = check_device(device);
   if (rc) return rc;
   cocons_ctx* c = new cocons_ctx();
   c->tiled = tiled;
+  c->batch = batch;
+  const int64_t nb = std::max<int64_t>(batch, 1);
   c->device = device;
   c->n = n, c->p = p, c->r = r;
   c->n_pad = round_up(n, kTile);
@@ -507,19 +517,24 @@ static int ctx_create(int device, int64_t n, int64_t p, int64_t r, const double*
   CTX_TRY(cudaMalloc(&c->dX, sizeof(double) * np * p));
   CTX_TRY(cudaMalloc(&c->dLocs, sizeof(double) * np * 2));
   CTX_TRY(cudaMalloc(&c->dZ, sizeof(double) * np * (r > 0 ? r : 1)));
-  CTX_TRY(cudaMalloc(&c->dTheta, sizeof(double) * 7 * p));
-  CTX_TRY(cudaMalloc(&c->dSite, sizeof(double) * SF_COUNT * np));
+  CTX_TRY(cudaMalloc(&c->dTheta, sizeof(double) * 7 * p * nb));
+  CTX_TRY(cudaMalloc(&c->dSite, sizeof(double) * SF_COUNT * np * nb));
   CTX_TRY(cudaMalloc(&c->dOrig, sizeof(int) * np));
-  if (!tiled) CTX_TRY(cudaMalloc(&c->dA, sizeof(double) * np * np));
-  if (chol_workspace_create(np, &c->ws, !tiled) != 0 || (!tiled && solve_workspace_create(np, &c->ws) != 0)) {
+  if (!tiled) CTX_TRY(cudaMalloc(&c->dA, sizeof(double) * np * np * nb));
+  if (batch > 0) {
+    CTX_TRY(cudaMalloc(&c->dRange, sizeof(double) * batch));
+    CTX_TRY(cudaMalloc(&c->dLogdetB, sizeof(double) * batch));
+  }
+  if (chol_workspace_create(np, &c->ws, !tiled && batch == 0, nb) != 0 ||
+      (!tiled && solve_workspace_create(np, &c->ws) != 0)) {
     set_error("ctx_create: out of device memory for the factorisation workspace");
     cocons_ctx_destroy(c);
     return COCONS_ERR_ALLOC;
   }
   CTX_TRY(cudaMalloc(&c->dRhs, sizeof(double) * np * 2 * kMaxRhs));
   CTX_TRY(cudaMalloc(&c->dGram, sizeof(double) * (kMaxRhs * kMaxRhs * 300 + 16)));
-  CTX_TRY(cudaMallocHost(&c->hStage, sizeof(double) * (7 * p + kMaxRhs * kMaxRhs + 16)));
-  CTX_TRY(cudaMallocHost(&c->hInfo, sizeof(int)));
+  CTX_TRY(cudaMallocHost(&c->hStage, sizeof(double) * (8 * p * nb + kMaxRhs * kMaxRhs + 16)));
+  CTX_TRY(cudaMallocHost(&c->hInfo, sizeof(int) * nb));
   for (auto& e : c->ev) CTX_TRY(cudaEventCreate(&e));
   {
     std::vector<int> orig((size_t)np);
@@ -543,6 +558,15 @@ int cocons_ctx_create(int device, int64_t n, int64_t p, int64_t r, const double*
   }
   *out = nullptr;
   return ctx_create(device, n, p, r, locs, X, z, stream, false, out);
+}
+
+// a batch context serves cocons_n2ll_batch, cocons_ctx_set_z, cocons_ctx_set_xbetas, cocons_ctx_dims,
+// cocons_ctx_timings and cocons_ctx_destroy only
+static int refuse_batch(cocons_ctx* c, const char* who) {
+  if (!c || !c->batch) return 0;
+  set_error("%s: not available on a batch context (cocons_ctx_create_batch); it supports cocons_n2ll_batch, "
+            "cocons_ctx_set_z, cocons_ctx_set_xbetas, cocons_ctx_dims and cocons_ctx_timings", who);
+  return COCONS_ERR_STATE;
 }
 
 // the entries that need the dense matrix refuse a tiled context
@@ -823,6 +847,38 @@ static int solve_status(cocons_ctx* c, const char* who) {
   return rc;
 }
 
+// quad[0, nc) of one block of right-hand sides from its Gram matrix hG (k x k, k = qx + nc: the qx solved mean-design
+// columns first); with qx > 0 also *lw = log det chol(W)
+static int compose_chunk(const double* hG, int k, int qx, int nc, double* quad, double* lw) {
+  if (qx == 0) {
+    for (int j = 0; j < nc; ++j) quad[j] = hG[j * k + j];
+    return 0;
+  }
+  // z'Pz = |y|^2 - b' W^-1 b with W = Yx'Yx, b = Yx'y  (SURVEY.md §8c: identical to the
+  // explicit projector route of :149-150 to 1e-14)
+  std::vector<double> W((size_t)qx * qx);
+  for (int a = 0; a < qx; ++a)
+    for (int b = 0; b < qx; ++b) W[(size_t)a * qx + b] = hG[a * k + b];
+  if (!small_chol(W, qx)) {
+    set_error("n2ll: X' Sigma^-1 X is not positive definite (rank-deficient mean design)");
+    return COCONS_ERR_STATE;
+  }
+  *lw = 0.0;
+  for (int a = 0; a < qx; ++a) *lw += std::log(W[(size_t)a * qx + a]);
+  for (int j = 0; j < nc; ++j) {
+    std::vector<double> t(qx);
+    double bb = 0.0;
+    for (int a = 0; a < qx; ++a) {  // forward solve chol(W) t = b
+      double s = hG[a * k + (qx + j)];
+      for (int b = 0; b < a; ++b) s -= W[(size_t)a * qx + b] * t[b];
+      t[a] = s / W[(size_t)a * qx + a];
+      bb += t[a] * t[a];
+    }
+    quad[j] = hG[(qx + j) * k + (qx + j)] - bb;
+  }
+  return 0;
+}
+
 static int n2ll_impl(cocons_ctx* c, int kind, const double* theta6, const double* limits, const double* mean_p,
                      double* logdet, double* quad, double* logdet_w, int* rank_x, bool taper) {
   if (!c || !theta6 || !limits || !logdet || !quad || kind < COCONS_ML || kind > COCONS_REML || c->r <= 0) {
@@ -875,32 +931,7 @@ static int n2ll_impl(cocons_ctx* c, int kind, const double* theta6, const double
       return *c->hInfo;  // > 0: not positive definite
     }
     *logdet = hG[kMaxRhs * kMaxRhs];
-    if (qx == 0) {
-      for (int j = 0; j < nc; ++j) quad[c0 + j] = hG[j * k + j];
-    } else {
-      // z'Pz = |y|^2 - b' W^-1 b with W = Yx'Yx, b = Yx'y  (SURVEY.md §8c: identical to the
-      // explicit projector route of :149-150 to 1e-14)
-      std::vector<double> W((size_t)qx * qx);
-      for (int a = 0; a < qx; ++a)
-        for (int b = 0; b < qx; ++b) W[(size_t)a * qx + b] = hG[a * k + b];
-      if (!small_chol(W, qx)) {
-        set_error("n2ll: X' Sigma^-1 X is not positive definite (rank-deficient mean design)");
-        return COCONS_ERR_STATE;
-      }
-      lw = 0.0;
-      for (int a = 0; a < qx; ++a) lw += std::log(W[(size_t)a * qx + a]);
-      for (int j = 0; j < nc; ++j) {
-        std::vector<double> t(qx);
-        double bb = 0.0;
-        for (int a = 0; a < qx; ++a) {  // forward solve chol(W) t = b
-          double s = hG[a * k + (qx + j)];
-          for (int b = 0; b < a; ++b) s -= W[(size_t)a * qx + b] * t[b];
-          t[a] = s / W[(size_t)a * qx + a];
-          bb += t[a] * t[a];
-        }
-        quad[c0 + j] = hG[(qx + j) * k + (qx + j)] - bb;
-      }
-    }
+    if ((rc = compose_chunk(hG, k, qx, nc, quad + c0, &lw))) return rc;
   }
   if (logdet_w) *logdet_w = lw;
   if (rank_x) {
@@ -917,7 +948,170 @@ static int n2ll_impl(cocons_ctx* c, int kind, const double* theta6, const double
 int cocons_n2ll(cocons_ctx* c, int kind, const double* theta6, const double* limits, const double* mean_p,
                 double* logdet, double* quad, double* logdet_w, int* rank_x) {
   if (int rc_ = refuse_tiled(c, "n2ll")) return rc_;
+  if (int rc_ = refuse_batch(c, "n2ll")) return rc_;
   return n2ll_impl(c, kind, theta6, limits, mean_p, logdet, quad, logdet_w, rank_x, false);
+}
+
+// ---- batch context -------------------------------------------------------------------------------------------------
+
+int cocons_ctx_create_batch(int device, int64_t n, int64_t p, int64_t r, const double* locs, const double* X,
+                            const double* z, int64_t batch, void* stream, cocons_ctx** out) {
+  if (!out || n <= 0 || p <= 0 || r < 0 || !locs || !X || (r > 0 && !z) || batch < 1 || batch > 65535) {
+    set_error("ctx_create_batch: bad argument (batch must be in 1..65535)");
+    return COCONS_ERR_ARG;
+  }
+  *out = nullptr;
+  if (round_up(n, kTile) >= kSyrkI8MinPad) {
+    set_error("ctx_create_batch: n_pad = %lld; a batch context takes n_pad < %lld (above it one evaluation fills the "
+              "device: use cocons_ctx_create)", (long long)round_up(n, kTile), (long long)kSyrkI8MinPad);
+    return COCONS_ERR_ARG;
+  }
+  const int rc = ctx_create(device, n, p, r, locs, X, z, stream, false, out, batch);
+  if (rc) cudaGetLastError();  // a failed allocation leaves nothing behind, not even the error state
+  return rc;
+}
+
+// The points [g0, g0 + cnt) of one group, cnt <= batch.  Slots are ordered by smoothness mode, so that the site stage
+// and the assembly take one launch per mode present; the factorisation is one chol_factor over all slots; the
+// log-determinant, the solves and the Gram reductions run per slot with the single context's kernels.  Every matrix
+// sees the arithmetic of cocons_n2ll, in the same order.  ms4: phase times added up.
+static int n2ll_group(cocons_ctx* c, int kind, int64_t g0, int cnt, const double* theta6, const double* lim,
+                      const double* mean_p, double* logdet, double* quad, double* logdet_w, int* status, double* ms4) {
+  const int64_t n = c->n, np = c->n_pad, p = c->p, B = c->batch;
+  cudaStream_t st = c->stream;
+  std::vector<int> mode((size_t)cnt), slot_pt((size_t)cnt);
+  std::vector<double> nu((size_t)cnt);
+  for (int i = 0; i < cnt; ++i) {
+    mode[(size_t)i] = smooth_mode_for(COCONS_PAR_DIFF, (int)p, theta6 + (g0 + i) * 6 * p, lim, &nu[(size_t)i]);
+    slot_pt[(size_t)i] = i;
+  }
+  std::stable_sort(slot_pt.begin(), slot_pt.end(), [&](int a, int b) { return mode[(size_t)a] < mode[(size_t)b]; });
+  double* up = c->hStage;  // theta + mean per slot, then the global ranges
+  for (int s = 0; s < cnt; ++s) {
+    const int64_t pt = g0 + slot_pt[(size_t)s];
+    std::memcpy(up + s * 7 * p, theta6 + pt * 6 * p, sizeof(double) * 6 * p);
+    if (kind == COCONS_ML && mean_p)
+      std::memcpy(up + s * 7 * p + 6 * p, mean_p + pt * p, sizeof(double) * p);
+    else
+      std::memset(up + s * 7 * p + 6 * p, 0, sizeof(double) * p);
+    up[7 * p * B + s] = 1 / std::exp(-2 * theta6[pt * 6 * p + p]);
+  }
+  COCONS_CUDA_TRY(cudaMemcpyAsync(c->dTheta, up, sizeof(double) * 7 * p * cnt, cudaMemcpyHostToDevice, st));
+  COCONS_CUDA_TRY(cudaMemcpyAsync(c->dRange, up + 7 * p * B, sizeof(double) * cnt, cudaMemcpyHostToDevice, st));
+  COCONS_CUDA_TRY(cudaEventRecord(c->ev[0], st));
+  for (int s0 = 0, s1; s0 < cnt; s0 = s1) {
+    const int m = mode[(size_t)slot_pt[(size_t)s0]];
+    for (s1 = s0 + 1; s1 < cnt && mode[(size_t)slot_pt[(size_t)s1]] == m;) ++s1;
+    const SiteTable T{c->dSite + s0 * SF_COUNT * np, np, c->dOrig};
+    launch_site_stage(n, np, (int)p, c->dX, np, c->dLocs, np, c->dTheta + s0 * 7 * p, lim[0], lim[1], m, T, st,
+                      s1 - s0);
+    launch_assemble_lower_batch(n, np, T, c->dRange + s0, nu[(size_t)slot_pt[(size_t)s0]], m, c->dA + s0 * np * np,
+                                s1 - s0, st);
+  }
+  COCONS_CUDA_TRY(cudaEventRecord(c->ev[1], st));
+  chol_factor(c->dA, np, np, c->ws, st, cnt);
+  COCONS_CUDA_TRY(cudaEventRecord(c->ev[2], st));
+  const int qx = (kind == COCONS_PROFILE) ? (int)c->q : (kind == COCONS_REML ? (int)p : 0);
+  const int chunk = kMaxRhs - qx;
+  const int64_t nchunks = (c->r + chunk - 1) / chunk, per_slot = nchunks * kMaxRhs * kMaxRhs;
+  if (c->down_cap < B * per_slot + B) {
+    if (c->hDown) cudaFreeHost(c->hDown), c->hDown = nullptr, c->down_cap = 0;
+    COCONS_CUDA_TRY(cudaMallocHost(&c->hDown, sizeof(double) * (B * per_slot + B)));
+    c->down_cap = B * per_slot + B;
+  }
+  for (int s = 0; s < cnt; ++s) {
+    const double* A = c->dA + s * np * np;
+    CholWorkspace w = c->ws;
+    w.winv += s * np * kTile;
+    w.info += s;
+    launch_logdet(A, n, np, c->dLogdetB + s, st);
+    if (qx > 0) {
+      const double* src = (kind == COCONS_PROFILE) ? c->dXb : c->dX;
+      COCONS_CUDA_TRY(cudaMemcpyAsync(c->dRhs, src, sizeof(double) * np * qx, cudaMemcpyDeviceToDevice, st));
+      forward_solve_ws(A, np, np, w, c->dRhs, np, qx, st);
+    }
+    for (int64_t c0 = 0, ci = 0; c0 < c->r; c0 += chunk, ++ci) {
+      const int nc = (int)((c->r - c0 < chunk) ? c->r - c0 : chunk);
+      double* rhs = c->dRhs + (int64_t)qx * np;
+      launch_residual(n, np, (int)p, nc, c->dX, c->dZ + c0 * np,
+                      kind == COCONS_ML ? c->dTheta + s * 7 * p + 6 * p : nullptr, rhs, st);
+      forward_solve_ws(A, np, np, w, rhs, np, nc, st);
+      const int k = qx + nc;
+      launch_gram(c->dRhs, n, np, k, c->dGram, st);
+      COCONS_CUDA_TRY(cudaMemcpyAsync(c->hDown + s * per_slot + ci * kMaxRhs * kMaxRhs, c->dGram,
+                                      sizeof(double) * k * k, cudaMemcpyDeviceToHost, st));
+    }
+  }
+  COCONS_CUDA_TRY(cudaEventRecord(c->ev[3], st));
+  COCONS_CUDA_TRY(cudaMemcpyAsync(c->hDown + B * per_slot, c->dLogdetB, sizeof(double) * cnt, cudaMemcpyDeviceToHost,
+                                  st));
+  COCONS_CUDA_TRY(cudaMemcpyAsync(c->hInfo, c->ws.info, sizeof(int) * cnt, cudaMemcpyDeviceToHost, st));
+  COCONS_CUDA_TRY(cudaStreamSynchronize(st));
+  COCONS_CUDA_TRY(cudaGetLastError());
+  for (int e = 0; e < 3; ++e) {
+    float t = 0;
+    COCONS_CUDA_TRY(cudaEventElapsedTime(&t, c->ev[e], c->ev[e + 1]));
+    ms4[e] += t, ms4[3] += t;
+  }
+  for (int s = 0; s < cnt; ++s) {
+    const int64_t pt = g0 + slot_pt[(size_t)s];
+    const int info = c->hInfo[s];
+    if (info != 0) {  // > 0: not positive definite
+      if (info < 0) set_error("n2ll_batch: point %lld: %s", (long long)pt, kSolveGaveUp);
+      status[pt] = info;
+      continue;
+    }
+    double lw = 0.0;
+    int rc = 0;
+    for (int64_t c0 = 0, ci = 0; c0 < c->r && rc == 0; c0 += chunk, ++ci) {
+      const int nc = (int)((c->r - c0 < chunk) ? c->r - c0 : chunk);
+      rc = compose_chunk(c->hDown + s * per_slot + ci * kMaxRhs * kMaxRhs, qx + nc, qx, nc, quad + pt * c->r + c0,
+                         &lw);
+    }
+    status[pt] = rc;
+    if (rc) continue;
+    logdet[pt] = c->hDown[B * per_slot + s];
+    if (logdet_w) logdet_w[pt] = lw;
+  }
+  return 0;
+}
+
+int cocons_n2ll_batch(cocons_ctx* c, int kind, int64_t npoints, const double* theta6, const double* limits,
+                      const double* mean_p, double* logdet, double* quad, double* logdet_w, int* rank_x,
+                      int* status) {
+  if (c && !c->batch) {
+    set_error("n2ll_batch: not a batch context (cocons_ctx_create_batch)");
+    return COCONS_ERR_STATE;
+  }
+  if (!c || npoints < 1 || !theta6 || !limits || !logdet || !quad || !status || kind < COCONS_ML ||
+      kind > COCONS_REML || c->r <= 0) {
+    set_error("n2ll_batch: bad argument");
+    return COCONS_ERR_ARG;
+  }
+  if (kind == COCONS_PROFILE && (!c->dXb || c->q <= 0)) {
+    set_error("n2ll_batch: COCONS_PROFILE needs cocons_ctx_set_xbetas first");
+    return COCONS_ERR_STATE;
+  }
+  if (kind == COCONS_REML && c->p >= kMaxRhs) {
+    set_error("n2ll_batch: REML supports at most %d design columns", kMaxRhs - 1);
+    return COCONS_ERR_ARG;
+  }
+  cudaSetDevice(c->device);
+  const double lim[2] = {limits[0], limits[1]};
+  double ms4[4] = {0, 0, 0, 0};
+  for (int64_t g0 = 0; g0 < npoints; g0 += c->batch) {
+    const int cnt = (int)std::min<int64_t>(c->batch, npoints - g0);
+    if (int rc = n2ll_group(c, kind, g0, cnt, theta6, lim, mean_p, logdet, quad, logdet_w, status, ms4)) return rc;
+  }
+  if (rank_x) {
+    *rank_x = 0;
+    if (kind == COCONS_REML) {
+      if (c->rank_x < 0) c->rank_x = qr_rank_dqrdc2(c->hX.data(), c->n, (int)c->p);
+      *rank_x = c->rank_x;
+    }
+  }
+  for (int i = 0; i < 4; ++i) c->ms[i] = ms4[i];
+  return 0;
 }
 
 // ---- sparse (tapered) model -------------------------------------------------
@@ -966,6 +1160,7 @@ static int attach_taper(cocons_ctx* c, const int32_t* colindices, const int32_t*
 
 int cocons_ctx_set_taper(cocons_ctx* c, const int32_t* colindices, const int32_t* rowpointers,
                          const double* taper_entries, int64_t nnz) {
+  if (int rc_ = refuse_batch(c, "ctx_set_taper")) return rc_;
   if (!c || !taper_entries) {
     set_error("ctx_set_taper: bad argument");
     return COCONS_ERR_ARG;
@@ -1065,6 +1260,7 @@ static int n2ll_tiled(cocons_ctx* c, const double* theta6, const double* limits,
 
 int cocons_n2ll_taper(cocons_ctx* c, const double* theta6, const double* limits, const double* mean_p,
                       double* logdet, double* quad) {
+  if (int rc_ = refuse_batch(c, "n2ll_taper")) return rc_;
   if (!c || !c->dTap) {
     set_error("n2ll_taper: cocons_ctx_set_taper first");
     return COCONS_ERR_STATE;
@@ -1153,6 +1349,7 @@ int cocons_cov_rns_taper_pred(int64_t n, int64_t m, int64_t p, const double* loc
 
 int cocons_profile_betas(cocons_ctx* c, int kind, double* betas) {
   if (int rc_ = refuse_tiled(c, "profile_betas")) return rc_;
+  if (int rc_ = refuse_batch(c, "profile_betas")) return rc_;
   if (!c || !betas || (kind != COCONS_PROFILE && kind != COCONS_REML)) {
     set_error("profile_betas: bad argument");
     return COCONS_ERR_ARG;
@@ -1211,6 +1408,7 @@ int cocons_profile_betas(cocons_ctx* c, int kind, double* betas) {
 
 int cocons_factor(cocons_ctx* c, int par, const double* theta6, const double* limits) {
   if (int rc_ = refuse_tiled(c, "factor")) return rc_;
+  if (int rc_ = refuse_batch(c, "factor")) return rc_;
   if (!c || !theta6 || (par != COCONS_PAR_DIFF && par != COCONS_PAR_CLASSIC) || (par == COCONS_PAR_DIFF && !limits)) {
     set_error("factor: bad argument");
     return COCONS_ERR_ARG;
@@ -1397,10 +1595,12 @@ static int predict_impl(cocons_ctx* c, int64_t m, const double* locs_pred, const
 int cocons_predict(cocons_ctx* c, int64_t m, const double* locs_pred, const double* Xp, const double* resid,
                    double* stochastic, double* explained) {
   if (int rc_ = refuse_tiled(c, "predict")) return rc_;
+  if (int rc_ = refuse_batch(c, "predict")) return rc_;
   return predict_impl(c, m, locs_pred, Xp, resid, stochastic, explained, nullptr);
 }
 
 int cocons_factor_taper(cocons_ctx* c, const double* theta6, const double* limits) {
+  if (int rc_ = refuse_batch(c, "factor_taper")) return rc_;
   if (!c || !theta6 || !limits) {
     set_error("factor_taper: bad argument");
     return COCONS_ERR_ARG;
@@ -1424,6 +1624,7 @@ int cocons_factor_taper(cocons_ctx* c, const double* theta6, const double* limit
 int cocons_predict_taper(cocons_ctx* c, int64_t m, const double* locs_pred, const double* Xp,
                          const int32_t* colindices, const int32_t* rowpointers, const double* taper_entries,
                          int64_t nnz, const double* resid, double* stochastic, double* explained) {
+  if (int rc_ = refuse_batch(c, "predict_taper")) return rc_;
   if (!c || m <= 0 || !taper_entries) {
     set_error("predict_taper: bad argument");
     return COCONS_ERR_ARG;
@@ -1477,6 +1678,7 @@ static int sim_tiled(cocons_ctx* c, int64_t k, const double* eps, double* out);
 
 int cocons_sim(cocons_ctx* c, int64_t k, const double* eps, double* out) {
   if (int rc_ = refuse_tiled(c, "sim")) return rc_;
+  if (int rc_ = refuse_batch(c, "sim")) return rc_;
   if (!c || k <= 0 || !eps || !out) {
     set_error("sim: bad argument");
     return COCONS_ERR_ARG;
@@ -1490,6 +1692,7 @@ int cocons_sim(cocons_ctx* c, int64_t k, const double* eps, double* out) {
 }
 
 int cocons_sim_taper(cocons_ctx* c, int64_t k, const double* eps, double* out) {
+  if (int rc_ = refuse_batch(c, "sim_taper")) return rc_;
   if (!c || k <= 0 || !eps || !out) {
     set_error("sim_taper: bad argument");
     return COCONS_ERR_ARG;
@@ -1637,6 +1840,7 @@ static int predict_tiled(cocons_ctx* c, int64_t m, const double* locs_pred, cons
 int cocons_sim_cond(cocons_ctx* c, int64_t m, const double* locs_pred, const double* Xp, int64_t k, const double* eps,
                     double* out) {
   if (int rc_ = refuse_tiled(c, "sim_cond")) return rc_;
+  if (int rc_ = refuse_batch(c, "sim_cond")) return rc_;
   if (!c || m <= 0 || k <= 0 || !locs_pred || !Xp || !eps || !out) {
     set_error("sim_cond: bad argument");
     return COCONS_ERR_ARG;
@@ -1709,6 +1913,7 @@ int cocons_sim_cond(cocons_ctx* c, int64_t m, const double* locs_pred, const dou
 }
 
 int cocons_ctx_get_factor(cocons_ctx* c, double* L, int64_t* perm) {
+  if (int rc_ = refuse_batch(c, "get_factor")) return rc_;
   if (!c || !L) {
     set_error("get_factor: bad argument");
     return COCONS_ERR_ARG;
@@ -1746,6 +1951,7 @@ int cocons_ctx_get_factor(cocons_ctx* c, double* L, int64_t* perm) {
 }
 
 int cocons_ctx_factor_rows(cocons_ctx* c, const int64_t* sites, int64_t m, double* rows, int64_t* pos) {
+  if (int rc_ = refuse_batch(c, "factor_rows")) return rc_;
   if (!c || !sites || !rows || !pos || m <= 0) {
     set_error("factor_rows: bad argument");
     return COCONS_ERR_ARG;
@@ -1810,6 +2016,7 @@ int cocons_ctx_timings(cocons_ctx* c, double* ms4) {
 
 int cocons_ctx_debug_checksums(cocons_ctx* c, double* out2) {
   if (int rc_ = refuse_tiled(c, "ctx_debug_checksums")) return rc_;
+  if (int rc_ = refuse_batch(c, "ctx_debug_checksums")) return rc_;
   if (!c || !out2) return COCONS_ERR_ARG;
   out2[0] = c->check[0], out2[1] = c->check[1];
   return 0;
@@ -1817,6 +2024,7 @@ int cocons_ctx_debug_checksums(cocons_ctx* c, double* out2) {
 
 int cocons_ctx_kernel_timing(cocons_ctx* c, double* ms, double* flops) {
   if (int rc_ = refuse_tiled(c, "ctx_kernel_timing")) return rc_;
+  if (int rc_ = refuse_batch(c, "ctx_kernel_timing")) return rc_;
   if (!c || !ms || !flops) return COCONS_ERR_ARG;
   *ms = c->kernel_ms, *flops = c->kernel_flops;
   return 0;

@@ -37,6 +37,9 @@ namespace cocons {
 constexpr int GBM = 128, GBK = 16, GSTAGES = 4;
 constexpr int GLDA = GBM + 4;  // padded leading dimension of a shared k-row (== 4 mod 16: conflict-free LDS.128)
 constexpr int kGemmMapped = 2;  // gemm_nt_tma_kernel's tile-mapped C -= A B^T (tiled factor, csrc/capi.cu)
+// gemm_nt_tma_kernel over a batch of matrices (chol_factor with batch > 0): blockIdx.y selects the matrix; C -= A B^T
+// (128 x 64 tiles) and C = A B^T (128 x 128 tiles)
+constexpr int kGemmBatchSub = 8, kGemmBatchSet = 9;
 
 template <int BN, int NU = 2>
 struct GemmCfg {
@@ -368,6 +371,9 @@ __device__ void tiled_product(const TiledArgs& a) {
 // carries the device address of the map, int64: [pairs: element offset of the target block from C][128-column
 // blocks: leading dimension of the target], pair (bi, c) numbered bi (bi + 1) / 2 + c with lower_only, bi * nj / 2 + c
 // without (c = the 128-column block of the CTA's tile).
+// kGemmBatchSub / kGemmBatchSet: as 0 / 1 on matrix blockIdx.y of a batch whose matrices are square with ld = lda and
+// lie back to back, each with its inverted diagonal tiles (lda x 128) back to back: A and C move by lda^2 per matrix,
+// B by lda ldb (the matrix itself, or its inverted tiles when ldb = 128).
 template <int BN, int NU, int ASSIGN>
 __global__ void __launch_bounds__(GemmCfg<BN, NU>::kThreads, GemmCfg<BN, NU>::kMinBlocks)
     gemm_nt_tma_kernel(int ni, int nj, int64_t K, const double* A, int64_t lda, const double* B, int64_t ldb,
@@ -376,7 +382,8 @@ __global__ void __launch_bounds__(GemmCfg<BN, NU>::kThreads, GemmCfg<BN, NU>::kM
   constexpr int kWarps = Cfg::kThreads / 32;
   constexpr uint32_t kStageBytes = GBK * (GBM + BN) * (uint32_t)sizeof(double);
   extern __shared__ __align__(16) double smem[];
-  if constexpr (ASSIGN >= kTiledFwd8) {  // the tiled context's solves and product (see above), ldc = &TiledArgs
+  constexpr bool kAssign = (ASSIGN == 1 || ASSIGN == kGemmBatchSet);
+  if constexpr (ASSIGN >= kTiledFwd8 && ASSIGN <= kTiledTrmm32) {  // the tiled context's solves and product (see above), ldc = &TiledArgs
     const TiledArgs& ta = *reinterpret_cast<const TiledArgs*>(ldc);
     if constexpr (ASSIGN == kTiledFwd8) tiled_forward<1>(ta, smem);
     if constexpr (ASSIGN == kTiledFwd32) tiled_forward<4>(ta, smem);
@@ -384,6 +391,11 @@ __global__ void __launch_bounds__(GemmCfg<BN, NU>::kThreads, GemmCfg<BN, NU>::kM
     if constexpr (ASSIGN == kTiledTrmm8) tiled_product<1>(ta);
     if constexpr (ASSIGN == kTiledTrmm32) tiled_product<4>(ta);
     return;
+  }
+  if constexpr (ASSIGN == kGemmBatchSub || ASSIGN == kGemmBatchSet) {
+    A += (int64_t)blockIdx.y * lda * lda;
+    B += (int64_t)blockIdx.y * lda * ldb;
+    C += (int64_t)blockIdx.y * lda * lda;
   }
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (size_t)GSTAGES * Cfg::kStageDoubles);
   const int tid = threadIdx.x;
@@ -442,7 +454,7 @@ __global__ void __launch_bounds__(GemmCfg<BN, NU>::kThreads, GemmCfg<BN, NU>::kM
     C += map[pair] + (int64_t)(bj & 1) * BN * ldc - (int64_t)bj * BN * ldc - (int64_t)bi * GBM;
   }
 #ifndef COCONS_GEMM_NO_PREFETCH
-  if (ASSIGN != 1) {  // pull the C tile towards L2 while the main loop runs
+  if (!kAssign) {  // pull the C tile towards L2 while the main loop runs
     const double* Cp = C + (int64_t)bj * BN * ldc + (int64_t)bi * GBM;
     for (int l = tid; l < BN * 8; l += Cfg::kThreads)
       asm volatile("prefetch.global.L2 [%0];" ::"l"(Cp + (int64_t)(l >> 3) * ldc + (l & 7) * 16));
@@ -511,7 +523,7 @@ __global__ void __launch_bounds__(GemmCfg<BN, NU>::kThreads, GemmCfg<BN, NU>::kM
       const int r0 = iw + 16 * u + 4 * c4;
       double2* p = reinterpret_cast<double2*>(Cg + (int64_t)j * ldc + r0);
       double2 lo, hi;
-      if (ASSIGN == 1) {
+      if (kAssign) {
         lo.x = acc[a][2 * u][0];
         lo.y = acc[a][2 * u + 1][0];
         hi.x = acc[a][2 * u][1];
@@ -526,7 +538,7 @@ __global__ void __launch_bounds__(GemmCfg<BN, NU>::kThreads, GemmCfg<BN, NU>::kM
         hi.x -= acc[a][2 * u][1];
         hi.y -= acc[a][2 * u + 1][1];
       }
-      if (ASSIGN == 1) {
+      if (kAssign) {
         p[0] = lo;
         p[1] = hi;
       } else {
@@ -547,18 +559,29 @@ static int debug_sync_mode() {
   return m;
 }
 
-// 128 x 64 tiles: C -= A B^T (EPI = 0) or the tile-mapped variant (EPI = kGemmMapped)
+// 128 x 64 tiles: C -= A B^T (EPI = 0), the tile-mapped variant (EPI = kGemmMapped) or the batched one (kGemmBatchSub,
+// nb matrices)
 template <int EPI>
 static void launch_gemm_64(int ni, int nj, int64_t K, const double* A, int64_t lda, const double* B, int64_t ldb,
-                           double* C, int64_t ldc, int lower_only, cudaStream_t st) {
+                           double* C, int64_t ldc, int lower_only, cudaStream_t st, unsigned nb = 1) {
   const int64_t tiles = total_tiles<2>(ni, nj, lower_only);
-  gemm_nt_tma_kernel<64, 2, EPI><<<(unsigned)tiles, GemmCfg<64, 2>::kThreads, GemmCfg<64, 2>::kSmemBytes + 64, st>>>(
-      ni, nj, K, A, lda, B, ldb, C, ldc, lower_only);
+  gemm_nt_tma_kernel<64, 2, EPI><<<dim3((unsigned)tiles, nb), GemmCfg<64, 2>::kThreads, GemmCfg<64, 2>::kSmemBytes + 64,
+                                   st>>>(ni, nj, K, A, lda, B, ldb, C, ldc, lower_only);
+}
+
+// 128 x 128 tiles: C = A B^T (EPI = 1) or its batched form (kGemmBatchSet, nb matrices)
+template <int EPI>
+static void launch_gemm_128(int ni, int nj, int64_t K, const double* A, int64_t lda, const double* B, int64_t ldb,
+                            double* C, int64_t ldc, int lower_only, cudaStream_t st, unsigned nb) {
+  const int64_t tiles = total_tiles<1>(ni, nj, lower_only);
+  gemm_nt_tma_kernel<128, 2, EPI><<<dim3((unsigned)tiles, nb), GemmCfg<128, 2>::kThreads,
+                                    GemmCfg<128, 2>::kSmemBytes + 64, st>>>(ni, nj, K, A, lda, B, ldb, C, ldc, lower_only);
 }
 
 // mode 2: as mode 0 with C addressed through a tile map whose device address is passed as ldc (see the kernel)
+// batch > 0 (modes 0 and 1): the same product on each of `batch` matrices laid out as the batched kernels expect
 void launch_gemm_nt(int mode, int64_t M, int64_t N, int64_t K, const double* A, int64_t lda, const double* B,
-                    int64_t ldb, double* C, int64_t ldc, int lower_only, cudaStream_t st) {
+                    int64_t ldb, double* C, int64_t ldc, int lower_only, cudaStream_t st, int batch) {
   if (M <= 0 || N <= 0 || K <= 0) return;
   static bool attr_done[16] = {};
   int dev = 0;
@@ -571,17 +594,23 @@ void launch_gemm_nt(int mode, int64_t M, int64_t N, int64_t K, const double* A, 
                          GemmCfg<128, 2>::kSmemBytes + 64);
     cudaFuncSetAttribute(gemm_nt_tma_kernel<64, 2, kGemmMapped>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                          GemmCfg<64, 2>::kSmemBytes + 64);
+    cudaFuncSetAttribute(gemm_nt_tma_kernel<64, 2, kGemmBatchSub>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                         GemmCfg<64, 2>::kSmemBytes + 64);
+    cudaFuncSetAttribute(gemm_nt_tma_kernel<128, 2, kGemmBatchSet>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                         GemmCfg<128, 2>::kSmemBytes + 64);
     attr_done[dev] = true;
   }
   const int ni = (int)(M / GBM);
   note_launch();
   if (mode == 1) {
-    const int nj = (int)(N / 128);
-    const int64_t tiles = total_tiles<1>(ni, nj, lower_only);
-    gemm_nt_tma_kernel<128, 2, 1><<<(unsigned)tiles, GemmCfg<128, 2>::kThreads, GemmCfg<128, 2>::kSmemBytes + 64, st>>>(
-        ni, nj, K, A, lda, B, ldb, C, ldc, lower_only);
+    if (batch > 0)
+      launch_gemm_128<kGemmBatchSet>(ni, (int)(N / 128), K, A, lda, B, ldb, C, ldc, lower_only, st, (unsigned)batch);
+    else
+      launch_gemm_128<1>(ni, (int)(N / 128), K, A, lda, B, ldb, C, ldc, lower_only, st, 1u);
   } else if (mode == kGemmMapped) {
     launch_gemm_64<kGemmMapped>(ni, (int)(N / 64), K, A, lda, B, ldb, C, ldc, lower_only, st);
+  } else if (batch > 0) {
+    launch_gemm_64<kGemmBatchSub>(ni, (int)(N / 64), K, A, lda, B, ldb, C, ldc, lower_only, st, (unsigned)batch);
   } else {
     launch_gemm_64<0>(ni, (int)(N / 64), K, A, lda, B, ldb, C, ldc, lower_only, st);
   }
@@ -919,10 +948,18 @@ __device__ __forceinline__ void potrf_diag_block(double* Dl, double* Dt, double*
   }
 }
 
+// BATCH = 1: CTA b factors the tile of matrix b of a batch (square, leading dimension ld, back to back), with its own
+// inverted tiles (ld x 128 per matrix) and its own info word
+template <int BATCH>
 __global__ void __launch_bounds__(256, 1)
     potrf_tile_blocked_kernel(double* __restrict__ A, int64_t ld, double* __restrict__ Winv, int* __restrict__ info,
                               int first_index) {
   extern __shared__ __align__(16) double psm[];
+  if constexpr (BATCH) {
+    A += (int64_t)blockIdx.x * ld * ld;
+    Winv += (int64_t)blockIdx.x * ld * PT;
+    info += blockIdx.x;
+  }
   double* Lb = psm;                  // lower blocks of the tile -> L
   double* Tb = psm + PNBLK * PBLK;   // lower blocks of T -> W
   __shared__ int fail;
@@ -1011,9 +1048,16 @@ __global__ void __launch_bounds__(256, 1)
   PROBEB(30);
 }
 
+template <int BATCH>
+static void launch_potrf_blocked(unsigned nb, double* A, int64_t ld, double* Winv, int* info, int first_index,
+                                 cudaStream_t st) {
+  potrf_tile_blocked_kernel<BATCH><<<nb, 256, kPotrfBlockedSmem, st>>>(A, ld, Winv, info, first_index);
+}
+
 // the blocked kernel is the default (53.8 vs 81.0 us per cold tile in tools/micro/potrf_check.cu);
-// COCONS_POTRF=1 selects the register-resident column-sweep kernel
-void launch_potrf_tile(double* A, int64_t ld, double* Winv, int* info, int first_index, cudaStream_t st) {
+// COCONS_POTRF=1 selects the register-resident column-sweep kernel (single matrices only: a batch always runs the
+// blocked kernel)
+void launch_potrf_tile(double* A, int64_t ld, double* Winv, int* info, int first_index, cudaStream_t st, int batch) {
   static int variant = -1;
   static bool attr_done[16] = {};
   if (variant < 0) {
@@ -1021,22 +1065,26 @@ void launch_potrf_tile(double* A, int64_t ld, double* Winv, int* info, int first
     variant = e ? atoi(e) : 2;
   }
   note_launch();
-  if (variant == 1) {
+  if (variant == 1 && batch == 0) {
     potrf_tile_kernel<<<1, 256, 0, st>>>(A, ld, Winv, info, first_index);
     return;
   }
   int dev = 0;
   cudaGetDevice(&dev);
   if (dev < 16 && !attr_done[dev]) {
-    cudaFuncSetAttribute(potrf_tile_blocked_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPotrfBlockedSmem);
+    cudaFuncSetAttribute(potrf_tile_blocked_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPotrfBlockedSmem);
+    cudaFuncSetAttribute(potrf_tile_blocked_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPotrfBlockedSmem);
     attr_done[dev] = true;
   }
-  potrf_tile_blocked_kernel<<<1, 256, kPotrfBlockedSmem, st>>>(A, ld, Winv, info, first_index);
+  if (batch > 0)
+    launch_potrf_blocked<1>((unsigned)batch, A, ld, Winv, info, first_index, st);
+  else
+    launch_potrf_blocked<0>(1u, A, ld, Winv, info, first_index, st);
 }
 
 SyrkI8Ops g_syrk_i8 = {nullptr, nullptr};
 
-int chol_workspace_create(int64_t n_pad, CholWorkspace* ws, bool with_i8) {
+int chol_workspace_create(int64_t n_pad, CholWorkspace* ws, bool with_i8, int64_t batch) {
   ws->winv = nullptr, ws->info = nullptr, ws->panel_stream = nullptr, ws->ev_a = nullptr, ws->ev_p = nullptr;
   ws->ev_k0 = nullptr, ws->ev_k1 = nullptr;
   ws->i8_slices = nullptr, ws->i8_scale = nullptr;
@@ -1044,8 +1092,8 @@ int chol_workspace_create(int64_t n_pad, CholWorkspace* ws, bool with_i8) {
   cudaDeviceGetStreamPriorityRange(&lo, &hi);  // hi = greatest priority (numerically lowest)
   if (const char* e = getenv("COCONS_PANEL_PRIORITY"))  // 0: panel stream at default priority (bisection aid)
     if (atoi(e) == 0) hi = 0;
-  if (cudaMalloc(&ws->winv, sizeof(double) * (n_pad / kTile) * kTile * kTile) != cudaSuccess ||
-      cudaMalloc(&ws->info, sizeof(int)) != cudaSuccess ||
+  if (cudaMalloc(&ws->winv, sizeof(double) * batch * (n_pad / kTile) * kTile * kTile) != cudaSuccess ||
+      cudaMalloc(&ws->info, sizeof(int) * batch) != cudaSuccess ||
       cudaStreamCreateWithPriority(&ws->panel_stream, cudaStreamNonBlocking, hi) != cudaSuccess ||
       cudaEventCreateWithFlags(&ws->ev_a, cudaEventDisableTiming) != cudaSuccess ||
       cudaEventCreateWithFlags(&ws->ev_p, cudaEventDisableTiming) != cudaSuccess ||
@@ -1078,18 +1126,19 @@ void chol_workspace_destroy(CholWorkspace* ws) {
 
 // one outer panel: tiles [J0, J0+jb), every 128-wide step on stream `st`
 void factor_panel(double* A, int64_t n_pad, int64_t ld, const CholWorkspace& ws, int64_t J0, int64_t jb,
-                  cudaStream_t st) {
+                  cudaStream_t st, int batch) {
   for (int64_t jj = J0; jj < J0 + jb; ++jj) {
     double* Ajj = A + jj * kTile * ld + jj * kTile;
     double* Wjj = ws.winv + jj * (int64_t)kTile * kTile;
-    launch_potrf_tile(Ajj, ld, Wjj, ws.info, (int)(jj * kTile), st);
+    launch_potrf_tile(Ajj, ld, Wjj, ws.info, (int)(jj * kTile), st, batch);
     const int64_t below = n_pad - (jj + 1) * kTile;
     if (below <= 0) continue;
     double* panel = Ajj + kTile;  // rows below the diagonal tile, 128 columns
     // X = A * W^T  (in place: a CTA reads all of its 128 x 128 block before writing it)
-    launch_gemm_nt(1, below, kTile, kTile, panel, ld, Wjj, kTile, panel, ld, 0, st);
+    launch_gemm_nt(1, below, kTile, kTile, panel, ld, Wjj, kTile, panel, ld, 0, st, batch);
     const int64_t rest = (J0 + jb - jj - 1) * kTile;  // remaining columns of this outer panel
-    if (rest > 0) launch_gemm_nt(0, below, rest, kTile, panel, ld, panel, ld, Ajj + kTile * ld + kTile, ld, 1, st);
+    if (rest > 0)
+      launch_gemm_nt(0, below, rest, kTile, panel, ld, panel, ld, Ajj + kTile * ld + kTile, ld, 1, st, batch);
   }
 }
 
@@ -1122,9 +1171,9 @@ static bool syrk_i8_enabled(const CholWorkspace& ws) {
   return !(e && atoi(e) == 0);
 }
 
-int chol_factor(double* A, int64_t n_pad, int64_t ld, CholWorkspace ws, cudaStream_t st) {
-  cudaMemsetAsync(ws.info, 0, sizeof(int), st);
-  const bool i8 = syrk_i8_enabled(ws);
+int chol_factor(double* A, int64_t n_pad, int64_t ld, CholWorkspace ws, cudaStream_t st, int batch) {
+  cudaMemsetAsync(ws.info, 0, sizeof(int) * std::max(batch, 1), st);
+  const bool i8 = batch == 0 && syrk_i8_enabled(ws);
   const int64_t nt = n_pad / kTile;
   const int64_t outer = chol_outer(n_pad);
   static int lookahead = -1;  // COCONS_CHOL_LOOKAHEAD=0: panel work on the main stream too (debugging knob)
@@ -1133,7 +1182,7 @@ int chol_factor(double* A, int64_t n_pad, int64_t ld, CholWorkspace ws, cudaStre
     lookahead = e ? atoi(e) : 1;
   }
   cudaStream_t ps = lookahead ? ws.panel_stream : st;
-  factor_panel(A, n_pad, ld, ws, 0, std::min<int64_t>(outer, nt), st);
+  factor_panel(A, n_pad, ld, ws, 0, std::min<int64_t>(outer, nt), st, batch);
   for (int64_t J0 = 0; J0 < nt; J0 += outer) {
     const int64_t jb = std::min<int64_t>(outer, nt - J0);
     const int64_t done = (J0 + jb) * kTile;
@@ -1148,11 +1197,11 @@ int chol_factor(double* A, int64_t n_pad, int64_t ld, CholWorkspace ws, cudaStre
       g_syrk_i8.split(P, ld, trail, ws.i8_slices, ws.i8_scale, st);
       g_syrk_i8.update(trail, wnext, ws.i8_slices, ws.i8_scale, 0, 0, A + done * ld + done, ld, 1, ws.info, st);
     } else {
-      launch_gemm_nt(0, trail, wnext, jb * kTile, P, ld, P, ld, A + done * ld + done, ld, 1, st);  // (a)
+      launch_gemm_nt(0, trail, wnext, jb * kTile, P, ld, P, ld, A + done * ld + done, ld, 1, st, batch);  // (a)
     }
     cudaEventRecord(ws.ev_a, st);
     cudaStreamWaitEvent(ps, ws.ev_a, 0);
-    factor_panel(A, n_pad, ld, ws, J0 + jb, nb_next, ps);
+    factor_panel(A, n_pad, ld, ws, J0 + jb, nb_next, ps, batch);
     cudaEventRecord(ws.ev_p, ps);
     if (rest > 0) {  // (b)
       double* C2 = A + (done + wnext) * ld + done + wnext;
@@ -1167,7 +1216,7 @@ int chol_factor(double* A, int64_t n_pad, int64_t ld, CholWorkspace ws, cudaStre
         g_syrk_i8.update(rest, rest, ws.i8_slices, ws.i8_scale, wnext, wnext, C2, ld, 1, ws.info, st);
       } else {
         const double* P2 = P + wnext;
-        launch_gemm_nt(0, rest, rest, jb * kTile, P2, ld, P2, ld, C2, ld, 1, st);
+        launch_gemm_nt(0, rest, rest, jb * kTile, P2, ld, P2, ld, C2, ld, 1, st, batch);
       }
       if (J0 == 0) cudaEventRecord(ws.ev_k1, st);
     }

@@ -63,11 +63,18 @@ void note_launch(int count = 1);  // kernel-launch counter behind cocons_launch_
 
 // ---- assembly.cu ---------------------------------------------------------
 int smooth_mode_for(int par, int p, const double* theta6_host, const double* limits_host, double* nu_fixed);
+// batch > 0: `batch` site tables, table b from theta6 + 7 p b into T.base + SF_COUNT T.stride b (one launch)
 void launch_site_stage(int64_t n, int64_t n_fill, int p, const double* dX, int64_t ldx, const double* dlocs,
                        int64_t ldl, const double* dtheta6, double lim0, double lim1, int mode, SiteTable T,
-                       cudaStream_t st);
+                       cudaStream_t st, int batch = 0);
 void launch_assemble_lower(int64_t n, int64_t n_out, SiteTable T, double global_range, double nu_fixed, int mode,
                            double* C, int64_t ld, cudaStream_t st);
+// the lower triangles of `batch` matrices (n_out x n_out, ld = T.stride = n_out, back to back from C) in one launch,
+// matrix b from the site table at T.base + SF_COUNT T.stride b with global range dranges[b] (device memory); it runs
+// in the instantiations assemble_lower_kernel<mode + kAsmBatch> of its own
+constexpr int kAsmBatch = 8;
+void launch_assemble_lower_batch(int64_t n, int64_t n_out, SiteTable T, const double* dranges, double nu_fixed,
+                                 int mode, double* C, int batch, cudaStream_t st);
 void launch_assemble_panel(int64_t n, int64_t n_out, SiteTable T, double global_range, double nu_fixed, int mode,
                            double* slab, int64_t ld, int col_tile0, int ncol_tiles, cudaStream_t st);
 void launch_assemble_cyclic(int64_t n, int64_t n_out, SiteTable T, double global_range, double nu_fixed, int mode,
@@ -129,20 +136,25 @@ struct CholWorkspace {
 };
 constexpr int kSolveMaxRhs = 8;   // right-hand sides per launch of the substitution kernels
 constexpr int kSolveChunk = 16;   // tile columns per work unit (2 MB of L)
-// with_i8: also the slice workspace of the split-int8 trailing update, when n_pad reaches it (kSyrkI8MinPad)
-int chol_workspace_create(int64_t n_pad, CholWorkspace* ws, bool with_i8 = false);
+// with_i8: also the slice workspace of the split-int8 trailing update, when n_pad reaches it (kSyrkI8MinPad);
+// batch: inverted diagonal tiles and info words for that many matrices (chol_factor with batch > 0)
+int chol_workspace_create(int64_t n_pad, CholWorkspace* ws, bool with_i8 = false, int64_t batch = 1);
 void chol_workspace_destroy(CholWorkspace* ws);
 // tiles [J0, J0+jb) of one outer panel (potrf + panel solve + in-panel update) on stream st; A is the
 // address element (0,0) of the full matrix would have (only columns of the panel are touched)
 void factor_panel(double* A, int64_t n_pad, int64_t ld, const CholWorkspace& ws, int64_t J0, int64_t jb,
-                  cudaStream_t st);
-int chol_factor(double* A, int64_t n_pad, int64_t ld, CholWorkspace ws, cudaStream_t st);
+                  cudaStream_t st, int batch = 0);
+// batch > 0: the `batch` matrices n_pad x n_pad (ld = n_pad) back to back from A, each launch serving all of them;
+// matrix b has the inverted tiles ws.winv + b n_pad 128 and the info word ws.info[b].  The arithmetic of each matrix
+// is that of batch = 0, in the same order.  The DMMA GEMM only: for n_pad < kSyrkI8MinPad.
+int chol_factor(double* A, int64_t n_pad, int64_t ld, CholWorkspace ws, cudaStream_t st, int batch = 0);
 int chol_outer(int64_t n_pad);  // tiles per outer panel of chol_factor
 // diagonal tile: Cholesky in place (leading dimension ld) and its explicit inverse into Winv (128 x 128); the first
 // failing pivot sets *info = first_index + its 1-based order
-void launch_potrf_tile(double* A, int64_t ld, double* Winv, int* info, int first_index, cudaStream_t st);
+void launch_potrf_tile(double* A, int64_t ld, double* Winv, int* info, int first_index, cudaStream_t st,
+                       int batch = 0);
 void launch_gemm_nt(int mode, int64_t M, int64_t N, int64_t K, const double* A, int64_t lda, const double* B,
-                    int64_t ldb, double* C, int64_t ldc, int lower_only, cudaStream_t st);
+                    int64_t ldb, double* C, int64_t ldc, int lower_only, cudaStream_t st, int batch = 0);
 // Tiled tapered context (K8a-c in chol.cu, run by gemm_nt_tma_kernel instantiations of their own).  Right-hand sides
 // are row-major n_pad x ldb, ldb a multiple of 8.  A dependency wait that does not end (a bug) sets *info =
 // COCONS_ERR_CUDA instead of hanging.  Each launch first copies its TiledArgs to `slot` (device memory).

@@ -87,6 +87,37 @@ GetNeg2loglikelihoodREML <- function(theta, par.pos, locs, x_covariates, x_betas
   sum_logliks + .cocons.getPen((n - p) * dim(z)[2], lambda, theta_list, smooth.limits)
 }
 
+# ---- many points per call: the finite-difference points of cocoOptim, the points of getHessian ----------------
+# One .Call evaluates every point of `thetas` (a list of parameter vectors) on a batch context, up to `batch` points
+# per launch of the assembly and the factorisation (n <= 16 256 sites).  The values are those of the closures above,
+# bit for bit, including `safe` -> 1e6 per point; with safe = FALSE the first point that is not PD stops.
+#   bctx <- .Call(`_cocons_ctx_new_batch`, locs, as.matrix(x_covariates), as.matrix(z), 8L, 0L)
+#   on.exit(.Call(`_cocons_ctx_free`, bctx))
+#   (PROFILE: .Call(`_cocons_ctx_set_xbetas`, bctx, as.matrix(x_betas)); REML: z are the contrasts)
+GetNeg2loglikelihoodBatch <- function(kind, thetas, par.pos, bctx, smooth.limits, n, r, lambda, safe = TRUE) {
+  lists <- lapply(thetas, function(theta) cocons::getModelLists(theta = theta, par.pos = par.pos, type = "diff"))
+  p <- length(lists[[1]]$scale)
+  means <- if (kind == 0L) lapply(lists, function(l) l$mean) else NULL
+  out <- .Call(`_cocons_ctx_n2ll_batch`, bctx, as.integer(kind), lapply(lists, function(l) l[-1]), p, r,
+               smooth.limits, means)
+  names(out) <- c("logdet", "quad", "logdet_w", "rank_x", "status")
+  vapply(seq_along(lists), function(i) {
+    if (out$status[i] < 0) stop("cocons_b200: evaluation ", i, " failed with status ", out$status[i])
+    if (out$status[i] > 0) {
+      if (safe) return(1e+06)
+      stop("Cholesky error")
+    }
+    quad <- out$quad[, i]
+    if (kind == 2L) {
+      np <- out$rank_x
+      sum((n - np) * log(2 * pi) + 2 * out$logdet[i] + 2 * out$logdet_w[i] + quad) +
+        .cocons.getPen((n - np) * r, lambda, lists[[i]], smooth.limits)
+    } else {
+      sum(n * log(2 * pi) + 2 * out$logdet[i] + quad) + .cocons.getPen(n * r, lambda, lists[[i]], smooth.limits)
+    }
+  }, numeric(1))
+}
+
 # ---- tapered objectives (R/neg2loglikelihood.R:20-108) -----------------------------------
 # The tapered matrix is factored densely on the device instead of by spam's sparse Cholesky, so `cholS`
 # is accepted and unused.  A context per call keeps the closures drop-in; cocoOptim's sparse branch

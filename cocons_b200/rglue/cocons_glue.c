@@ -303,6 +303,76 @@ SEXP _cocons_ctx_n2ll(SEXP ptr, SEXP kindS, SEXP thetaS, SEXP pS, SEXP rS, SEXP 
   return out;
 }
 
+/* ---- batch context: many points per call (cocons_ctx_create_batch) ------------------------------------------------ */
+
+SEXP _cocons_ctx_new_batch(SEXP locsS, SEXP xS, SEXP zS, SEXP batchS, SEXP deviceS) {
+  SEXP locs = PROTECT(as_real(locsS)), x = PROTECT(as_real(xS)), z = PROTECT(as_real(zS));
+  check_sites("ctx_new_batch", locs, x);
+  need(rows_of(z) == Rf_nrows(locs), "ctx_new_batch", "z must have nrow(locs) rows");
+  const int batch = Rf_asInteger(batchS);
+  need(batch >= 1, "ctx_new_batch", "batch must be a positive integer");
+  const int n = Rf_nrows(locs), p = Rf_ncols(x), r = Rf_isMatrix(z) ? Rf_ncols(z) : 1;
+  cocons_ctx* c = NULL;
+  int rc = cocons_ctx_create_batch(Rf_asInteger(deviceS), n, p, r, REAL(locs), REAL(x), REAL(z), batch, NULL, &c);
+  UNPROTECT(3);
+  raise(rc);
+  SEXP ptr = PROTECT(R_MakeExternalPtr(c, R_NilValue, R_NilValue));
+  R_RegisterCFinalizerEx(ptr, ctx_finalizer, TRUE);
+  UNPROTECT(1);
+  return ptr;
+}
+
+/* list(logdet[npoints], quad (r x npoints), logdet_w[npoints], rank_x, status[npoints]) for a list of named theta
+ * lists and a list of mean vectors (or NULL); status[i] is what _cocons_ctx_n2ll's status would be for point i */
+SEXP _cocons_ctx_n2ll_batch(SEXP ptr, SEXP kindS, SEXP thetasS, SEXP pS, SEXP rS, SEXP limS, SEXP meansS) {
+  const ctx_view v = view_of(ptr);
+  SEXP lim = PROTECT(as_real(limS));
+  const int p = Rf_asInteger(pS), r = Rf_asInteger(rS);
+  need(p == v.p && r == v.r, "ctx_n2ll_batch", "p / r differ from the context's");
+  check_limits("ctx_n2ll_batch", lim);
+  need(TYPEOF(thetasS) == VECSXP && XLENGTH(thetasS) >= 1, "ctx_n2ll_batch", "thetas must be a non-empty list");
+  const int npts = LENGTH(thetasS);
+  need(Rf_isNull(meansS) || (TYPEOF(meansS) == VECSXP && LENGTH(meansS) == npts), "ctx_n2ll_batch",
+       "means must be NULL or a list with one vector per point");
+  /* every check that can raise an R error before the buffers exist (pack_theta raises only before its malloc) */
+  for (int i = 0; i < npts; ++i) {
+    free(pack_theta(VECTOR_ELT(thetasS, i), p));
+    if (!Rf_isNull(meansS)) need(LENGTH(VECTOR_ELT(meansS, i)) == p, "ctx_n2ll_batch", "every mean must have length p");
+  }
+  SEXP means = PROTECT(Rf_allocVector(VECSXP, Rf_isNull(meansS) ? 0 : npts));
+  for (int i = 0; !Rf_isNull(meansS) && i < npts; ++i) SET_VECTOR_ELT(means, i, as_real(VECTOR_ELT(meansS, i)));
+  SEXP out = PROTECT(Rf_allocVector(VECSXP, 5));
+  SEXP logdet = PROTECT(Rf_allocVector(REALSXP, npts)), quad = PROTECT(Rf_allocMatrix(REALSXP, r, npts));
+  SEXP ldw = PROTECT(Rf_allocVector(REALSXP, npts)), status = PROTECT(Rf_allocVector(INTSXP, npts));
+  for (int i = 0; i < npts; ++i) REAL(logdet)[i] = R_NaReal, REAL(ldw)[i] = 0.0;
+  for (R_xlen_t i = 0; i < (R_xlen_t)r * npts; ++i) REAL(quad)[i] = R_NaReal;
+  double* th = (double*)malloc(sizeof(double) * 6 * (size_t)p * npts);
+  double* mean = Rf_isNull(meansS) ? NULL : (double*)malloc(sizeof(double) * (size_t)p * npts);
+  const int oom = !th || (!mean && !Rf_isNull(meansS));
+  int rc = 0, rank = 0;
+  if (!oom) {
+    for (int i = 0; i < npts; ++i) {
+      double* one = pack_theta(VECTOR_ELT(thetasS, i), p);
+      memcpy(th + (size_t)6 * p * i, one, sizeof(double) * 6 * (size_t)p);
+      free(one);
+      if (mean) memcpy(mean + (size_t)p * i, REAL(VECTOR_ELT(means, i)), sizeof(double) * (size_t)p);
+    }
+    rc = cocons_n2ll_batch(v.c, Rf_asInteger(kindS), npts, th, REAL(lim), mean, REAL(logdet), REAL(quad), REAL(ldw),
+                           &rank, INTEGER(status));
+  }
+  free(th);
+  free(mean);
+  SET_VECTOR_ELT(out, 0, logdet);
+  SET_VECTOR_ELT(out, 1, quad);
+  SET_VECTOR_ELT(out, 2, ldw);
+  SET_VECTOR_ELT(out, 3, Rf_ScalarInteger(rank));
+  SET_VECTOR_ELT(out, 4, status);
+  UNPROTECT(7);
+  if (oom) Rf_error("out of memory");
+  raise(rc);
+  return out;
+}
+
 SEXP _cocons_ctx_factor(SEXP ptr, SEXP parS, SEXP thetaS, SEXP pS, SEXP limS) {
   const ctx_view v = view_of(ptr);
   SEXP lim = PROTECT(Rf_isNull(limS) ? limS : as_real(limS));
@@ -487,6 +557,8 @@ static const R_CallMethodDef CallEntries[] = {
     {"_cocons_ctx_set_z", (DL_FUNC)&_cocons_ctx_set_z, 2},
     {"_cocons_ctx_set_xbetas", (DL_FUNC)&_cocons_ctx_set_xbetas, 2},
     {"_cocons_ctx_n2ll", (DL_FUNC)&_cocons_ctx_n2ll, 7},
+    {"_cocons_ctx_new_batch", (DL_FUNC)&_cocons_ctx_new_batch, 5},
+    {"_cocons_ctx_n2ll_batch", (DL_FUNC)&_cocons_ctx_n2ll_batch, 7},
     {"_cocons_ctx_factor", (DL_FUNC)&_cocons_ctx_factor, 5},
     {"_cocons_ctx_profile_betas", (DL_FUNC)&_cocons_ctx_profile_betas, 3},
     {"_cocons_ctx_predict", (DL_FUNC)&_cocons_ctx_predict, 4},

@@ -110,6 +110,33 @@ int cocons_ctx_set_xbetas(cocons_ctx* ctx, int64_t q, const double* x_betas);
 int cocons_n2ll(cocons_ctx* ctx, int kind, const double* theta6, const double* smooth_limits, const double* mean_p,
                 double* logdet, double* quad, double* logdet_w, int* rank_x);
 
+/* ---- batch context: many objective evaluations per call --------------------
+ * Fits and Hessians evaluate the objective at many independent points (the 2p + 1 finite-difference points of an
+ * L-BFGS-B step, R/optim.R:237-259; the 1 + p + p(p+1)/2 points of getHessian, R/getFunctions.R:979-1016).  Below
+ * ~16 000 sites one evaluation cannot fill a B200; a batch context holds `batch` matrices over the same data (locs,
+ * x_covariates, z and the Morton order shared) and evaluates up to `batch` points with one launch per step of the
+ * assembly and the factorisation across all of them.
+ *
+ * n_pad = ceil(n/128)*128 must be < 16 384 (above it the split-int8 update takes over and one evaluation fills the
+ * device): COCONS_ERR_ARG otherwise.  COCONS_ERR_ALLOC, with nothing left allocated, if the matrices do not fit.
+ * On a batch context cocons_n2ll_batch, cocons_ctx_set_z, cocons_ctx_set_xbetas, cocons_ctx_dims, cocons_ctx_timings
+ * (the phases of the last call, added up over its groups) and cocons_ctx_destroy work; every other context entry
+ * returns COCONS_ERR_STATE. */
+int cocons_ctx_create_batch(int device, int64_t n, int64_t p, int64_t r, const double* locs,
+                            const double* x_covariates, const double* z, int64_t batch, void* stream,
+                            cocons_ctx** out);
+/* npoints >= 1 points, `batch` at a time; the arguments are those of cocons_n2ll, one column per point:
+ *   theta6 6p x npoints, mean_p p x npoints (ML) or NULL; logdet[npoints], quad r x npoints, logdet_w[npoints]
+ *   (or NULL), rank_x one value (or NULL), status[npoints].
+ * status[i] is what cocons_n2ll returns for point i alone: 0, k > 0 when that point is not PD, or that point's own
+ * error; the outputs of a point with status != 0 are not written.  Each point's values are bit for bit those of
+ * cocons_n2ll on a dense context, whatever the other points of the call and their order.  The return value is < 0
+ * only for a failure of the whole call (arguments, state, CUDA); COCONS_ERR_STATE on a context that is not a batch
+ * context. */
+int cocons_n2ll_batch(cocons_ctx* ctx, int kind, int64_t npoints, const double* theta6, const double* smooth_limits,
+                      const double* mean_p, double* logdet, double* quad, double* logdet_w, int* rank_x,
+                      int* status);
+
 /* ---- sparse (tapered) model, src/cocons_taper.cpp ------------------------
  * The pattern is spam's CSR layout as the reference receives it: 1-based
  * `colindices` (nnz) and `rowpointers` (rows + 1), INTSXP slots of the spam

@@ -31,7 +31,7 @@ int main() {
   cudaMalloc(&dA, sizeof(double) * n * n * reps);
   cudaMalloc(&dW, sizeof(double) * n * n * reps);
   cudaMalloc(&dinfo, 4);
-  cudaFuncSetAttribute(cocons::potrf_tile_blocked_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+  cudaFuncSetAttribute(cocons::potrf_tile_blocked_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                        cocons::kPotrfBlockedSmem);
   for (int cas = 0; cas < 3; ++cas) {
     std::vector<double> A((size_t)n * n);
@@ -59,7 +59,7 @@ int main() {
       if (variant == 1)
         cocons::potrf_tile_kernel<<<1, 256>>>(dA, n, dW, dinfo, 0);
       else
-        cocons::potrf_tile_blocked_kernel<<<1, 256, cocons::kPotrfBlockedSmem>>>(dA, n, dW, dinfo, 0);
+        cocons::potrf_tile_blocked_kernel<0><<<1, 256, cocons::kPotrfBlockedSmem>>>(dA, n, dW, dinfo, 0);
       cudaError_t e = cudaDeviceSynchronize();
       std::vector<double> L((size_t)n * n), W((size_t)n * n);
       int info = -1;
@@ -96,7 +96,7 @@ int main() {
       if (variant == 1)
         cocons::potrf_tile_kernel<<<1, 256>>>(dA, n, dW, dinfo, 1000);
       else
-        cocons::potrf_tile_blocked_kernel<<<1, 256, cocons::kPotrfBlockedSmem>>>(dA, n, dW, dinfo, 1000);
+        cocons::potrf_tile_blocked_kernel<0><<<1, 256, cocons::kPotrfBlockedSmem>>>(dA, n, dW, dinfo, 1000);
       cudaDeviceSynchronize();
       int info = -1;
       cudaMemcpy(&info, dinfo, 4, cudaMemcpyDeviceToHost);
@@ -121,7 +121,7 @@ int main() {
           if (variant == 1)
             cocons::potrf_tile_kernel<<<1, 256>>>(dA + (size_t)r * n * n, n, dW + (size_t)r * n * n, dinfo, 0);
           else
-            cocons::potrf_tile_blocked_kernel<<<1, 256, cocons::kPotrfBlockedSmem>>>(dA + (size_t)r * n * n, n,
+            cocons::potrf_tile_blocked_kernel<0><<<1, 256, cocons::kPotrfBlockedSmem>>>(dA + (size_t)r * n * n, n,
                                                                                      dW + (size_t)r * n * n, dinfo, 0);
         }
         cudaEventRecord(e1);
