@@ -8,7 +8,8 @@
 //   Product: S_w = sum_{t+u=w} A_t A_u^T for the 8 weights w = 2..9 (36 slice products), each exact in int32
 //   (|S_w| < 768 (2 127 64 + 6 64^2) < 2^25), then per entry hi = sum_{w<=5} S_w 2^7(5-w) and lo = sum_{w>5}
 //   S_w 2^7(9-w), exact in int64, and C_ij -= ((hi 2^-35 + lo 2^-63) s_i) s_j: one rounding for the sum, one
-//   for the subtraction, in a fixed order - the result is bitwise reproducible and independent of the tiling.
+//   for the subtraction (the scalings are exact unless they underflow), in a fixed order - the result is bitwise
+//   reproducible, independent of the tiling and equal to tools/ozaki_model.py.
 //
 // Layout of the slices: for every 128-row tile r of P and every 32-column chunk c (24 of them), a 32 KB block of
 // the 8 slices, each 128 rows x 32 B in the UMMA K-major SWIZZLE_32B layout (row i at 32 i, 16-byte half h stored
@@ -172,21 +173,32 @@ __host__ __device__ __forceinline__ uint32_t sw32_offset(int i, int b) {
 
 }  // namespace
 
-// one thread per row, 128 rows (one tile) per block
+// one thread per row, 128 rows (one tile) per block.  A row with a NaN or infinite entry gets the scale NaN (its
+// slices are then immaterial): every entry of C in its row and column becomes NaN, as on the DMMA path, and the
+// factorisation's pivot check reports the matrix as not positive definite.
 __global__ void __launch_bounds__(kSplitThreads) syrk_i8_split_kernel(const double* __restrict__ P, int64_t ld,
                                                                   int8_t* __restrict__ q, double* __restrict__ scale) {
   const int i = threadIdx.x;
   const int64_t tile = blockIdx.x, row = tile * kRowsA + i;
   const double* p = P + row;
-  double m = 0.0;
-  for (int k = 0; k < kSyrkI8K; ++k) m = fmax(m, fabs(p[(int64_t)k * ld]));
+  // max |P_ik| on the bit patterns, sign cleared: for non-negative doubles the integer order is the numeric one, and
+  // every NaN lies above infinity - unlike fmax, which skips a NaN
+  unsigned long long mb = 0;
+  for (int k = 0; k < kSyrkI8K; ++k)
+    mb = max(mb, (unsigned long long)__double_as_longlong(p[(int64_t)k * ld]) & 0x7FFFFFFFFFFFFFFFull);
+  const double m = __longlong_as_double((long long)mb);
+  const bool finite = mb < 0x7FF0000000000000ull;
   int e = 0;
-  if (m > 0.0) {
+  if (finite && m > 0.0) {
     frexp(m, &e);
     if (ldexp(m, 7 - e) >= 127.5) ++e;
   }
-  scale[row] = ldexp(1.0, e);
-  const double inv = ldexp(1.0, -e);
+  scale[row] = finite ? ldexp(1.0, e) : __longlong_as_double(0x7FF8000000000000ll);
+  // x = P_ik 2^-e as (P_ik f0) f1, both products exact: for a row maximum below 2^-1000, where 2^-e overflows or
+  // comes close, 2^-e = 2^64 2^(-e-64); otherwise f0 = 1 and f1 = 2^-e.  (ldexp(P_ik, -e) gives the same bits but
+  // compiles to a branchy sequence that kept the loads of the loop below from being unrolled: 5 % slower.)
+  const int e0 = e < -1000 ? 64 : 0;
+  const double f0 = ldexp(1.0, e0), f1 = ldexp(1.0, -e - e0);
   int8_t* qt = q + tile * kChunks * (int64_t)kBlockBytes;
   for (int c = 0; c < kChunks; ++c) {
 #pragma unroll
@@ -198,7 +210,7 @@ __global__ void __launch_bounds__(kSplitThreads) syrk_i8_split_kernel(const doub
         for (int t = 0; t < kSlices; ++t) w[t][k4] = 0;
 #pragma unroll
         for (int kb = 0; kb < 4; ++kb) {
-          double x = p[(int64_t)(c * kChunk + 16 * h + 4 * k4 + kb) * ld] * inv;
+          double x = __dmul_rn(__dmul_rn(p[(int64_t)(c * kChunk + 16 * h + 4 * k4 + kb) * ld], f0), f1);
 #pragma unroll
           for (int t = 0; t < kSlices; ++t) {
             const double y = x * 128.0;
@@ -449,7 +461,8 @@ __global__ void __launch_bounds__(kThreads, 1)
 #pragma unroll
           for (int j = 0; j < kEpiBatch; ++j) c[j] = __ldcs(Cg + (int64_t)(j0 + j) * ldc), s[j] = sbj[j0 + j];
 #pragma unroll
-          for (int j = 0; j < kEpiBatch; ++j) __stcs(Cg + (int64_t)(j0 + j) * ldc, c[j] - (v[j0 + j] * si) * s[j]);
+          for (int j = 0; j < kEpiBatch; ++j)  // three roundings, never contracted to an FMA: the model's arithmetic
+            __stcs(Cg + (int64_t)(j0 + j) * ldc, __dsub_rn(c[j], __dmul_rn(__dmul_rn(v[j0 + j], si), s[j])));
         }
       }
       I8_PROBE(if (tid == 64) p_epi += clock64() - t0;)

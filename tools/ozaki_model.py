@@ -31,21 +31,33 @@ PANEL = 768  # chol_factor's outer panel at n_pad >= 16 384 (6 tiles of 128)
 HI_TOP = 5   # weights 2..HI_TOP go to the high int64 word of the combination
 
 
-def row_scale(P):
-    """2^e per row: the least power of two with max |P_i.| 2^(7-e) < 127.5 (1 for a zero row)."""
-    m = np.max(np.abs(P), axis=1)
+def row_exponent(P):
+    """e per row: the least power of two 2^e with max |P_i.| 2^(7-e) < 127.5 (0 for a zero row), and whether the
+    row is finite"""
+    m = np.max(np.abs(P), axis=1)  # NaN when the row holds one
+    finite = np.isfinite(m)
     _, e = np.frexp(m)
     e = e.astype(np.int64)
     bump = np.ldexp(m, 7 - e) >= 127.5
     e = np.where(bump, e + 1, e)
-    e = np.where(m > 0, e, 0)
-    return np.ldexp(1.0, e)
+    e = np.where(finite & (m > 0), e, 0)
+    return e, finite
+
+
+def row_scale(P):
+    """2^e per row (1 for a zero row, NaN for a row with a NaN or infinite entry: the products of that row and
+    column are NaN, as in an FP64 product)"""
+    e, finite = row_exponent(P)
+    return np.where(finite, np.ldexp(1.0, e), np.nan)
 
 
 def split(P, slices):
-    """int8-valued slices A_t (as float64 arrays) and the row scales of P (m x K)."""
-    s = row_scale(P)
-    x = P / s[:, None]
+    """int8-valued slices A_t (as float64 arrays) and the row scales of P (m x K).  x = P_ik 2^-e_i is exact even
+    for a subnormal row maximum, where 2^-e_i itself overflows; a non-finite row gets zero slices (immaterial: its
+    scale is NaN)."""
+    e, finite = row_exponent(P)
+    s = np.where(finite, np.ldexp(1.0, e), np.nan)
+    x = np.where(finite[:, None], np.ldexp(P, -e[:, None]), 0.0)
     out = []
     for _ in range(slices):
         y = x * 128.0
